@@ -8,6 +8,7 @@ N > 1 one NCCL all-reduce of the parameter gradients per step.  One "step" = one
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            our arm (CUDA, one process per GPU under torchrun)
   python bench.py --impl reference [...]                          the CPU path (oracle port, all host threads), same metric
+  python bench.py [...] --dump-outputs DIR                        also write the last timed step's outputs as DIR/<name>.npy
 
 Prints ONE JSON line (rank 0).  See DESIGN.md section "Measurement" for how every field is computed.
 """
@@ -64,7 +65,15 @@ def parse():
     ap.add_argument("--parity-trials", type=int, default=8, help="trials of the in-bench oracle parity check (0 = skip)")
     ap.add_argument("--parity-steps", type=int, default=40)
     ap.add_argument("--probe-trials", type=int, default=1024, help="global trials of the sharding-invariance probe (0 = skip)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="c4: after the timed steps, write what the last timed step returned (loss, parameter gradients, a seeded "
+                         "sample of the trajectory) as DIR/<name>.npy, to compare two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "c4"):
+        ap.error("--dump-outputs is implemented for the c4 workload of --impl ours")
+    return args
 
 
 # ----------------------------------------------------------------------------------------------------------------------
@@ -315,6 +324,25 @@ def probe_block(torch, dist, odecol, net, args, tv, sel, dev, options, rank, wor
         p.grad = None
     return out
 
+
+def dump_outputs(torch, out_dir, loss, net, traj, budget=48 << 20):
+    """What the last timed step handed its caller, as float32 .npy files in out_dir: the loss, the gradients of both
+    parameters and the trajectory of the selected components (T, trials, components) of the step's last chunk.  The
+    trajectory (6 GB at the default shape) is sampled: a fixed, seeded set of at most 32 trials, every time point while the
+    sample fits `budget` bytes, every k-th otherwise.  Loss and trajectory repeat bit for bit from run to run; the gradients
+    are reduced over trials with float atomics (odeint's options['deterministic'] is off here, as in the timed steps), so
+    two runs of one build differ in their last bits (5e-7 relative on a B200): compare them with a float32 tolerance."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    T, B, S = traj.shape
+    k = max(1, min(32, B, budget // (4 * T * S)))
+    trials = torch.randperm(B, generator=torch.Generator(device="cpu").manual_seed(0))[:k].sort().values
+    every = -(-4 * T * S * k // budget)
+    out = {"loss": loss, "grad_recurrent_weights": net.recurrent_weights.grad, "grad_input_weights": net.input_weights.grad,
+           "trajectory_sample": traj[::every, trials.to(traj.device)]}
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v.detach().float().cpu().numpy())
+
 # ----------------------------------------------------------------------------------------------------------------------
 def init_nccl(torch, dist, dev):
     """One process per GPU over NCCL.  NCCL writes its version banner to STDOUT when the first communicator is created
@@ -380,6 +408,7 @@ def run_ours(args):
         loss + dW go back to the host inside the pass (the e2e leg)."""
         for p in params:
             p.grad = None
+        step.traj = None
         total = None
         for c in range(chunks):
             if from_host:
@@ -395,6 +424,8 @@ def run_ours(args):
             loss.backward()
             launches["n"] += ext.last_launch_count()
             total = loss.detach() if total is None else total + loss.detach()
+            if step.keep_traj and c == chunks - 1:
+                step.traj = traj.detach()
             del traj, loss
         total = total / chunks
         if world > 1:
@@ -408,6 +439,7 @@ def run_ours(args):
     step.y0_dev = y0_host.to(dev)
     step.ku_devs = [k.to(dev) for k in ku_hosts]
     step.ku_dev = step.ku_devs[0]
+    step.keep_traj = False                               # the timed steps keep their last trajectory for --dump-outputs
 
     def timed(n_steps, from_host):
         if world > 1:
@@ -432,9 +464,13 @@ def run_ours(args):
     if rank == 0:
         sampler.start()
     launches["n"] = 0
+    step.keep_traj = bool(args.dump_outputs)
     sec, (loss, _) = timed(args.steps, False)
     n_launch = launches["n"]
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, args.dump_outputs, loss, net, step.traj)
+    step.keep_traj, step.traj = False, None
     pop_steps_job = n * B * chunks * world * (T - 1)
     value = pop_steps_job * args.steps / sec
 

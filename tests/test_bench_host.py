@@ -41,6 +41,34 @@ def test_reference_arm_is_silent_on_the_other_ranks():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_dump_outputs_is_refused_where_it_is_not_implemented_and_steps_must_be_positive(tmp_path):
+    for extra in (["--dump-outputs", str(tmp_path)], ["--steps", "0"]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *TINY, *extra], capture_output=True, text=True, timeout=300)
+        assert r.returncode == 2 and r.stdout == "", r.stderr[-2000:]
+    assert not any(tmp_path.iterdir())
+
+
+def test_dump_outputs_writes_a_seeded_float32_sample_within_the_budget(tmp_path):
+    import numpy as np
+    from types import SimpleNamespace
+    g = torch.Generator().manual_seed(0)
+    net = SimpleNamespace(recurrent_weights=SimpleNamespace(grad=torch.randn(16, 16, generator=g)),
+                          input_weights=SimpleNamespace(grad=torch.randn(16, 2, generator=g)))
+    traj = torch.randn(50, 40, 6, generator=g)
+    trials = torch.randperm(40, generator=torch.Generator().manual_seed(0))
+    for budget, shape, every in ((10**9, (50, 32, 6), 1), (12000, (50, 10, 6), 1), (600, (25, 1, 6), 2)):
+        out = tmp_path / str(budget)
+        bench.dump_outputs(torch, str(out), torch.tensor(0.25), net, traj, budget=budget)
+        d = {p.stem: np.load(p) for p in out.iterdir()}
+        assert set(d) == {"loss", "grad_recurrent_weights", "grad_input_weights", "trajectory_sample"}
+        assert all(v.dtype == np.float32 for v in d.values()) and d["loss"] == np.float32(0.25)
+        assert np.array_equal(d["grad_recurrent_weights"], net.recurrent_weights.grad.numpy())
+        assert np.array_equal(d["grad_input_weights"], net.input_weights.grad.numpy())
+        assert d["trajectory_sample"].shape == shape and d["trajectory_sample"].nbytes <= budget
+        want = traj[::every, trials[:shape[1]].sort().values].numpy()
+        assert np.array_equal(d["trajectory_sample"], want)
+
+
 def test_loss_components_select_v_and_a_of_the_readout_populations_and_f_on_request():
     sel = bench.loss_components(torch, 4)
     n = 32
