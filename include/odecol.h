@@ -170,7 +170,9 @@ int odecol_rk4_fwd(const odecol_problem* p, const float* t, int32_t T, const flo
  * torchdiffeq's unrolled steps computes; scripts/xor_ode.py:177, scripts/parity_ode.py:250).
  *   y_traj      (T, B, 3N) the forward result with out_every = 1
  *   grad_y      (T, B, G)  dL/dy_out restricted to the state components sel[0..G); sel == NULL means
- *                          G = 3N, all components in order
+ *                          G = 3N, all components in order.  sel must hold DISTINCT components: each component reads
+ *                          one column of grad_y (with a repeat, which one is unspecified); a caller whose loss reads a
+ *                          component twice passes it once with the summed gradient
  *   grad_y0     (B, 3N)    out, may be NULL
  *   grad_W_aug  (N, ld_w)  out, OVERWRITTEN with sum over trials of dL/dW_aug (dW | dU | dbias) */
 int odecol_rk4_bwd(const odecol_problem* p, const float* t, int32_t T, const float* y_traj,

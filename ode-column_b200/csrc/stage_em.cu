@@ -742,7 +742,8 @@ int stage_drift(const DevProblem& p, const float* t_trial, const float* y, float
 // per trial block that forms the embedded error, takes the accept / reject decision and runs the step-size controller
 // exactly like k_dopri5_fwd_small (RMS over the trial's whole state in float64, controller in float64, time in
 // float64, state and tableau in float32), emits every output time inside an accepted step through the quartic dense
-// output and commits the step.  Forward only: training through dopri5 needs the on-chip family (N <= 128).
+// output and commits the step.  With a record (training) it leaves every accepted step for the staged reverse sweep,
+// stage_dopri5_bwd below.
 // ---------------------------------------------------------------------------------------------------------------
 namespace tc {
 

@@ -135,12 +135,24 @@ def _check_status(status: torch.Tensor, options: dict, what: str):
 
 
 def _sel_tensors(components, N3, device):
+    """(sel_long, sel_i32, inverse) of a component selection.  The kernels map each state component to one column of
+    grad_y (include/odecol.h), so they get the distinct components; when some repeat, ``_expand`` rebuilds the requested
+    columns outside the autograd Functions and autograd sums the gradients of the copies, as torch.index_select does."""
     if components is None:
-        return None, None
-    idx = torch.as_tensor(components, dtype=torch.int64, device=device).flatten()
+        return None, None, None
+    idx = torch.as_tensor(components, dtype=torch.int64).flatten().cpu()
     if idx.numel() == 0 or int(idx.min()) < 0 or int(idx.max()) >= N3:
         raise ValueError("odecol: components out of range")
-    return idx, idx.to(torch.int32).contiguous()
+    inverse = None
+    uniq, inv = torch.unique(idx, return_inverse=True)
+    if uniq.numel() < idx.numel():
+        idx, inverse = uniq, inv.to(device)
+    idx = idx.to(device)
+    return idx, idx.to(torch.int32).contiguous(), inverse
+
+
+def _expand(y, inverse):
+    return y if inverse is None else y.index_select(2, inverse)
 
 
 class _RK4Function(torch.autograd.Function):
@@ -249,7 +261,7 @@ def odeint(func, y0, t, *, rtol=1e-7, atol=1e-9, method=None, options=None, even
     options = dict(options or {})
     method = method or "dopri5"
     setup = _Setup(func, y0, t, options.pop("family", None), options.pop("deterministic", None))
-    sel_long, sel_i32 = _sel_tensors(components, 3 * setup.lf.N, y0.device)
+    sel_long, sel_i32, inverse = _sel_tensors(components, 3 * setup.lf.N, y0.device)
     if method == "rk4":
         if options.get("step_size") is not None:
             raise NotImplementedError("odecol rk4 integrates on the grid `t` (the reference passes no step_size)")
@@ -258,21 +270,24 @@ def odeint(func, y0, t, *, rtol=1e-7, atol=1e-9, method=None, options=None, even
         if sel_i32 is not None and needs_grad and ckpt is not False:
             nbytes = setup.ext.rk4_ckpt_bytes(setup.problem(setup.lf.W_aug), setup.t.numel())
             if nbytes > 0 and (ckpt is True or _ckpt_fits(nbytes, y0.device)):
-                return _RK4CkptFunction.apply(y0, setup.lf.W_aug, setup, sel_i32)
+                return _expand(_RK4CkptFunction.apply(y0, setup.lf.W_aug, setup, sel_i32), inverse)
             if ckpt is True:
                 raise RuntimeError("odecol: checkpoint mode is not available for this problem (tensor family only)")
-        return _RK4Function.apply(y0, setup.lf.W_aug, setup, sel_long, sel_i32)
+        return _expand(_RK4Function.apply(y0, setup.lf.W_aug, setup, sel_long, sel_i32), inverse)
     if method == "dopri5":
+        # torchdiffeq rejects such a grid; the kernels would emit NaN (on-chip) or y0 (staged) at a repeated time
+        if setup.t.numel() > 1 and not bool((setup.t[1:] > setup.t[:-1]).all()):
+            raise ValueError("odecol: dopri5 needs a strictly increasing time grid t")
         if torch.is_grad_enabled() and (y0.requires_grad or setup.lf.W_aug.requires_grad):
             from .dopri5_adjoint import dopri5_with_grad   # discrete adjoint through the accepted steps (both families)
-            return dopri5_with_grad(setup, y0, rtol, atol, options, sel_long, sel_i32, stats)
+            return _expand(dopri5_with_grad(setup, y0, rtol, atol, options, sel_long, sel_i32, stats), inverse)
         prob = setup.problem(setup.lf.W_aug)
         y, na, nr, st = setup.ext.dopri5_fwd(prob, setup.t, y0.detach().to(torch.float32).contiguous(), float(rtol),
                                              float(atol), int(options.get("max_num_steps", _DEFAULT_MAX_STEPS)))
         if stats is not None:
             stats.update(n_accept=na, n_reject=nr, status=st)
         _check_status(st, options, "dopri5")
-        return y if sel_long is None else y.index_select(2, sel_long)
+        return y if sel_long is None else _expand(y.index_select(2, sel_long), inverse)
     raise ValueError(f"odecol: method {method!r} is not fused (have 'rk4', 'dopri5')")
 
 
@@ -360,7 +375,7 @@ def sdeint(sde, y0, ts, bm=None, method=None, dt=1e-3, adaptive=False, rtol=1e-5
         if sc.numel() != setup.B:
             raise ValueError(f"odecol: options['sigma_scale'] needs {setup.B} entries (one per trial), got {sc.numel()}")
         setup.sigma_scale = sc
-    sel_long, sel_i32 = _sel_tensors(components, 3 * setup.lf.N, y0.device)
+    sel_long, sel_i32, inverse = _sel_tensors(components, 3 * setup.lf.N, y0.device)
     ext = setup.ext
     if seed is None:
         # torchsde builds a fresh BrownianInterval (new entropy) per call: draw a new key from torch's global generator, so
@@ -380,13 +395,13 @@ def sdeint(sde, y0, ts, bm=None, method=None, dt=1e-3, adaptive=False, rtol=1e-5
             if stats is not None:
                 stats.update(n_accept=na, n_reject=nr, status=st)
             _check_status(st, options, "adaptive srk")
-            return y if sel_long is None else y.index_select(2, sel_long)
+            return y if sel_long is None else _expand(y.index_select(2, sel_long), inverse)
         y, na, nr, st, _ = ext.em_fwd(prob, setup.t, y0.detach().to(torch.float32).contiguous(), None, seed,
                                       int(trial_offset), dt, True, float(rtol), float(atol), float(dt_min), 0)
         if stats is not None:
             stats.update(n_accept=na, n_reject=nr, status=st)
         _check_status(st, options, "adaptive Euler-Maruyama")
-        return y if sel_long is None else y.index_select(2, sel_long)
+        return y if sel_long is None else _expand(y.index_select(2, sel_long), inverse)
     ts_cpu = setup.t.cpu()
     n_steps = int(ext.em_num_steps(ts_cpu, dt))
     if method == "srk":
@@ -400,8 +415,8 @@ def sdeint(sde, y0, ts, bm=None, method=None, dt=1e-3, adaptive=False, rtol=1e-5
                 dW, dU = _tabulate_bm(bm, ts_cpu, dt, setup.B, y0.device, with_u=True)
                 if dW.shape != (n_steps, setup.B):
                     raise ValueError(f"odecol: bm produced increments of shape {tuple(dW.shape)}")
-        return _SRKFunction.apply(y0, setup.lf.W_aug, setup, dW, dU, seed, int(trial_offset), dt, n_steps, sel_long,
-                                  sel_i32, stats)
+        return _expand(_SRKFunction.apply(y0, setup.lf.W_aug, setup, dW, dU, seed, int(trial_offset), dt, n_steps, sel_long,
+                                          sel_i32, stats), inverse)
     dW = None
     if bm is not None:
         if torch.is_tensor(bm):
@@ -410,7 +425,8 @@ def sdeint(sde, y0, ts, bm=None, method=None, dt=1e-3, adaptive=False, rtol=1e-5
             dW = _tabulate_bm(bm, ts_cpu, dt, setup.B, y0.device)
             if dW.shape != (n_steps, setup.B):
                 raise ValueError(f"odecol: bm produced increments of shape {tuple(dW.shape)}")
-    return _EMFunction.apply(y0, setup.lf.W_aug, setup, dW, seed, int(trial_offset), dt, n_steps, sel_long, sel_i32, stats)
+    return _expand(_EMFunction.apply(y0, setup.lf.W_aug, setup, dW, seed, int(trial_offset), dt, n_steps, sel_long, sel_i32, stats),
+                   inverse)
 
 
 def sdeint_adjoint(sde, y0, ts, bm=None, method=None, adjoint_method=None, dt=1e-3, adaptive=False, adjoint_adaptive=False,

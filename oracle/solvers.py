@@ -168,8 +168,8 @@ def _dense_coeffs(y0, y1, k, dt, c_mid):
     return [e, d, c, b, a]
 
 
-def _dense_eval(coeffs, t0, t1, t):
-    x = ((t - t0) / (t1 - t0)).to(coeffs[0].dtype)
+def _dense_poly(coeffs, x):
+    """The dense-output quartic at abscissa x = (t - t0) / (t1 - t0)."""
     total = coeffs[0] + x * coeffs[1]
     xp = x
     for c in coeffs[2:]:
@@ -178,15 +178,70 @@ def _dense_eval(coeffs, t0, t1, t):
     return total
 
 
+def _dense_eval(coeffs, t0, t1, t):
+    return _dense_poly(coeffs, ((t - t0) / (t1 - t0)).to(coeffs[0].dtype))
+
+
+def _dp_tableau(dtype):
+    cast = lambda v: torch.tensor(v, dtype=torch.float64).to(dtype)
+    return cast(DP_ALPHA), [cast(b) for b in DP_BETA], cast(DP_C_ERR), cast(DP_C_MID)
+
+
+def dopri5_step(func, y0: torch.Tensor, t0, dt, f0: Optional[torch.Tensor] = None):
+    """One Dormand-Prince step of size dt from (t0, y0), state in y0's dtype, time in float64 -- the step odeint_dopri5
+    takes.  f0 = func(t0, y0) unless given (FSAL).  Returns (y1, f1, err, coeffs): the solution, its slope, the embedded
+    error estimate and the dense-output coefficients (evaluate with ``dense_output``).  Started from a recorded state it
+    checks one step of a solver in isolation."""
+    alpha, beta, c_err, c_mid = _dp_tableau(y0.dtype)
+    t0 = torch.as_tensor(t0, dtype=torch.float64)
+    dt = torch.as_tensor(dt, dtype=torch.float64)
+    if f0 is None:
+        f0 = _call(func, t0, y0)
+    y1, f1, err, k = _dp_step(func, y0, f0, t0, dt, t0 + dt, alpha, beta, c_err)
+    return y1, f1, err, _dense_coeffs(y0, y1, k, dt, c_mid)
+
+
+def dense_output(coeffs, x) -> torch.Tensor:
+    """The dense output of a step (coefficients from dopri5_step) at abscissa x in [0, 1]."""
+    return _dense_poly(coeffs, torch.as_tensor(x, dtype=torch.float64).to(coeffs[0].dtype))
+
+
+def dopri5_error_ratio(y0, y1, err, rtol: float, atol: float) -> torch.Tensor:
+    """torchdiffeq's RMS error ratio of a step (accepted iff <= 1)."""
+    return _rms(err / (atol + rtol * torch.max(y0.abs(), y1.abs()))).abs()
+
+
+def dopri5_replay(func, y0: torch.Tensor, t0, dt, n_accept: int, out_step, out_x) -> torch.Tensor:
+    """Differentiable replay of a recorded dopri5 solve of one trial group: accepted step n starts at t0[n] with size
+    dt[n] (chained from y0 with the FSAL slope, as the solver chains them); output j >= 1 is the dense output of step
+    out_step[j] at abscissa out_x[j], row 0 is y0.  The record fixes the discrete map, so autograd through the replay
+    gives the exact gradient of the computation a discrete adjoint differentiates, free of step-controller noise.  The
+    abscissae are taken as recorded (a float32 record is replayed at its float32 x)."""
+    T = len(out_step)
+    sol = [y0]
+    y, f = y0, None
+    j = 1
+    for n in range(int(n_accept)):
+        y1, f1, _, coeffs = dopri5_step(func, y, float(t0[n]), float(dt[n]), f)
+        while j < T and int(out_step[j]) == n:
+            sol.append(dense_output(coeffs, float(out_x[j])))
+            j += 1
+        y, f = y1, f1
+    if j != T:
+        raise ValueError(f"record places output {j} in no replayed step (out_step {int(out_step[j])}, n_accept {int(n_accept)})")
+    return torch.stack(sol, dim=0)
+
+
 def odeint_dopri5(func, y0: torch.Tensor, t: torch.Tensor, rtol: float = 1e-7, atol: float = 1e-9,
                   safety: float = 0.9, ifactor: float = 10.0, dfactor: float = 0.2,
-                  max_num_steps: int = 2 ** 31 - 1, stats: Optional[Dict] = None) -> torch.Tensor:
-    """Adaptive solve of ONE trial group (the error norm is taken over the whole tensor y)."""
+                  max_num_steps: int = 2 ** 31 - 1, stats: Optional[Dict] = None,
+                  record: Optional[Dict] = None) -> torch.Tensor:
+    """Adaptive solve of ONE trial group (the error norm is taken over the whole tensor y).  ``record`` (a dict) receives
+    the accepted steps in the layout of include/odecol.h's dopri5 record: ``t0`` / ``dt`` (float64, one entry per
+    accepted step) and, for every output j >= 1, ``out_step[j]`` (the accepted step it lies in) and ``out_x[j]`` (its
+    dense-output abscissa); entry 0 of both is 0.  ``dopri5_replay`` recomputes the solve from it."""
     dtype = y0.dtype
-    alpha = torch.tensor(DP_ALPHA, dtype=torch.float64).to(dtype)
-    beta = [torch.tensor(b, dtype=torch.float64).to(dtype) for b in DP_BETA]
-    c_err = torch.tensor(DP_C_ERR, dtype=torch.float64).to(dtype)
-    c_mid = torch.tensor(DP_C_MID, dtype=torch.float64).to(dtype)
+    alpha, beta, c_err, c_mid = _dp_tableau(dtype)
 
     t64 = t.to(torch.float64)
     f0 = _call(func, t64[0], y0)
@@ -195,6 +250,7 @@ def odeint_dopri5(func, y0: torch.Tensor, t: torch.Tensor, rtol: float = 1e-7, a
     coeffs = [y0] * 5
     n_acc = n_rej = 0
     sol = [y0]
+    rec_t0, rec_dt, out_step, out_x = [], [], [0], [0.0]
     for i in range(1, len(t64)):
         next_t = t64[i]
         n_steps = 0
@@ -211,6 +267,8 @@ def odeint_dopri5(func, y0: torch.Tensor, t: torch.Tensor, rtol: float = 1e-7, a
             if accept:
                 coeffs = _dense_coeffs(y_, y1, k, dt_, c_mid)
                 st_y, st_f, st_t0, st_t1 = y1, f1, t0_, t1_
+                rec_t0.append(float(t0_))
+                rec_dt.append(float(dt_))
                 n_acc += 1
             else:
                 st_t0 = t0_
@@ -225,9 +283,13 @@ def odeint_dopri5(func, y0: torch.Tensor, t: torch.Tensor, rtol: float = 1e-7, a
                     st_dt = dt_ * fac
             n_steps += 1
         sol.append(_dense_eval(coeffs, st_t0, st_t1, next_t))
+        out_step.append(n_acc - 1)
+        out_x.append(float((next_t - st_t0) / (st_t1 - st_t0)))
     if stats is not None:
         stats["n_accept"] = n_acc
         stats["n_reject"] = n_rej
+    if record is not None:
+        record.update(t0=rec_t0, dt=rec_dt, out_step=out_step, out_x=out_x)
     return torch.stack(sol, dim=0)
 
 

@@ -1,12 +1,14 @@
 """Differential test on problem shapes the reference networks do not reach: every register-tile size of the on-chip
 family (KP = 40 / 64 / 96 / 128), two trials per warp with and without it, more stimulus channels than lanes (the
 uncached knot path), ragged batches -- rk4 forward and reverse through the extension, against the CPU oracle's autograd;
-and the same problems forced through the staged FFMA and tensor families."""
+and the same problems forced through the staged FFMA and tensor families.  dopri5 is judged against a float64 replay of
+the steps its record holds (the oracle's adaptive solve takes another step sequence)."""
 import numpy as np
 import pytest
 import torch
 
 import odecol
+from helpers import check_dopri5_against_replay, ext_problem
 from oracle import rhs as orhs, solvers as S
 from oracle.column_model import LinearForm
 
@@ -70,6 +72,41 @@ def test_rk4_forward_and_reverse_on_random_problems(shape, family):
     print(f"\n[{shape} family {family}] trajectory {et:.1e}  grad y0 {e0:.1e}  grad W_aug {eW:.1e}")
     assert et < 1e-5 and e0 < 5e-5 and eW < 5e-5
     assert float(gW.cpu()[:, N + n_in + 1:].abs().max()) == 0 if ld > N + n_in + 1 else True     # padding columns stay zero
+
+
+#             rtol  atol  output grid: points over the 4.7 ms window
+DP_GRIDS = {"defaults": (1e-7, 1e-9, 48),       # the reference's tolerances: several steps between outputs, steps without one
+            "loose_dense": (1e-4, 1e-6, 189),   # several outputs inside one step (the dense-output adjoint)
+            "T2": (1e-7, 1e-9, 2)}              # one output at the end
+
+
+@pytest.mark.parametrize("grid", list(DP_GRIDS))
+@pytest.mark.parametrize("family", [0, "staged"])
+@pytest.mark.parametrize("shape", [(8, 1, 3, 2), (16, 20, 5, 3), (8, 40, 2, 3), (40, 8, 4, 5), (72, 10, 2, 3), (120, 7, 3, 4)],
+                         ids=lambda s: "N%d_in%d_B%d_K%d" % s)
+def test_dopri5_record_and_adjoint_against_a_float64_replay(shape, family, grid):
+    """dopri5 record / reverse sweep on every on-chip tile size (KP = 40 / 64 / 96 / 128), more stimulus channels than
+    lanes, ragged batches, and the same problems through the staged family, against a float64 replay of the recorded
+    steps.  The last trial is quiet (stimulus x 0.1, F starting at its rest value, so no fast transient): trials accept
+    different numbers of steps, so the staged reverse sweep runs ragged rounds, some with first steps and some without."""
+    N, n_in, B, K = shape
+    rtol, atol, T = DP_GRIDS[grid]
+    lf, tv, kt, ku, y0 = _problem(N, n_in, B, K, seed=N * 31 + n_in)
+    ku[-1] *= 0.1
+    y0[-1, 2 * N:] = orhs.phi(torch.tensor(y0[-1, :N] - y0[-1, N:2 * N])).numpy()
+    tv = np.linspace(0, tv[-1], T, dtype=np.float32)
+    ext = odecol._native.ext()
+    flags = {0: 0, "staged": ext.FLAG_FORCE_STAGED}[family]
+    prob = ext_problem(ext, lf, kt, ku, flags)
+    assert prob.kernel_family(ext.OP_DOPRI5_FWD) == {0: 0, "staged": 1}[family]
+    _, na, _, out_step, _ = check_dopri5_against_replay(ext, prob, lf, kt, ku, y0, tv, rtol, atol, f"{shape} {family} {grid}",
+                                                        controller=grid == "loose_dense", seed=N)
+    assert len(set(na.tolist())) > 1                          # ragged rounds in the staged reverse sweep
+    steps = out_step[:, 1:]
+    if grid == "defaults":
+        assert (np.diff(steps, axis=1) > 1).any()             # accepted steps that hold no output
+    if grid == "loose_dense":
+        assert (np.diff(steps, axis=1) == 0).any()            # several outputs inside one step
 
 
 @pytest.mark.parametrize("method", ["srk", "euler"])

@@ -215,6 +215,46 @@ def test_srk_strong_order_on_a_shared_brownian_path():
 # ---------------------------------------------------------------------------------------------------------------
 # independent third-party anchor that IS installed: scipy's Dormand-Prince (scipy.integrate.RK45)
 # ---------------------------------------------------------------------------------------------------------------
+@pytest.mark.parametrize("rtol,atol", [(1e-7, 1e-9), (1e-4, 1e-6)], ids=["reference_defaults", "loose"])
+def test_dopri5_replay_of_the_record_reproduces_the_solve_and_its_gradients(rtol, atol):
+    """The record of odeint_dopri5 (accepted t0 / dt, output step and abscissa) fixes the discrete map: replaying it in
+    float64 gives the solver's outputs and autograd's gradients (y0, W, U, bias) through its adaptive solve."""
+    from oracle import rhs as orhs
+    from oracle.column_model import LinearForm
+    rng = np.random.default_rng(5)
+    N, n_in, T = 8, 3, 25
+    lf = LinearForm(W=rng.standard_normal((N, N)) * 0.04, U=rng.standard_normal((N, n_in)) * 0.02, bias=rng.random(N) * 0.3,
+                    kappa=rng.random(N) * 1.5, sigma=np.zeros(3 * N), tau_s=5e-4, tau_m=0.02, tau_a=10.0, resistance=80.0)
+    kt = np.array([-1e-4, 6e-4, 1.1e-3, 2e-3])
+    ku = rng.random((1, 4, n_in)) * 20
+    t = torch.linspace(0, 2.4e-3, T, dtype=torch.float64)
+    y0 = torch.tensor(np.concatenate((rng.random(N) * 8 - 10, rng.random(N), rng.random(N) * 3))[None])
+    wgt = torch.tensor(rng.standard_normal((T, 1, 3 * N)))
+    runs = []
+    for replay in (False, True):
+        ode = orhs.UnifiedColumnODE(lf, kt, ku, dtype=torch.float64, requires_grad=True)
+        y0g = y0.clone().requires_grad_(True)
+        if replay:
+            y = S.dopri5_replay(ode, y0g, rec["t0"], rec["dt"], st["n_accept"], rec["out_step"], rec["out_x"])
+        else:
+            rec, st = {}, {}
+            y = S.odeint_dopri5(ode, y0g, t, rtol=rtol, atol=atol, stats=st, record=rec)
+        (y * wgt).sum().backward()
+        runs.append([y.detach(), y0g.grad, ode.W.grad, ode.U.grad, ode.bias.grad])
+    n = st["n_accept"]
+    assert len(rec["t0"]) == len(rec["dt"]) == n and len(rec["out_step"]) == len(rec["out_x"]) == T
+    assert all(rec["t0"][i + 1] == rec["t0"][i] + rec["dt"][i] for i in range(n - 1))
+    steps = np.array(rec["out_step"][1:])
+    assert np.all(np.diff(steps) >= 0) and steps[-1] == n - 1 and all(0 < x <= 1 for x in rec["out_x"][1:])
+    errs = [float((a - b).abs().max() / b.abs().max()) for a, b in zip(runs[1], runs[0])]
+    print(f"\n[oracle dopri5 replay rtol {rtol:g}] {n} accepted steps; trajectory / dy0 / dW / dU / dbias {errs}")
+    assert max(errs) < 1e-13
+    if rtol == 1e-7:
+        assert np.any(np.diff(steps) > 1)                      # steps with no output inside
+    else:
+        assert np.any(np.diff(steps) == 0)                     # several outputs inside one step
+
+
 def test_dopri5_tableau_equals_scipy_rk45():
     from scipy.integrate._ivp.rk import RK45
     A = np.asarray(RK45.A)                       # (6, 5): stage rows 0..5 (row 0 empty)
