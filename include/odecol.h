@@ -78,9 +78,10 @@ enum {
 
 /* odecol_problem.flags */
 enum {
-    ODECOL_FLAG_FORCE_STAGED = 1,  /* use the staged (global-state) FP32-FFMA kernel family even when the
-                                      problem fits the persistent on-chip family; for testing and measurement */
-    ODECOL_FLAG_FORCE_TENSOR = 2,  /* use the staged tcgen05 (split-operand, FP32-accurate) family regardless of size */
+    ODECOL_FLAG_FORCE_STAGED = 1,  /* skip the persistent on-chip family: use the staged (global-state) solvers even
+                                      when the problem fits on chip; for testing and measurement */
+    ODECOL_FLAG_FORCE_TENSOR = 2,  /* the same as ODECOL_FLAG_FORCE_STAGED (both values are kept for binary
+                                      compatibility; staged rk4 always runs in the tcgen05 family) */
     ODECOL_FLAG_DETERMINISTIC = 4  /* tensor family, rk4 reverse sweep: reduce grad_W_aug over trials in a fixed order
                                       (per-split copies summed at the end) instead of float atomics: bit-reproducible
                                       gradients for ~2 % of the sweep's time                                      */
@@ -371,7 +372,8 @@ int odecol_tc_contract_tn(const float* A, const float* B, float* C, int32_t M, i
                           void* workspace, size_t workspace_bytes, void* stream);
 
 /* Which kernel family a call would use: 0 = persistent on-chip ("small", W row in registers),
- * 1 = staged FP32-FFMA contraction, 2 = staged 3xTF32 tcgen05 contraction.  Diagnostic only. */
+ * 1 = staged dopri5 / Euler-Maruyama / srk (drift on the tensor cores), 2 = staged rk4 on the tcgen05 split-operand
+ * contraction.  rk4 ops report 0 or 2, the others 0 or 1.  Diagnostic only. */
 int odecol_kernel_family(const odecol_problem* p, int op);
 
 /* Number of kernel launches the most recent entry-point call enqueued (process-wide, for bench bookkeeping). */

@@ -24,14 +24,14 @@ LIB = LIBDIR / "libodecol.so"
 VARIANT_OUT = os.environ.get("ODECOL_LIB_OUT")
 EXT = PKG / ("_odecol_ext" + (sysconfig.get_config_var("EXT_SUFFIX") or ".so"))
 
-CUDA_SOURCES = ["abi.cu", "small_kernels.cu", "stage_kernels.cu", "stage_bwd.cu", "stage_em.cu", "stage_tc.cu", "stage_tc_bwd.cu", "stage_tc_persist.cu", "tiny_tc.cu", "ww_kernel.cu", "readout_kernels.cu"]
+CUDA_SOURCES = ["abi.cu", "small_kernels.cu", "stage_em.cu", "stage_tc.cu", "stage_tc_bwd.cu", "stage_tc_persist.cu", "tiny_tc.cu", "ww_kernel.cu", "readout_kernels.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "--expt-relaxed-constexpr", "-Xcompiler", "-fPIC",
 ]
 
 
-# experiments: extra nvcc flags (e.g. ODECOL_NVCC_EXTRA="-DODECOL_PREFETCH_AHEAD=0 -DODECOL_DIAG") for an A/B rebuild on the GPU box
+# experiments: extra nvcc flags (e.g. ODECOL_NVCC_EXTRA="-DODECOL_TC_STAGES=4") for an A/B rebuild on the GPU box
 NVCC_FLAGS += os.environ.get("ODECOL_NVCC_EXTRA", "").split()
 
 

@@ -28,16 +28,6 @@ static bool use_small(const odecol_problem* p, const DevProblem& d) {
     return !(p->flags & (ODECOL_FLAG_FORCE_STAGED | ODECOL_FLAG_FORCE_TENSOR)) && small_kp(d) != 0;
 }
 
-// staged problems (beyond the on-chip family): rk4 runs in the tensor family -- persistent tcgen05 forward solve, checkpoint
-// mode, chained reverse stages -- unless the FFMA family is forced or N is not a multiple of 4 (never the case for column
-// networks, N = 8 x columns).  Measured at 8192 trials (round 2): N = 136: 4.2e9 vs 1.1e9, N = 192: 5.5e9 vs 1.4e9
-// population-steps/s forward + adjoint; the former threshold (N >= 256) left a 4x on the table.
-static bool use_tensor(const odecol_problem* p, const DevProblem& d) {
-    if (p->flags & ODECOL_FLAG_FORCE_TENSOR) return true;
-    if (p->flags & ODECOL_FLAG_FORCE_STAGED) return false;
-    return d.N % 4 == 0;
-}
-
 // rk4 of a network that FITS the on-chip family still goes to the tensor family when the batch is large enough to fill the
 // machine with 128-row tiles: measured on the reference's parity network (N = 104; bench.py --workload small, round 2) the
 // two families break even at ~2048 trials (forward + adjoint 1.77e9 vs 1.67e9 population-steps/s); at 4096 trials the
@@ -87,10 +77,11 @@ int64_t odecol_last_launch_count(void) { return g_launches.load(std::memory_orde
 int odecol_kernel_family(const odecol_problem* p, int op) {
     DevProblem d;
     if (to_dev(p, d) != ODECOL_OK) return -1;
-    (void)op;
+    // rk4 beyond the on-chip family runs in the tensor family (persistent tcgen05 forward solve, checkpoint mode, chained
+    // reverse stages); the other solvers' staged paths are family 1
     const bool rk4 = op == ODECOL_OP_RK4_FWD || op == ODECOL_OP_RK4_BWD;
     if (rk4 ? use_small_rk4(p, d) : use_small(p, d)) return 0;
-    return use_tensor(p, d) && rk4 ? 2 : 1;
+    return rk4 ? 2 : 1;
 }
 
 size_t odecol_workspace_bytes(const odecol_problem* p, int op, int32_t T, int64_t n_steps) {
@@ -98,8 +89,8 @@ size_t odecol_workspace_bytes(const odecol_problem* p, int op, int32_t T, int64_
     if (to_dev(p, d) != ODECOL_OK) return 0;
     const bool small = use_small(p, d), small_rk4 = use_small_rk4(p, d);
     switch (op) {
-        case ODECOL_OP_RK4_FWD: return small_rk4 ? (tiny_rk4_applicable(d) ? 256 : 0) : (use_tensor(p, d) ? tc_rk4_fwd_workspace_bytes(d, T) : stage_rk4_fwd_workspace_bytes(d, T));
-        case ODECOL_OP_RK4_BWD: return small_rk4 ? 0 : (use_tensor(p, d) ? tc_rk4_bwd_workspace_bytes(d, T) : stage_rk4_bwd_workspace_bytes(d, T));
+        case ODECOL_OP_RK4_FWD: return small_rk4 ? (tiny_rk4_applicable(d) ? 256 : 0) : tc_rk4_fwd_workspace_bytes(d, T);
+        case ODECOL_OP_RK4_BWD: return small_rk4 ? 0 : tc_rk4_bwd_workspace_bytes(d, T);
         case ODECOL_OP_EM_FWD: return small ? 0 : stage_em_fwd_workspace_bytes(d, T);
         case ODECOL_OP_DOPRI5_FWD: return small ? 0 : stage_dopri5_fwd_workspace_bytes(d, T);
         case ODECOL_OP_DOPRI5_BWD: return small ? 0 : stage_dopri5_bwd_workspace_bytes(d, T);
@@ -153,8 +144,7 @@ int odecol_rk4_fwd(const odecol_problem* p, const float* t, int32_t T, const flo
         return launch_rk4_fwd_small(d, t, T, y0, y_out, out_every, s);
     }
     if (misaligned(y0) || misaligned(y_out) || misaligned(workspace)) return ODECOL_E_ALIGN;
-    if (use_tensor(p, d)) return tc_rk4_fwd(d, t, T, y0, y_out, out_every, workspace, workspace_bytes, s);
-    return stage_rk4_fwd(d, t, T, y0, y_out, out_every, workspace, workspace_bytes, s);
+    return tc_rk4_fwd(d, t, T, y0, y_out, out_every, workspace, workspace_bytes, s);
 }
 
 int odecol_rk4_bwd(const odecol_problem* p, const float* t, int32_t T, const float* y_traj, const float* grad_y,
@@ -171,14 +161,13 @@ int odecol_rk4_bwd(const odecol_problem* p, const float* t, int32_t T, const flo
     if (cudaMemsetAsync(grad_W_aug, 0, sizeof(float) * (size_t)p->N * p->ld_w, s) != cudaSuccess) return ODECOL_E_CUDA;
     if (use_small_rk4(p, d)) return launch_rk4_bwd_small(d, t, T, y_traj, grad_y, sel, G, grad_y0, grad_W_aug, s);
     if (misaligned(y_traj) || misaligned(workspace) || misaligned(grad_W_aug)) return ODECOL_E_ALIGN;
-    if (use_tensor(p, d)) return tc_rk4_bwd(d, t, T, y_traj, grad_y, sel, G, grad_y0, grad_W_aug, workspace, workspace_bytes, s);
-    return stage_rk4_bwd(d, t, T, y_traj, grad_y, sel, G, grad_y0, grad_W_aug, workspace, workspace_bytes, s);
+    return tc_rk4_bwd(d, t, T, y_traj, grad_y, sel, G, grad_y0, grad_W_aug, workspace, workspace_bytes, s);
 }
 
 size_t odecol_rk4_ckpt_bytes(const odecol_problem* p, int32_t T) {
     DevProblem d;
     if (to_dev(p, d) != ODECOL_OK || T < 2) return 0;
-    if (use_small_rk4(p, d) || !use_tensor(p, d) || p->N % 4 != 0) return 0;
+    if (use_small_rk4(p, d) || p->N % 4 != 0) return 0;
     return tc_rk4_ckpt_bytes(d, T);
 }
 
@@ -190,7 +179,7 @@ int odecol_rk4_fwd_ckpt(const odecol_problem* p, const float* t, int32_t T, cons
     if (d.lat_gain) return ODECOL_E_UNSUPPORTED;      // the lateral-gain axis exists in the staged Euler-Maruyama path only
     if (!t || !y0 || !y_sel || !ckpt) return ODECOL_E_NULL;
     if (T < 2 || G < 1 || G > 3 * p->N) return ODECOL_E_SHAPE;
-    if (use_small_rk4(p, d) || !use_tensor(p, d)) return ODECOL_E_UNSUPPORTED;
+    if (use_small_rk4(p, d)) return ODECOL_E_UNSUPPORTED;
     if (misaligned(y0) || misaligned(ckpt) || misaligned(workspace)) return ODECOL_E_ALIGN;
     g_launches.store(0, std::memory_order_relaxed);
     return tc_rk4_fwd_ckpt(d, t, T, y0, sel, G, y_sel, ckpt, ckpt_bytes, workspace, workspace_bytes,
@@ -206,7 +195,7 @@ int odecol_rk4_bwd_ckpt(const odecol_problem* p, const float* t, int32_t T, cons
     if (d.lat_gain) return ODECOL_E_UNSUPPORTED;      // the lateral-gain axis exists in the staged Euler-Maruyama path only
     if (!t || !ckpt || !grad_y_sel || !grad_W_aug) return ODECOL_E_NULL;
     if (T < 2 || G < 1 || G > 3 * p->N) return ODECOL_E_SHAPE;
-    if (use_small_rk4(p, d) || !use_tensor(p, d)) return ODECOL_E_UNSUPPORTED;
+    if (use_small_rk4(p, d)) return ODECOL_E_UNSUPPORTED;
     if (misaligned(ckpt) || misaligned(workspace) || misaligned(grad_W_aug)) return ODECOL_E_ALIGN;
     g_launches.store(0, std::memory_order_relaxed);
     cudaStream_t s = static_cast<cudaStream_t>(stream);

@@ -97,15 +97,8 @@ int launch_huber_rate_loss(const float* y_sel, int T, int B, int G, int P, const
 int launch_window_rate_l1_loss(const float* y_sel, int T, int B, int P, int L, const float* w, const float* target,
                                float* loss, float* pred, float* grad, float* grad_w, double* acc, cudaStream_t s);
 
-// ---- family L (stage_kernels.cu): state in global memory, one fused contraction + epilogue per RK stage ------
-struct StageWorkspace;   // carved from the caller's workspace
-size_t stage_rk4_fwd_workspace_bytes(const DevProblem& p, int T);
-size_t stage_rk4_bwd_workspace_bytes(const DevProblem& p, int T);
+// ---- staged Euler-Maruyama (stage_em.cu): state in global memory, the drift contraction on the tensor cores ------
 size_t stage_em_fwd_workspace_bytes(const DevProblem& p, int T);
-int stage_rk4_fwd(const DevProblem& p, const float* t_dev, int T, const float* y0, float* y_out, int out_every,
-                  void* ws, size_t ws_bytes, cudaStream_t s);
-int stage_rk4_bwd(const DevProblem& p, const float* t_dev, int T, const float* y_traj, const float* grad_y,
-                  const int* sel, int G, float* grad_y0, float* grad_W, void* ws, size_t ws_bytes, cudaStream_t s);
 int stage_em_fwd(const DevProblem& p, const float* ts_dev, int T, const float* y0, float* y_out, const float* dW,
                  uint64_t seed, int64_t trial_offset, float dt, int adaptive, float rtol, float atol, float dt_min,
                  int* n_accept, int* n_reject, int* status, float* y_steps, void* ws, size_t ws_bytes, cudaStream_t s);

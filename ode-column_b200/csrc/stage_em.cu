@@ -54,7 +54,6 @@ struct RhsEpi {
             fb[2 * N] = (r - yb[2 * N]) * inv_ts;
         }
     }
-    ODECOL_DEVINL void pre_tile(int, int, int, int) const {}
     ODECOL_DEVINL void tile_done(int, int, int, int, int) const {}
 };
 
@@ -551,39 +550,30 @@ static int em_fwd_impl(const DevProblem& p, const float* ts_dev, int T, const fl
     } else if (!make_map(&mWhi, Whi, L.Np, L.KPa, L.KPa, BM) || !make_map(&mWlo, Wlo, L.Np, L.KPa, L.KPa, BM) ||
                !make_map(&mRhi, Rhi, L.Bp, L.KPa, L.KPa, L.TN) || !make_map(&mRlo, Rlo, L.Bp, L.KPa, L.KPa, L.TN))
         return ODECOL_E_CUDA;
-    const TileShape tsh{L.Np / BM, L.Bp / L.TN, L.TN, f16 ? L.KP16 / BK16 : L.KPa / BK, 0, nullptr};
-    // CTA pairs (tcgen05 cta_group::2, ODECOL_PAIR=1): each SM stages half of the trial tile
-    const bool use_pair = !f16 && pair_enabled() && tsh.MT % 2 == 0;
-    CUtensorMap mRhHi, mRhLo;
-    if (use_pair && (!make_map(&mRhHi, Rhi, L.Bp, L.KPa, L.KPa, L.TN / 2) || !make_map(&mRhLo, Rlo, L.Bp, L.KPa, L.KPa, L.TN / 2)))
-        return ODECOL_E_CUDA;
+    const TileShape tsh{L.Np / BM, L.Bp / L.TN, L.TN, f16 ? L.KP16 / BK16 : L.KPa / BK, 0};
     auto rhs = [&](const float* ysrc, float* fdst) {
         RhsEpi e;
         e.p = p; e.y = ysrc; e.Rhi = Rhi; e.Rlo = Rlo; e.f = fdst; e.KPa = KPr; e.loc = loc; e.wscale = f16 ? aux : nullptr;
         e.inv_tm = 1.0f / p.c.tau_m; e.inv_ta = 1.0f / p.c.tau_a; e.inv_ts = 1.0f / p.c.tau_s;
         if (f16) return launch_contract16(mWhi, mWlo, mRhi, mRlo, tsh, e, s);
-        if (use_pair) return launch_contract_pair(mWhi, mWlo, mRhHi, mRhLo, tsh, e, s);
         return launch_contract(mWhi, mWlo, mRhi, mRlo, tsh, e, s);
     };
     // adaptive sweep: the midpoint evaluation f(t_mid, y_mid) reads operand set 1 (written by k_ad_half1), so that the
     // operand of f(t_cur, y) in set 0 (written by k_ad_commit) survives a rejected attempt
     float *Rhi1 = F(L.off_Rhi1), *Rlo1 = F(L.off_Rlo1);
     float* loc1 = p.lat_gain ? F(L.off_loc1) : nullptr;
-    CUtensorMap mRhi1, mRlo1, mRhHi1, mRhLo1;
+    CUtensorMap mRhi1, mRlo1;
     if (adaptive && f16) {
         if (!make_map16(&mRhi1, Rhi1, L.Bp, L.KP16, L.KP16, L.TN, false) || !make_map16(&mRlo1, Rlo1, L.Bp, L.KP16, L.KP16, L.TN, false))
             return ODECOL_E_CUDA;
     } else if (adaptive) {
         if (!make_map(&mRhi1, Rhi1, L.Bp, L.KPa, L.KPa, L.TN) || !make_map(&mRlo1, Rlo1, L.Bp, L.KPa, L.KPa, L.TN)) return ODECOL_E_CUDA;
-        if (use_pair && (!make_map(&mRhHi1, Rhi1, L.Bp, L.KPa, L.KPa, L.TN / 2) || !make_map(&mRhLo1, Rlo1, L.Bp, L.KPa, L.KPa, L.TN / 2)))
-            return ODECOL_E_CUDA;
     }
     auto rhs_mid = [&](const float* ysrc, float* fdst) {
         RhsEpi e;
         e.p = p; e.y = ysrc; e.Rhi = Rhi1; e.Rlo = Rlo1; e.f = fdst; e.KPa = KPr; e.loc = loc1; e.wscale = f16 ? aux : nullptr;
         e.inv_tm = 1.0f / p.c.tau_m; e.inv_ta = 1.0f / p.c.tau_a; e.inv_ts = 1.0f / p.c.tau_s;
         if (f16) return launch_contract16(mWhi, mWlo, mRhi1, mRlo1, tsh, e, s);
-        if (use_pair) return launch_contract_pair(mWhi, mWlo, mRhHi1, mRhLo1, tsh, e, s);
         return launch_contract(mWhi, mWlo, mRhi1, mRlo1, tsh, e, s);
     };
     const int ew_grid = (int)((st + 255) / 256 < 148 * 16 ? (st + 255) / 256 : 148 * 16);
@@ -727,7 +717,7 @@ int stage_drift(const DevProblem& p, const float* t_trial, const float* y, float
     if (!make_map(&mWhi, Whi, L.Np, L.KPa, L.KPa, BM) || !make_map(&mWlo, Wlo, L.Np, L.KPa, L.KPa, BM) ||
         !make_map(&mRhi, Rhi, L.Bp, L.KPa, L.KPa, L.TN) || !make_map(&mRlo, Rlo, L.Bp, L.KPa, L.KPa, L.TN))
         return ODECOL_E_CUDA;
-    const TileShape tsh{L.Np / BM, L.Bp / L.TN, L.TN, L.KPa / BK, 0, nullptr};
+    const TileShape tsh{L.Np / BM, L.Bp / L.TN, L.TN, L.KPa / BK, 0};
     RhsEpi e;
     e.p = p; e.y = y; e.Rhi = Rhi; e.Rlo = Rlo; e.f = f; e.KPa = L.KPa; e.loc = loc;
     e.inv_tm = 1.0f / p.c.tau_m; e.inv_ta = 1.0f / p.c.tau_a; e.inv_ts = 1.0f / p.c.tau_s;
@@ -1012,7 +1002,7 @@ static int dopri5_fwd_impl(const DevProblem& p, const float* ts_dev, int T, cons
     } else if (!make_map(&mWhi, Whi, L.Np, L.KPa, L.KPa, BM) || !make_map(&mWlo, Wlo, L.Np, L.KPa, L.KPa, BM) ||
                !make_map(&mRhi, Rhi, L.Bp, L.KPa, L.KPa, L.TN) || !make_map(&mRlo, Rlo, L.Bp, L.KPa, L.KPa, L.TN))
         return ODECOL_E_CUDA;
-    const TileShape tsh{L.Np / BM, L.Bp / L.TN, L.TN, f16 ? L.KP16 / BK16 : L.KPa / BK, 0, nullptr};
+    const TileShape tsh{L.Np / BM, L.Bp / L.TN, L.TN, f16 ? L.KP16 / BK16 : L.KPa / BK, 0};
     // f(t_stage[b], ysrc[b]) -> fdst for every trial (finished trials compute along harmlessly: rows are independent)
     auto rhs = [&](const float* ysrc, const float* t_trial, float t_shared, float* fdst) {
         k_em_operand<<<p.B, 128, 0, s>>>(p, ysrc, t_trial, t_shared, Rhi, Rlo, KPr, nullptr, nullptr, ovf);
@@ -1201,7 +1191,7 @@ static int srk_fwd_impl(const DevProblem& p, const float* ts_dev, int T, const f
     } else if (!make_map(&mWhi, Whi, L.Np, L.KPa, L.KPa, BM) || !make_map(&mWlo, Wlo, L.Np, L.KPa, L.KPa, BM) ||
                !make_map(&mRhi, Rhi, L.Bp, L.KPa, L.KPa, L.TN) || !make_map(&mRlo, Rlo, L.Bp, L.KPa, L.KPa, L.TN))
         return ODECOL_E_CUDA;
-    const TileShape tsh{L.Np / BM, L.Bp / L.TN, L.TN, f16 ? L.KP16 / BK16 : L.KPa / BK, 0, nullptr};
+    const TileShape tsh{L.Np / BM, L.Bp / L.TN, L.TN, f16 ? L.KP16 / BK16 : L.KPa / BK, 0};
     auto rhs = [&](const float* ysrc, float tq, float* fdst) {
         k_em_operand<<<p.B, 128, 0, s>>>(p, ysrc, nullptr, tq, Rhi, Rlo, KPr, nullptr, nullptr, ovf);
         count_launch();
@@ -1305,7 +1295,6 @@ struct VjpEpi {
             bt[2 * N] = -aF * inv_ts;
         }
     }
-    ODECOL_DEVINL void pre_tile(int, int, int, int) const {}
     ODECOL_DEVINL void tile_done(int, int, int, int, int) const {}
 };
 
@@ -1438,8 +1427,8 @@ struct AdjCtx {
             !make_map(&mRhi, F(L.off_Rhi), L.Bp, L.KPa, L.KPa, L.TN) || !make_map(&mRlo, F(L.off_Rlo), L.Bp, L.KPa, L.KPa, L.TN) ||
             !make_map(&mAVhi, F(L.off_AVhi), L.Bp, L.NPk, L.NPk, L.TN) || !make_map(&mAVlo, F(L.off_AVlo), L.Bp, L.NPk, L.NPk, L.TN))
             return ODECOL_E_CUDA;
-        tsF = TileShape{L.Np / BM, L.Bp / L.TN, L.TN, L.KPa / BK, 0, nullptr};
-        tsB = TileShape{L.Np / BM, L.Bp / L.TN, L.TN, L.NPk / BK, 0, nullptr};
+        tsF = TileShape{L.Np / BM, L.Bp / L.TN, L.TN, L.KPa / BK, 0};
+        tsB = TileShape{L.Np / BM, L.Bp / L.TN, L.TN, L.NPk / BK, 0};
         return ODECOL_OK;
     }
     int grid(size_t n) const { return (int)((n + 255) / 256 < 148 * 16 ? (n + 255) / 256 : 148 * 16); }

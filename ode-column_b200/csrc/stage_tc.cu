@@ -1,5 +1,4 @@
 // Family T drivers: forward RK4 stages on the tensor cores and the diagnostic contraction (kernels in stage_tc.cuh).
-#include <cstdio>
 #include <cstdlib>
 #include "stage_tc.cuh"
 
@@ -20,7 +19,6 @@ struct StoreEpi {
             if (j < TNq && b < N) C[(size_t)b * ldc + i] = tot[j];
         }
     }
-    ODECOL_DEVINL void pre_tile(int, int, int, int) const {}
     ODECOL_DEVINL void tile_done(int, int, int, int, int) const {}
 };
 
@@ -40,11 +38,10 @@ static ContractLayout contract_layout(int M, int N, int K) {
 
 
 // initial operand (r_aug at t_ptr[0], split hi/lo), constant-one column + zero padding of the second operand buffer,
-// and the tile-major copies of y0 and r.  One CTA per (padded) trial.
+// and the tile-major copy of y0.  One CTA per (padded) trial.
 __global__ void k_tc_init(DevProblem p, TileGeom tg, const float* __restrict__ y, const float* __restrict__ t_ptr,
                           float* __restrict__ hi0, float* __restrict__ lo0, float* __restrict__ hi1, float* __restrict__ lo1,
-                          float* __restrict__ V0T, float* __restrict__ A0T, float* __restrict__ F0T, float* __restrict__ RT,
-                          int KPa) {
+                          float* __restrict__ V0T, float* __restrict__ A0T, float* __restrict__ F0T, int KPa) {
     const int b = blockIdx.x, N = p.N, Kaug = N + p.n_in + 1;
     const size_t ro = (size_t)b * KPa;
     const int nt = b / tg.TN, g = (b % tg.TN) / tg.TNq, jq = (b % tg.TN) % tg.TNq;
@@ -53,7 +50,7 @@ __global__ void k_tc_init(DevProblem p, TileGeom tg, const float* __restrict__ y
         for (int k = threadIdx.x; k < KPa; k += blockDim.x) { hi0[ro + k] = 0.f; lo0[ro + k] = 0.f; hi1[ro + k] = 0.f; lo1[ro + k] = 0.f; }
         for (int i = threadIdx.x; i < tg.Np; i += blockDim.x) {
             const size_t o = tg.off(nt, g, q, i) + e4;
-            V0T[o] = 0.f; A0T[o] = 0.f; F0T[o] = 0.f; RT[o] = 0.f;
+            V0T[o] = 0.f; A0T[o] = 0.f; F0T[o] = 0.f;
         }
         return;
     }
@@ -75,13 +72,12 @@ __global__ void k_tc_init(DevProblem p, TileGeom tg, const float* __restrict__ y
         const bool in = i < N;
         const float V = in ? yb[i] : 0.f, A = in ? yb[N + i] : 0.f, F = in ? yb[2 * N + i] : 0.f;
         V0T[o] = V; A0T[o] = A; F0T[o] = F;
-        RT[o] = in ? phi_fast(V - A) : 0.f;
     }
 }
 
 struct TcFwdLayout {
     int Np, Bp, KPa, TN, KP16;
-    size_t off_Whi, off_Wlo, off_Rhi[2], off_Rlo[2], off_K[3], off_Y[2], off_RT[4], off_done, off_inv, total;
+    size_t off_Whi, off_Wlo, off_Rhi[2], off_Rlo[2], off_K[3], off_Y[2], off_done, off_inv, total;
     size_t off_W16[2], off_R16[2], off_wscale;      // mixed 16-bit operand format of the persistent forward kernel
 };
 
@@ -98,7 +94,6 @@ static TcFwdLayout tc_fwd_layout(const DevProblem& p) {
     const size_t plane = (size_t)L.Np * L.Bp;
     for (int i = 0; i < 3; ++i) L.off_K[i] = take(plane);            // V slope of stages 1..3
     for (int i = 0; i < 2; ++i) L.off_Y[i] = take(3 * plane);
-    for (int i = 0; i < 4; ++i) L.off_RT[i] = take(plane);           // r of stages 1..4
     L.off_done = take((size_t)(L.Bp / L.TN) + 64);          // one uint32 per trial tile (floats == 4 bytes)
     L.off_inv = take(3ull * p.N + 4);                       // component -> selection position (checkpoint mode) + F flag
     L.KP16 = round_up(p.N + p.n_in + 1, BK16);
@@ -112,14 +107,14 @@ static TcFwdLayout tc_fwd_layout(const DevProblem& p) {
 }  // namespace tc
 
 void tc_launch_init(const DevProblem& p, const tc::TileGeom& tg, const float* y0, const float* t_dev, float* hi0, float* lo0,
-                    float* hi1, float* lo1, float* V0T, float* A0T, float* F0T, float* RT, int KPa, int Bp, cudaStream_t s) {
-    tc::k_tc_init<<<Bp, 128, 0, s>>>(p, tg, y0, t_dev, hi0, lo0, hi1, lo1, V0T, A0T, F0T, RT, KPa);
+                    float* hi1, float* lo1, float* V0T, float* A0T, float* F0T, int KPa, int Bp, cudaStream_t s) {
+    tc::k_tc_init<<<Bp, 128, 0, s>>>(p, tg, y0, t_dev, hi0, lo0, hi1, lo1, V0T, A0T, F0T, KPa);
 }
 
 int tc_rk4_fwd_persistent(const DevProblem& p, const float* t_dev, int T, const float* y0, float* y_out, int out_every,
                           float* Whi, float* Wlo, float* const Rhi[2], float* const Rlo[2], float* const KT[3],
-                          float* const YT[2], float* const RT[4], unsigned int* done, int Np, int Bp, int KPa, int TN,
-                          const tc::CkptView* ck, const tc::Mixed16* mx, cudaStream_t s);
+                          float* const YT[2], unsigned int* done, int Np, int Bp, int KPa, int TN, const tc::CkptView* ck,
+                          const tc::Mixed16* mx, cudaStream_t s);
 
 namespace tc {
 static Mixed16 mixed16_view(const TcFwdLayout& L, char* w) {
@@ -151,7 +146,6 @@ int tc_rk4_fwd(const DevProblem& p, const float* t_dev, int T, const float* y0, 
     float* Rlo[2] = {F(L.off_Rlo[0]), F(L.off_Rlo[1])};
     float* KT[3] = {F(L.off_K[0]), F(L.off_K[1]), F(L.off_K[2])};
     float* YT[2] = {F(L.off_Y[0]), F(L.off_Y[1])};
-    float* RT[4] = {F(L.off_RT[0]), F(L.off_RT[1]), F(L.off_RT[2]), F(L.off_RT[3])};
     const int Kaug = p.N + p.n_in + 1;
     const size_t st = (size_t)p.B * 3 * p.N;
     const TileGeom tg{L.Bp / L.TN, L.Np, L.TN, L.TN / 4};
@@ -159,13 +153,13 @@ int tc_rk4_fwd(const DevProblem& p, const float* t_dev, int T, const float* y0, 
     // persistent kernel keeps the rotating-accumulator scheme that is accurate up to that length
     if (persistent_enabled() && L.KPa / BK <= kChunkMin) {
         const Mixed16 mx = mixed16_view(L, w);
-        return tc_rk4_fwd_persistent(p, t_dev, T, y0, y_out, out_every, Whi, Wlo, Rhi, Rlo, KT, YT, RT,
+        return tc_rk4_fwd_persistent(p, t_dev, T, y0, y_out, out_every, Whi, Wlo, Rhi, Rlo, KT, YT,
                                      reinterpret_cast<unsigned int*>(w + L.off_done), L.Np, L.Bp, L.KPa, L.TN, nullptr, &mx, s);
     }
 
     k_split_pad<<<296, 256, 0, s>>>(p.W_aug, p.N, Kaug, p.ld_w, Whi, Wlo, L.Np, L.KPa);
     k_tc_init<<<L.Bp, 128, 0, s>>>(p, tg, y0, t_dev, Rhi[0], Rlo[0], Rhi[1], Rlo[1], YT[0], YT[0] + tg.plane(),
-                                   YT[0] + 2 * tg.plane(), RT[0], L.KPa);
+                                   YT[0] + 2 * tg.plane(), L.KPa);
     count_launch(2);
     if (cudaMemcpyAsync(y_out, y0, sizeof(float) * st, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
     CUtensorMap mWhi, mWlo, mRhi[2], mRlo[2];
@@ -173,30 +167,9 @@ int tc_rk4_fwd(const DevProblem& p, const float* t_dev, int T, const float* y0, 
     for (int i = 0; i < 2; ++i)
         ok = ok && make_map(&mRhi[i], Rhi[i], L.Bp, L.KPa, L.KPa, L.TN) && make_map(&mRlo[i], Rlo[i], L.Bp, L.KPa, L.KPa, L.TN);
     if (!ok) return ODECOL_E_CUDA;
-    const TileShape ts0{L.Np / BM, L.Bp / L.TN, L.TN, L.KPa / BK, 0, nullptr};
-    // CTA pairs (tcgen05 cta_group::2, ODECOL_PAIR=1): maps of the same operands with half-tile boxes
-    const bool use_pair = pair_enabled() && ts0.MT % 2 == 0;
-    CUtensorMap mRhHi[2], mRhLo[2];
-    for (int i = 0; i < 2 && use_pair; ++i)
-        if (!make_map(&mRhHi[i], Rhi[i], L.Bp, L.KPa, L.KPa, L.TN / 2) || !make_map(&mRhLo[i], Rlo[i], L.Bp, L.KPa, L.KPa, L.TN / 2))
-            return ODECOL_E_CUDA;
+    const TileShape ts{L.Np / BM, L.Bp / L.TN, L.TN, L.KPa / BK, 0};
     int cur = 0;
-    auto launch = [&](auto& e, const TileShape& ts) {
-        return use_pair ? launch_contract_pair(mWhi, mWlo, mRhHi[cur], mRhLo[cur], ts, e, s)
-                        : launch_contract(mWhi, mWlo, mRhi[cur], mRlo[cur], ts, e, s);
-    };
-
-    // diagnostics (compiled in with -DODECOL_DIAG only; the shipped library never allocates, synchronises or skips work):
-    // ODECOL_TIMELINE=1 per-CTA globaltimer stamps of the eight launches of steps 2 and 3, ODECOL_DBG_SKIP partial epilogues
-    unsigned long long* tl_buf = nullptr;
-    int dbg_skip = 0;
-#ifdef ODECOL_DIAG
-    if (getenv("ODECOL_TIMELINE") && T > 5) {
-        cudaMalloc(&tl_buf, sizeof(unsigned long long) * 8 * 148 * 8);
-        cudaMemsetAsync(tl_buf, 0, sizeof(unsigned long long) * 8 * 148 * 8, s);
-    }
-    dbg_skip = getenv("ODECOL_DBG_SKIP") ? atoi(getenv("ODECOL_DBG_SKIP")) : 0;
-#endif
+    auto launch = [&](auto& e) { return launch_contract(mWhi, mWlo, mRhi[cur], mRlo[cur], ts, e, s); };
     for (int n = 0; n < T - 1; ++n) {
         const int j = n + 1;
         const bool emit = (j % out_every == 0) || (j == T - 1);
@@ -208,60 +181,20 @@ int tc_rk4_fwd(const DevProblem& p, const float* t_dev, int T, const float* y0, 
             e.V1T = YT[(n + 1) & 1]; e.A1T = YT[(n + 1) & 1] + pl; e.F1T = YT[(n + 1) & 1] + 2 * pl;
             e.traj_row = emit ? y_out + r * st : nullptr; e.ysel_row = nullptr; e.inv = nullptr; e.G = 0;
             e.K1T = KT[0]; e.K2T = KT[1]; e.K3T = KT[2];
-            for (int q = 0; q < 4; ++q) e.RsT[q] = RT[q];
-            e.store_r = 1; e.Rhi_nxt = Rhi[cur ^ 1]; e.Rlo_nxt = Rlo[cur ^ 1]; e.DRT_nxt = nullptr; e.dbg_skip = dbg_skip;
+            e.Rhi_nxt = Rhi[cur ^ 1]; e.Rlo_nxt = Rlo[cur ^ 1]; e.DRT_nxt = nullptr;
             e.inv_tm = 1.0f / p.c.tau_m; e.inv_ta = 1.0f / p.c.tau_a; e.inv_ts = 1.0f / p.c.tau_s;
             e.t0 = e.t1 = e.dt = 0.f;
         };
         for (int S = 1; S <= 4; ++S) {
             int rc;
-            TileShape ts = ts0;
-            if (tl_buf && n >= 2 && n < 4) ts.dbg = tl_buf + (size_t)((n - 2) * 4 + (S - 1)) * 8 * 148;
-            if (S == 1) { FwdEpiT<1> e; fill(e); rc = launch(e, ts); }
-            else if (S == 2) { FwdEpiT<2> e; fill(e); rc = launch(e, ts); }
-            else if (S == 3) { FwdEpiT<3> e; fill(e); rc = launch(e, ts); }
-            else { FwdEpiT<4> e; fill(e); rc = launch(e, ts); }
+            if (S == 1) { FwdEpiT<1> e; fill(e); rc = launch(e); }
+            else if (S == 2) { FwdEpiT<2> e; fill(e); rc = launch(e); }
+            else if (S == 3) { FwdEpiT<3> e; fill(e); rc = launch(e); }
+            else { FwdEpiT<4> e; fill(e); rc = launch(e); }
             if (rc != ODECOL_OK) return rc;
             cur ^= 1;
         }
     }
-#ifdef ODECOL_DIAG
-    if (tl_buf) {
-        cudaStreamSynchronize(s);
-        static unsigned long long h[8 * 8 * 148];
-        cudaMemcpy(h, tl_buf, sizeof(h), cudaMemcpyDeviceToHost);
-        cudaFree(tl_buf);
-        unsigned long long origin = ~0ull;
-        for (int c = 0; c < 148; ++c) if (h[8 * c] && h[8 * c] < origin) origin = h[8 * c];
-        for (int l = 0; l < 8; ++l) {
-            const unsigned long long* hl = h + (size_t)l * 8 * 148;
-            double seg[6] = {0, 0, 0, 0, 0, 0}, end_mean = 0;
-            unsigned long long s_min = ~0ull, s_max = 0, e_min = ~0ull, e_max = 0;
-            int cnt = 0;
-            for (int c = 0; c < 148; ++c) {
-                const unsigned long long* r = hl + 8 * c;
-                if (!r[0] || !r[6]) continue;
-                ++cnt;
-                for (int k = 0; k < 6; ++k) seg[k] += (double)(r[k + 1] - r[k]);
-                end_mean += (double)(r[6] - origin);
-                if (r[0] < s_min) s_min = r[0];
-                if (r[0] > s_max) s_max = r[0];
-                if (r[6] < e_min) e_min = r[6];
-                if (r[6] > e_max) e_max = r[6];
-            }
-            if (!cnt) continue;
-            if (atoi(getenv("ODECOL_TIMELINE")) >= 2 && l == 4)
-                for (int c = 0; c < 148; ++c) {
-                    const unsigned long long* r = hl + 8 * c;
-                    fprintf(stderr, "[odecol cta] %d sm %llu start %llu ml1 %llu epi1 %llu epi2 %llu end %llu\n", c, r[7], r[0] - s_min,
-                            r[1] - r[0], r[3] - r[2], r[6] - r[5], r[6] - s_min);
-                }
-            fprintf(stderr, "[odecol timeline] step %d stage %d (%d CTAs) ns: start %llu..%llu end %llu..%llu (mean %.0f) | mainloop1 %.0f drain1 %.0f "
-                            "epilogue1 %.0f wait2 %.0f drain2 %.0f epilogue2 %.0f\n", 2 + l / 4, 1 + l % 4, cnt, s_min - origin, s_max - origin,
-                    e_min - origin, e_max - origin, end_mean / cnt, seg[0] / cnt, seg[1] / cnt, seg[2] / cnt, seg[3] / cnt, seg[4] / cnt, seg[5] / cnt);
-        }
-    }
-#endif
     return cudaGetLastError() == cudaSuccess ? ODECOL_OK : ODECOL_E_CUDA;
 }
 
@@ -291,7 +224,6 @@ int tc_rk4_fwd_ckpt(const DevProblem& p, const float* t_dev, int T, const float*
     float* Rlo[2] = {F(L.off_Rlo[0]), F(L.off_Rlo[1])};
     float* KT[3] = {F(L.off_K[0]), F(L.off_K[1]), F(L.off_K[2])};
     float* YT[2] = {F(L.off_Y[0]), F(L.off_Y[1])};
-    float* RT[4] = {F(L.off_RT[0]), F(L.off_RT[1]), F(L.off_RT[2]), F(L.off_RT[3])};
     int* inv = reinterpret_cast<int*>(w + L.off_inv);
     const size_t plane = (size_t)L.Np * L.Bp;
     k_tc_build_inv<<<1, 256, 0, s>>>(sel, G, 3 * p.N, inv);
@@ -300,7 +232,7 @@ int tc_rk4_fwd_ckpt(const DevProblem& p, const float* t_dev, int T, const float*
     CkptView ck;
     ck.VA = static_cast<float*>(ckpt); ck.K = ck.VA + 2 * plane * (size_t)T; ck.y_sel = y_sel; ck.inv = inv; ck.G = G;
     const Mixed16 mx = mixed16_view(L, w);
-    return tc_rk4_fwd_persistent(p, t_dev, T, y0, nullptr, 1, F(L.off_Whi), F(L.off_Wlo), Rhi, Rlo, KT, YT, RT,
+    return tc_rk4_fwd_persistent(p, t_dev, T, y0, nullptr, 1, F(L.off_Whi), F(L.off_Wlo), Rhi, Rlo, KT, YT,
                                  reinterpret_cast<unsigned int*>(w + L.off_done), L.Np, L.Bp, L.KPa, L.TN, &ck, &mx, s);
 }
 
@@ -320,14 +252,8 @@ int tc_contract(const float* A, const float* B, float* C, int M, int N, int K, v
     if (!make_map(&ma_hi, Ahi, L.Mp, L.Kp, L.Kp, BM) || !make_map(&ma_lo, Alo, L.Mp, L.Kp, L.Kp, BM) ||
         !make_map(&mb_hi, Bhi, L.Np, L.Kp, L.Kp, L.TN) || !make_map(&mb_lo, Blo, L.Np, L.Kp, L.Kp, L.TN))
         return ODECOL_E_CUDA;
-    TileShape ts{L.Mp / BM, L.Np / L.TN, L.TN, L.Kp / BK, 0, nullptr};
+    const TileShape ts{L.Mp / BM, L.Np / L.TN, L.TN, L.Kp / BK, 0};
     StoreEpi epi{C, M, N, M};
-    if (pair_enabled() && ts.MT % 2 == 0) {          // CTA pairs (cta_group::2): half trial-tile boxes
-        CUtensorMap mbh_hi, mbh_lo;
-        if (!make_map(&mbh_hi, Bhi, L.Np, L.Kp, L.Kp, L.TN / 2) || !make_map(&mbh_lo, Blo, L.Np, L.Kp, L.Kp, L.TN / 2))
-            return ODECOL_E_CUDA;
-        return launch_contract_pair(ma_hi, ma_lo, mbh_hi, mbh_lo, ts, epi, s);
-    }
     return launch_contract(ma_hi, ma_lo, mb_hi, mb_lo, ts, epi, s);
 }
 

@@ -18,9 +18,22 @@
 #pragma once
 #include <cuda.h>
 #include <cuda_fp16.h>
-#include "stage_common.cuh"
+#include "odecol_common.cuh"
 
 namespace odecol {
+
+constexpr float kOneThirdL = 0.3333333333333333f;
+constexpr float kTwoThirdsL = 0.6666666666666666f;
+
+static inline int round_up(int x, int m) { return (x + m - 1) / m * m; }
+
+ODECOL_DEVINL float4 ld4(const float* p) { return *reinterpret_cast<const float4*>(p); }
+ODECOL_DEVINL void st4(float* p, float4 v) { *reinterpret_cast<float4*>(p) = v; }
+// scratch that is streamed once per launch: L2 only.  (With ~200 KB of the SM's array carved out as shared memory the
+// remaining L1 is too small to hold a line for every outstanding load, and allocating loads stall on it.)
+ODECOL_DEVINL float4 ld4s(const float* p) { return __ldcg(reinterpret_cast<const float4*>(p)); }
+ODECOL_DEVINL void st4s(float* p, float4 v) { __stcg(reinterpret_cast<float4*>(p), v); }
+
 namespace tc {
 
 constexpr int BM = 128;          // populations per tile = TMEM lanes
@@ -171,7 +184,6 @@ struct Mixed16 {
 struct TileShape {
     int MT, NT, TN, KB;      // m tiles, trial tiles, trials per tile (multiple of 16, <= 128), K blocks of 32
     int b_row0;              // first row of the B operand inside its tensor map (stacked per-stage operand buffers)
-    unsigned long long* dbg; // optional per-CTA timeline stamps (globaltimer ns): [cta][8], diagnostics only
 };
 
 ODECOL_DEVINL unsigned int ld_acquire_u32(const unsigned int* p) {
@@ -185,40 +197,12 @@ ODECOL_DEVINL void st_global(float* p, float v) { asm volatile("st.global.f32 [%
 ODECOL_DEVINL void st_global_if(float* p, float v, bool ok) {
     asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.b32 q, %2, 0;\n\t@q st.global.f32 [%0], %1;\n\t}" ::"l"(p), "f"(v), "r"((int)ok) : "memory");
 }
-ODECOL_DEVINL void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
-
-ODECOL_DEVINL unsigned long long gtimer() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-    return t;
-}
-
 constexpr int kMaxQ = 32;    // accumulator columns per epilogue thread = TN / 4 <= 32
-// L2 prefetch of the epilogues' scratch planes, this many groups ahead of the pipelined loads (0 = off, the default).
-// Measured on the C4 step, A/B on one box (scratch/ab_bench.sh, -DODECOL_PREFETCH_AHEAD=2 vs 0): forward 370 vs 352 ms,
-// reverse sweep 626 vs 615 ms -- SLOWER with the prefetch.  The stage passes are bound by L2 throughput, not by the latency
-// of the scratch loads: every extra L2 transaction (and every operand line a prefetched plane evicts) costs more than the
-// shorter load latency buys.
-#ifndef ODECOL_PREFETCH_AHEAD
-#define ODECOL_PREFETCH_AHEAD 0
-#endif
-constexpr bool kPrefetch = ODECOL_PREFETCH_AHEAD > 0;
-// Forward stage epilogues: the rates r_1 .. r_S of the earlier stages of the step (they feed the A and F slopes) are
-// RECOMPUTED from the step's start state and the stored V slopes -- the recurrences of the checkpoint replay -- instead of
-// being kept in four tile-major planes.  A stage pass costs about 1.45 us per byte per element, a phi evaluation about 2 us
-// per pass: dropping the r planes takes the epilogues from 28 / 36 / 44 / 56 to 20 / 24 / 28 / 36 bytes per element.
-// -DODECOL_R_PLANES=1 restores the planes (comparison build).
-#ifndef ODECOL_R_PLANES
-#define ODECOL_R_PLANES 0
-#endif
-constexpr bool kRPlanes = ODECOL_R_PLANES != 0;
-constexpr int kPrefetchAhead = ODECOL_PREFETCH_AHEAD;
 
 // ---------------------------------------------------------------------------------------------------------------
 // the persistent warp-specialised contraction.  Epi supplies
 //   prepare()                                             once per epilogue thread
 //   rows(m_tile, i, n0, nt, g, tot)                       population i, trials n0 + g*TN/4 + [0, TN/4): tot[] = W_aug.r_aug
-//   pre_tile(row, nt, g, TNq)                             per tile, before the accumulator is ready (prefetch only)
 //   tile_done(m_tile, n0, tile_n, etid, nthreads)         per tile, all epilogue threads
 // ---------------------------------------------------------------------------------------------------------------
 // tile -> (population tile, trial tile).  Population tiles are taken in groups of kTileGroupM: consecutive tiles (= the
@@ -282,12 +266,6 @@ k_tc_contract(const __grid_constant__ CUtensorMap mA_hi, const __grid_constant__
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = tmem_base_slot;
-    if (ts.dbg && threadIdx.x == 0) {
-        unsigned int smid;
-        asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-        ts.dbg[blockIdx.x * 8 + 0] = gtimer();
-        ts.dbg[blockIdx.x * 8 + 7] = smid;
-    }
 
     if (warp == kTmaWarp) {
         if (lane == 0) {
@@ -395,7 +373,6 @@ k_tc_contract(const __grid_constant__ CUtensorMap mA_hi, const __grid_constant__
             const int n0 = nt * ts.TN;
             const int row = m_tile * BM + quarter * 32 + lane;
             float tot[kMaxQ];
-            epi.pre_tile(row, nt, g, TNq);            // warm L2 with the first groups' scratch while the contraction runs
             if (chunked) {
                 const uint32_t lb = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(g * TNq);
 #pragma unroll
@@ -435,8 +412,6 @@ k_tc_contract(const __grid_constant__ CUtensorMap mA_hi, const __grid_constant__
             }
             mbar_wait(tfull, tphase);
             tc_fence_after();
-            const int tslot = (tile - blockIdx.x) / gridDim.x;
-            if (ts.dbg && etid == 0 && tslot < 2) ts.dbg[blockIdx.x * 8 + 1 + 3 * tslot] = gtimer();
             const uint32_t lane_base = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(g * TNq);
 #pragma unroll
             for (int q = 0; q < kMaxQ / 4; ++q) {
@@ -458,189 +433,14 @@ k_tc_contract(const __grid_constant__ CUtensorMap mA_hi, const __grid_constant__
             __syncwarp();
             if (lane == 0) mbar_arrive(tempty);        // TMEM is free again: warp 1 may start the next tile
             tphase ^= 1;
-            if (ts.dbg && etid == 0 && tslot < 2) ts.dbg[blockIdx.x * 8 + 2 + 3 * tslot] = gtimer();
             epi.rows(m_tile, row, n0, nt, g, TNq, tot);
             epi.tile_done(m_tile, n0, ts.TN, etid, kEpiWarps * 32);
-            if (ts.dbg && etid == 0 && tslot < 2) ts.dbg[blockIdx.x * 8 + 3 + 3 * tslot] = gtimer();
         }
     }
     tc_fence_before();
     __syncthreads();
     if (warp == kMmaWarp) {
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(ncols) : "memory");
-    }
-}
-
-// ---------------------------------------------------------------------------------------------------------------
-// CTA-pair variant (tcgen05 cta_group::2): the two population tiles 2m, 2m+1 of one trial tile run on the two SMs of a
-// TPC as ONE M = 256 contraction.  Each CTA stages its own W_aug tile and HALF of the trial tile (TN/2 rows), so the
-// operand bytes entering an SM per K block drop from (128 + TN) to (128 + TN/2) rows -- operand ingress is what binds
-// the single-CTA kernel (DESIGN.md section 5).  Protocol:
-//   * both CTAs' TMA loads complete on the LEADER's `full` barrier (mbarrier address with the peer bit cleared); the
-//     leader alone posts arrive.expect_tx with the bytes of both;
-//   * the leader's elected thread issues every tcgen05.mma.cta_group::2 (A / B descriptors name the same shared-memory
-//     offsets in both CTAs) and releases ring slots / publishes accumulators with tcgen05.commit ... multicast::cluster
-//     to the `empty` / `tfull` barriers of both CTAs;
-//   * each CTA keeps its own 128 TMEM lanes x TN columns: the epilogues are those of the single-CTA kernel; the peer's
-//     epilogue warps arrive remotely on the leader's `tempty`.
-// ---------------------------------------------------------------------------------------------------------------
-constexpr int PSTAGES = 4;                      // (32 KB + TN/2 * 256 B) per stage: four stages fit next to the barriers
-constexpr uint32_t kPeerBitMask = 0xFEFFFFFFu;  // shared::cluster address of the same offset in the pair's leader (even) CTA
-
-ODECOL_DEVINL uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-ODECOL_DEVINL void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-ODECOL_DEVINL void tma_load_2d_pair(uint32_t dst, const CUtensorMap* map, uint32_t leader_bar, int c0, int c1) {
-    asm volatile("cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-                 ::"r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(leader_bar), "r"(c0), "r"(c1) : "memory");
-}
-ODECOL_DEVINL void umma_tf32_pair(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-                 ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-ODECOL_DEVINL void umma_commit_pair(uint32_t bar) {
-    const uint16_t mask = 3;
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-                 ::"r"(bar), "h"(mask) : "memory");
-}
-ODECOL_DEVINL void mbar_arrive_leader(uint32_t bar) {
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(bar & kPeerBitMask) : "memory");
-}
-
-template <class Epi>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
-k_tc_contract_pair(const __grid_constant__ CUtensorMap mA_hi, const __grid_constant__ CUtensorMap mA_lo,
-                   const __grid_constant__ CUtensorMap mBh_hi, const __grid_constant__ CUtensorMap mBh_lo, TileShape ts, Epi epi) {
-    extern __shared__ uint8_t smem_raw[];
-    __shared__ __align__(8) uint64_t bars[2 * PSTAGES + 2];
-    __shared__ uint32_t tmem_base_slot;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t rank = cluster_ctarank();
-    const int pair = blockIdx.x >> 1, npairs = gridDim.x >> 1;
-    const uint32_t ring = (smem_u32(smem_raw) + 1023u) & ~1023u;
-    const uint32_t a_bytes = BM * BK * 4, bh_bytes = (uint32_t)(ts.TN >> 1) * BK * 4;     // half of the trial tile per CTA
-    const uint32_t stage_bytes = 2 * a_bytes + 2 * bh_bytes;
-    const uint32_t full0 = smem_u32(&bars[0]), empty0 = smem_u32(&bars[PSTAGES]);
-    const uint32_t tfull = smem_u32(&bars[2 * PSTAGES]), tempty = smem_u32(&bars[2 * PSTAGES + 1]);
-    const int MT2 = ts.MT >> 1;
-    const int tiles = MT2 * ts.NT;
-    const uint32_t acc_stride = (uint32_t)ts.TN;
-    uint32_t ncols = 32;
-    while (ncols < (kMainAcc + 1) * acc_stride) ncols <<= 1;
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < PSTAGES; ++s) { mbar_init(full0 + 8 * s, 1); mbar_init(empty0 + 8 * s, 1); }
-        mbar_init(tfull, 1);
-        mbar_init(tempty, 2 * kEpiWarps);             // the epilogue warps of BOTH CTAs (only the leader's is waited on)
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == kMmaWarp) {
-        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_slot)), "r"(ncols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    cluster_sync_all();
-    tc_fence_after();
-    const uint32_t tmem_base = tmem_base_slot;
-
-    if (warp == kTmaWarp) {
-        if (lane == 0) {
-            int stage = 0; uint32_t phase = 0;
-            for (int tile = pair; tile < tiles; tile += npairs) {
-                const int m0 = (2 * (tile % MT2) + (int)rank) * BM;
-                const int n0 = (tile / MT2) * ts.TN + (int)rank * (ts.TN >> 1);
-                for (int kb = 0; kb < ts.KB; ++kb) {
-                    mbar_wait(empty0 + 8 * stage, phase ^ 1);
-                    const uint32_t base = ring + stage * stage_bytes;
-                    const uint32_t fb = (full0 + 8 * stage) & kPeerBitMask;      // the leader's barrier collects both CTAs' bytes
-                    if (rank == 0) mbar_expect_tx(full0 + 8 * stage, 2 * stage_bytes);
-                    tma_load_2d_pair(base, &mA_hi, fb, kb * BK, m0);
-                    tma_load_2d_pair(base + a_bytes, &mA_lo, fb, kb * BK, m0);
-                    tma_load_2d_pair(base + 2 * a_bytes, &mBh_hi, fb, kb * BK, n0 + ts.b_row0);
-                    tma_load_2d_pair(base + 2 * a_bytes + bh_bytes, &mBh_lo, fb, kb * BK, n0 + ts.b_row0);
-                    if (++stage == PSTAGES) { stage = 0; phase ^= 1; }
-                }
-            }
-        }
-    } else if (warp == kMmaWarp) {
-        if (lane == 0 && rank == 0) {
-            // M = 256 across the pair: (256 >> 4) at [24, 29)
-            const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(ts.TN >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
-            const uint32_t d_small = tmem_base + kMainAcc * acc_stride;
-            int stage = 0; uint32_t phase = 0, tphase = 0;
-            for (int tile = pair; tile < tiles; tile += npairs) {
-                mbar_wait(tempty, tphase ^ 1);
-                tc_fence_after();
-                int j = 0;
-                for (int kb = 0; kb < ts.KB; ++kb) {
-                    mbar_wait(full0 + 8 * stage, phase);
-                    tc_fence_after();
-                    const uint32_t base = ring + stage * stage_bytes;
-                    const uint64_t a_hi = make_smem_desc(base), a_lo = make_smem_desc(base + a_bytes);
-                    const uint64_t b_hi = make_smem_desc(base + 2 * a_bytes), b_lo = make_smem_desc(base + 2 * a_bytes + bh_bytes);
-#pragma unroll
-                    for (int k = 0; k < BK / 8; ++k, ++j) {
-                        const uint64_t adv = (uint64_t)(k * 32 >> 4);
-                        umma_tf32_pair(d_small, a_lo + adv, b_hi + adv, idesc, j != 0);
-                        umma_tf32_pair(d_small, a_hi + adv, b_lo + adv, idesc, 1);
-                        umma_tf32_pair(tmem_base + (uint32_t)(j % kMainAcc) * acc_stride, a_hi + adv, b_hi + adv, idesc, j >= kMainAcc);
-                    }
-                    umma_commit_pair(empty0 + 8 * stage);
-                    if (++stage == PSTAGES) { stage = 0; phase ^= 1; }
-                }
-                umma_commit_pair(tfull);
-                tphase ^= 1;
-            }
-        }
-    } else if (warp >= kEpiWarp0) {
-        const int ew = warp - kEpiWarp0;
-        const int quarter = warp & 3;
-        const int g = ew >> 2;
-        const int etid = ew * 32 + lane;
-        const int TNq = ts.TN >> 2;
-        epi.prepare();
-        uint32_t tphase = 0;
-        for (int tile = pair; tile < tiles; tile += npairs) {
-            const int m_tile = 2 * (tile % MT2) + (int)rank, nt = tile / MT2, n0 = nt * ts.TN;
-            const int row = m_tile * BM + quarter * 32 + lane;
-            float tot[kMaxQ];
-            epi.pre_tile(row, nt, g, TNq);
-            mbar_wait(tfull, tphase);
-            tc_fence_after();
-            const uint32_t lane_base = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(g * TNq);
-#pragma unroll
-            for (int q = 0; q < kMaxQ / 4; ++q) {
-                if (4 * q < TNq) {
-                    uint32_t u[kMainAcc + 1][4];
-#pragma unroll
-                    for (int a = 0; a <= kMainAcc; ++a) tmem_ld4_issue(lane_base + a * acc_stride + 4 * q, u[a]);
-                    tmem_ld_wait();
-#pragma unroll
-                    for (int e = 0; e < 4; ++e) {
-                        float sum = __uint_as_float(u[kMainAcc][e]);
-#pragma unroll
-                        for (int a = 0; a < kMainAcc; ++a) sum += __uint_as_float(u[a][e]);
-                        tot[4 * q + e] = sum;
-                    }
-                }
-            }
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive_leader(tempty);
-            tphase ^= 1;
-            epi.rows(m_tile, row, n0, nt, g, TNq, tot);
-            epi.tile_done(m_tile, n0, ts.TN, etid, kEpiWarps * 32);
-        }
-    }
-    tc_fence_before();
-    cluster_sync_all();           // the peer's shared memory and barriers stay alive until the leader's last MMA / commit landed
-    if (warp == kMmaWarp) {
-        asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(ncols) : "memory");
     }
 }
 
@@ -728,12 +528,7 @@ static int launch_contract(const CUtensorMap& a_hi, const CUtensorMap& a_lo, con
     }
     const int tiles = ts.MT * ts.NT;
     const int grid = tiles < num_sms() ? tiles : num_sms();
-#ifdef ODECOL_DIAG
-    static const int nochunk = getenv("ODECOL_NOCHUNK") ? atoi(getenv("ODECOL_NOCHUNK")) : 0;    // accuracy comparison only
-#else
-    constexpr int nochunk = 0;
-#endif
-    if (ts.KB > kChunkMin && !nochunk) k_tc_contract<Epi, true><<<grid, kThreads, smem, s>>>(a_hi, a_lo, b_hi, b_lo, ts, epi);
+    if (ts.KB > kChunkMin) k_tc_contract<Epi, true><<<grid, kThreads, smem, s>>>(a_hi, a_lo, b_hi, b_lo, ts, epi);
     else k_tc_contract<Epi, false><<<grid, kThreads, smem, s>>>(a_hi, a_lo, b_hi, b_lo, ts, epi);
     count_launch();
     return cudaGetLastError() == cudaSuccess ? ODECOL_OK : ODECOL_E_CUDA;
@@ -755,31 +550,6 @@ static int launch_contract16(const CUtensorMap& a_hi, const CUtensorMap& a_lo, c
     const int grid = tiles < num_sms() ? tiles : num_sms();
     if (ts.KB > kChunkMin / 2) k_tc_contract<Epi, true, true><<<grid, kThreads, smem, s>>>(a_hi, a_lo, b_hi, b_lo, ts, epi);
     else k_tc_contract<Epi, false, true><<<grid, kThreads, smem, s>>>(a_hi, a_lo, b_hi, b_lo, ts, epi);
-    count_launch();
-    return cudaGetLastError() == cudaSuccess ? ODECOL_OK : ODECOL_E_CUDA;
-}
-
-// pair launch: bh_* are maps of the SAME operand with a box of TN/2 rows.  Needs an even number of population tiles.
-inline bool pair_enabled() {
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("ODECOL_PAIR"); v = e ? (atoi(e) != 0) : 0; }
-    return v != 0;
-}
-
-template <class Epi>
-static int launch_contract_pair(const CUtensorMap& a_hi, const CUtensorMap& a_lo, const CUtensorMap& bh_hi, const CUtensorMap& bh_lo,
-                                const TileShape& ts, const Epi& epi, cudaStream_t s) {
-    if ((ts.MT & 1) || (ts.TN & 15)) return ODECOL_E_UNSUPPORTED;
-    const size_t smem = (size_t)PSTAGES * (2 * BM * BK * 4 + 2 * (size_t)(ts.TN / 2) * BK * 4) + 1024;
-    static bool configured = false;
-    if (!configured) {
-        if (cudaFuncSetAttribute(k_tc_contract_pair<Epi>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess)
-            return ODECOL_E_CUDA;
-        configured = true;
-    }
-    const int tiles = (ts.MT / 2) * ts.NT;
-    const int pairs = tiles < num_sms() / 2 ? tiles : num_sms() / 2;
-    k_tc_contract_pair<Epi><<<2 * pairs, kThreads, smem, s>>>(a_hi, a_lo, bh_hi, bh_lo, ts, epi);
     count_launch();
     return cudaGetLastError() == cudaSuccess ? ODECOL_OK : ODECOL_E_CUDA;
 }
@@ -1004,10 +774,13 @@ ODECOL_DEVINL void stimulus_columns16(const DevProblem& p, int KP16, size_t plan
 }
 
 // Forward stage epilogue (3/8 rule, reference step: torchdiffeq rk_common.py rk4_alt_step_func).  Only what cannot be
-// recomputed crosses a stage boundary through HBM: the V slope of each stage (it carries the contraction) and r of each
-// stage.  The A and F slopes are linear in r, so every stage re-derives them in registers from A0 / F0 and r_1..r_S with
-// the same expressions, in the same order, as a kernel that had stored them; F is only touched at stage 4.
-// Bytes per (population, trial): 28 / 36 / 44 / 64 (+12 trajectory) for stages 1..4.
+// recomputed crosses a stage boundary through HBM: the V slope of each stage (it carries the contraction).  The rates
+// r_1 .. r_S of the earlier stages are recomputed from the step's start state and the stored V slopes -- the recurrences
+// of the checkpoint replay -- and the A and F slopes, linear in r, are re-derived in registers from A0 / F0 and r_1..r_S
+// with the same expressions, in the same order, as a kernel that had stored them; F is only touched at stage 4.  A stage
+// pass costs about 1.45 us per byte per element, a phi evaluation about 2 us per pass: recomputing r instead of keeping
+// it in four planes takes the epilogues from 28 / 36 / 44 / 56 to 20 / 24 / 28 / 36 bytes per element (stages 1..4,
+// +12 for the trajectory).
 template <int S, bool F16 = false>      // F16: the next operand is written in the 16-bit format (two FP16 planes)
 struct FwdEpiT {
     DevProblem p;
@@ -1025,11 +798,8 @@ struct FwdEpiT {
     const int* inv;        // [3N] component -> position in the selection, -1 if not selected (with ysel_row)
     int G;
     float* K1T; float* K2T; float* K3T;     // [1 plane] each: V slope of stages 1..3
-    float* RsT[4];         // [1 plane] each: r of stages 1..4; stage S reads 0..S-1 and writes r of the next stage to S % 4
-    int store_r;           // 0: the next stage's r plane is not needed (last recomputed stage of the reverse sweep)
     float* Rhi_nxt; float* Rlo_nxt;         // [Bp][KPa] operand of the next contraction
     float* DRT_nxt;        // optional [1 plane]: phi'(x) of the next stage state (reverse-sweep recompute)
-    int dbg_skip;          // diagnostics: 1 skip trajectory stores, 2 skip operand stores, 4 skip phi, 8 skip all stores
     float inv_tm, inv_ta, inv_ts;
     float t0, t1, dt;
     int needF;             // stage 4: advance F (always, except in checkpoint mode when no F component is selected)
@@ -1042,29 +812,12 @@ struct FwdEpiT {
     }
 
     // One float4 group (4 trials) of population i: what stage S reads from the scratch planes.
-    struct Group { float4 V0, A0, R1, k1V, R2, k2V, R3, k3V, R4, F0; };
+    struct Group { float4 V0, A0, k1V, k2V, k3V, F0; };
     ODECOL_DEVINL void load_group(Group& L, size_t oq) const {
         L.V0 = ld4s(V0T + oq); L.A0 = ld4s(A0T + oq);
-        if (kRPlanes) L.R1 = ld4s(RsT[0] + oq);
-        if (S >= 2) { L.k1V = ld4s(K1T + oq); if (kRPlanes) L.R2 = ld4s(RsT[1] + oq); }
-        if (S >= 3) { L.k2V = ld4s(K2T + oq); if (kRPlanes) L.R3 = ld4s(RsT[2] + oq); }
-        if (S >= 4) { L.k3V = ld4s(K3T + oq); if (kRPlanes) L.R4 = ld4s(RsT[3] + oq); if (needF) L.F0 = ld4s(F0T + oq); }
-    }
-    // L2 prefetch of what load_group(oq) will read: the planes were written one stage pass (tens of microseconds, several
-    // hundred MB of traffic) ago and are mostly back in HBM; a prefetch two groups ahead turns the demand loads of the
-    // pipelined loop into L2 hits without holding registers (the loop keeps ONE group in flight in registers).
-    ODECOL_DEVINL void prefetch_group(size_t oq) const {
-        prefetch_l2(V0T + oq); prefetch_l2(A0T + oq);
-        if (S >= 2) prefetch_l2(K1T + oq);
-        if (S >= 3) prefetch_l2(K2T + oq);
-        if (S >= 4) { prefetch_l2(K3T + oq); if (needF) prefetch_l2(F0T + oq); }
-    }
-    // before the tile's accumulator is ready: the first groups of this thread
-    ODECOL_DEVINL void pre_tile(int i, int nt, int g, int TNq) const {
-        if (i >= p.N || !kPrefetch) return;
-        const size_t o0 = tg.off(nt, g, 0, i), qstride = (size_t)tg.Np * 4;
-        const int nq = TNq >> 2;
-        for (int q = 0; q < kPrefetchAhead + 1 && q < nq; ++q) prefetch_group(o0 + q * qstride);
+        if (S >= 2) L.k1V = ld4s(K1T + oq);
+        if (S >= 3) L.k2V = ld4s(K2T + oq);
+        if (S >= 4) { L.k3V = ld4s(K3T + oq); if (needF) L.F0 = ld4s(F0T + oq); }
     }
 
     // The group loop is rolled (its body is ~1000 instructions; seven unrolled copies missed the instruction cache) and
@@ -1087,8 +840,7 @@ struct FwdEpiT {
             const size_t oq = o0 + q * qstride;
             const Group L = nxt;
             if (q + 1 < nq) load_group(nxt, oq + qstride);
-            if (kPrefetch && q + 1 + kPrefetchAhead < nq) prefetch_group(oq + (1 + kPrefetchAhead) * qstride);
-            const float4 &V0 = L.V0, &A0 = L.A0, &R1 = L.R1, &R2 = L.R2, &R3 = L.R3, &R4 = L.R4, &F0 = L.F0;
+            const float4 &V0 = L.V0, &A0 = L.A0, &F0 = L.F0;
             const float4 &k1V = L.k1V, &k2V = L.k2V, &k3V = L.k3V;
             const int q4 = 4 * q;
             float oKV[4], oNV[4], oNA[4], oNF[4], oR[4], oD[4];
@@ -1096,26 +848,25 @@ struct FwdEpiT {
             for (int e = 0; e < 4; ++e) {
                 const float v0 = (&V0.x)[e], a0 = (&A0.x)[e];
                 // A (and at stage 4 F) slopes of the earlier stages, re-derived from the rates r_1 .. r_{S-1}; the rates
-                // themselves from the stage states (kRPlanes: from their planes), which follow from V0, A0 and the V slopes
+                // themselves from the stage states, which follow from V0, A0 and the V slopes
                 float k1A = 0.f, k2A = 0.f, k3A = 0.f, A = a0, V = v0;
-                float r1 = 0.f, r2 = 0.f, r3 = 0.f, r;
-                if (kRPlanes) { r1 = (&R1.x)[e]; r2 = (&R2.x)[e]; r3 = (&R3.x)[e]; }
-                else r1 = phi_fast(v0 - a0);
-                r = r1;
+                float r2 = 0.f, r3 = 0.f;
+                const float r1 = phi_fast(v0 - a0);
+                float r = r1;
                 if (S >= 2) {
                     k1A = (kap * r1 - a0) * inv_ta;
                     const float v2 = v0 + dt * (&k1V.x)[e] * third, a2 = a0 + dt * k1A * third;
-                    if (!kRPlanes) r2 = phi_fast(v2 - a2);
+                    r2 = phi_fast(v2 - a2);
                     if (S == 2) { V = v2; A = a2; r = r2; }
                     if (S >= 3) {
                         k2A = (kap * r2 - a2) * inv_ta;
                         const float v3 = v0 + dt * ((&k2V.x)[e] - (&k1V.x)[e] * third), a3 = a0 + dt * (k2A - k1A * third);
-                        if (!kRPlanes) r3 = phi_fast(v3 - a3);
+                        r3 = phi_fast(v3 - a3);
                         if (S == 3) { V = v3; A = a3; r = r3; }
                         if (S >= 4) {
                             k3A = (kap * r3 - a3) * inv_ta;
                             V = v0 + dt * ((&k1V.x)[e] - (&k2V.x)[e] + (&k3V.x)[e]); A = a0 + dt * (k1A - k2A + k3A);
-                            r = kRPlanes ? (&R4.x)[e] : phi_fast(V - A);
+                            r = phi_fast(V - A);
                         }
                     }
                 }
@@ -1144,9 +895,8 @@ struct FwdEpiT {
                 }
                 oNV[e] = nV; oNA[e] = nA; oNF[e] = nF;
                 if (DRT_nxt) phi_dphi_fast(nV - nA, oR[e], oD[e]);
-                else oR[e] = (dbg_skip & 4) ? (nV - nA) : phi_fast(nV - nA);
+                else oR[e] = phi_fast(nV - nA);
             }
-            if (dbg_skip & 8) continue;
             if (DRT_nxt) st4s(DRT_nxt + oq, make_float4(oD[0], oD[1], oD[2], oD[3]));
             const float4 kV4 = make_float4(oKV[0], oKV[1], oKV[2], oKV[3]);
             if (S == 1) st4s(K1T + oq, kV4);
@@ -1157,13 +907,12 @@ struct FwdEpiT {
                 st4s(A1T + oq, make_float4(oNA[0], oNA[1], oNA[2], oNA[3]));
                 if (needF) st4s(F1T + oq, make_float4(oNF[0], oNF[1], oNF[2], oNF[3]));
             }
-            if (kRPlanes && store_r) st4s(RsT[S & 3] + oq, make_float4(oR[0], oR[1], oR[2], oR[3]));
             // operand rows of the next contraction: one 64-bit row address per group, the other seven stores at fixed
             // offsets from it, predicated (the branchy form spent ~27 instructions per element on these two stores)
             const int b0 = n0 + g * TNq + q4;
             float* rh = Rhi_nxt + (size_t)b0 * KPa + i;
             const ptrdiff_t lo_off = Rlo_nxt - Rhi_nxt;
-            float* yr = (S == 4 && traj_row && !(dbg_skip & 1)) ? traj_row + (size_t)b0 * 3 * N + i : nullptr;
+            float* yr = (S == 4 && traj_row) ? traj_row + (size_t)b0 * 3 * N + i : nullptr;
             uint16_t* r16 = F16 ? R16_nxt + (size_t)b0 * KP16 + i : nullptr;
 #pragma unroll
             for (int e = 0; e < 4; ++e) {
@@ -1174,7 +923,7 @@ struct FwdEpiT {
                     st_global_u16_if(ph, t2.h, ok);
                     st_global_u16_if(ph + r16_plane, t2.l, ok);
                     if (ok && !(fabsf(oR[e]) <= kF16Limit)) *ovf = 1u;
-                } else if (!(dbg_skip & 2)) {
+                } else {
                     const float h = tf32_rna(oR[e]);
                     float* ph = rh + (size_t)e * KPa;
                     st_global_if(ph, h, ok);

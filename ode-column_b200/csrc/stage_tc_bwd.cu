@@ -11,7 +11,7 @@ namespace odecol {
 namespace tc {
 
 // ---------------------------------------------------------------------------------------------------------------
-// reverse stage epilogue.  S = 4, 3, 2, 1: the stage whose Jacobian is applied (same algebra as stage_bwd.cu)
+// reverse stage epilogue.  S = 4, 3, 2, 1: the stage whose Jacobian is applied
 // ---------------------------------------------------------------------------------------------------------------
 // The F component never feeds back into the dynamics, so its adjoint within a step is a fixed linear chain of lambda_F:
 // every stage re-derives its own kbar_F from lambda_F in registers (same expressions a stored version would use) and no
@@ -63,20 +63,6 @@ struct BwdEpiT {
             }
         }
     }
-    ODECOL_DEVINL void prefetch_group(size_t oq, size_t pl) const {      // see FwdEpiT::prefetch_group
-        prefetch_l2(DRT + oq); prefetch_l2(lamT + oq); prefetch_l2(lamT + pl + oq);
-        if (needF) prefetch_l2(lamT + 2 * pl + oq);
-        if (S == 1) { prefetch_l2(acurT + oq); prefetch_l2(acurT + pl + oq); }
-        if (S <= 3) { prefetch_l2(b4T + oq); prefetch_l2(b4T + pl + oq); }
-        if (S == 2) { prefetch_l2(b3T + oq); prefetch_l2(b3T + pl + oq); }
-    }
-    ODECOL_DEVINL void pre_tile(int j, int nt, int g, int TNq) const {
-        if (j >= p.N || !kPrefetch) return;
-        const size_t o0 = tg.off(nt, g, 0, j), qstride = (size_t)tg.Np * 4, pl = tg.plane();
-        const int nq = TNq >> 2;
-        for (int q = 0; q < kPrefetchAhead + 1 && q < nq; ++q) prefetch_group(o0 + q * qstride, pl);
-    }
-
     // rolled, software-pipelined group loop (see FwdEpiT::rows)
     ODECOL_DEVINL void rows(int, int j, int n0, int nt, int g, int TNq, const float (&graw)[kMaxQ]) const {
         if (j >= p.N) return;
@@ -97,7 +83,6 @@ struct BwdEpiT {
             const size_t oq = o0 + q * qstride;
             const Group L = nxt;
             if (q + 1 < nq) load_group(nxt, oq + qstride, pl, bg + 4 * (q + 1), gV, gA, gF);
-            if (kPrefetch && q + 1 + kPrefetchAhead < nq) prefetch_group(oq + (1 + kPrefetchAhead) * qstride, pl);
             float nV[4], nA[4], sV[4], sA[4], sF[4];
 #pragma unroll
             for (int e = 0; e < 4; ++e) {
@@ -181,8 +166,7 @@ struct BwdEpiT {
 constexpr int DW_BK = 32;        // rows (trials) per K block = four 8-row swizzle atoms
 constexpr int DW_T = 128;        // output tile: 128 x 128
 struct DwShape { int MT, NT, Z, rows_per_split, total_rows, N, Kaug, ld_w; float* grad_W; uint32_t lbo, sbo, major_bits, kadv;
-                 int two_products;        // 1: drop the A_hi . B_lo term and never stage B_lo (experiment, ODECOL_DW_2X=1)
-                 float* partial; };       // [Z][N][ld_w] or NULL: row split z accumulates into its OWN copy with plain
+                 float* partial; };             // [Z][N][ld_w] or NULL: row split z accumulates into its OWN copy with plain
                                           // read-modify-writes (one CTA per (tile, z) and launch, launches stream-ordered), summed
                                           // over z in a fixed order at the end of the sweep -- bit-reproducible, no float atomics
 ODECOL_DEVINL uint64_t make_smem_desc_mn(uint32_t smem_addr, uint32_t lbo, uint32_t sbo) {
@@ -208,8 +192,7 @@ struct BwdChainArgs {
     const float* grad_y; const int* inv;
     float gamma, inv_tm, inv_ta, inv_ts;
     unsigned int* done; unsigned int done_base;
-    int fuse_dw;               // 1: run the dW contraction of this step as a fifth phase (maps dA_* / dB_*, shape ds)
-    DwShape ds;
+    DwShape ds;                // FUSE_DW: the dW contraction of this step, run as a fifth phase (maps dA_* / dB_*)
 };
 
 template <int S>
@@ -225,14 +208,6 @@ ODECOL_DEVINL void chain_epilogue(const BwdChainArgs& a, int m_tile, int row, in
     e.inv_tm = a.inv_tm; e.inv_ta = a.inv_ta; e.inv_ts = a.inv_ts;
     e.prepare();
     e.rows(m_tile, row, n0, nt, g, TNq, tot);
-}
-
-template <int S>
-ODECOL_DEVINL void chain_pre_tile(const BwdChainArgs& a, int row, int nt, int g, int TNq) {
-    BwdEpiT<S> e;
-    e.p = a.p; e.tg = a.tg; e.acurT = a.acurT; e.lamT = a.lamT; e.b4T = a.b4T; e.b3T = a.b3T; e.DRT = a.DRT[S - 1];
-    e.needF = __ldg(a.inv + 3 * a.p.N);
-    e.pre_tile(row, nt, g, TNq);
 }
 
 template <bool FUSE_DW>
@@ -336,14 +311,13 @@ k_tc_bwd_chain(const __grid_constant__ CUtensorMap mW_hi, const __grid_constant_
                     const int row = r0 + kb * DW_BK;
                     mbar_wait(empty0 + 8 * stage, phase ^ 1);
                     const uint32_t base = ring + stage * stride, fb = full0 + 8 * stage;
-                    mbar_expect_tx(fb, ds.two_products ? 3 * dw_op : dw_stage);
-                    const int arow = row;                             // dA_* are the maps of this step's operand set
+                    mbar_expect_tx(fb, dw_stage);
 #pragma unroll
-                    for (int m = 0; m < 4; ++m) {
-                        tma_load_2d(base + m * dw_box, &dA_hi, fb, i0 + 32 * m, arow);
-                        tma_load_2d(base + dw_op + m * dw_box, &dA_lo, fb, i0 + 32 * m, arow);
+                    for (int m = 0; m < 4; ++m) {                     // dA_* are the maps of this step's operand set
+                        tma_load_2d(base + m * dw_box, &dA_hi, fb, i0 + 32 * m, row);
+                        tma_load_2d(base + dw_op + m * dw_box, &dA_lo, fb, i0 + 32 * m, row);
                         tma_load_2d(base + 2 * dw_op + m * dw_box, &dB_hi, fb, k0 + 32 * m, row);
-                        if (!ds.two_products) tma_load_2d(base + 3 * dw_op + m * dw_box, &dB_lo, fb, k0 + 32 * m, row);
+                        tma_load_2d(base + 3 * dw_op + m * dw_box, &dB_lo, fb, k0 + 32 * m, row);
                     }
                     if (++stage == STAGES) { stage = 0; phase ^= 1; }
                 }
@@ -402,7 +376,7 @@ k_tc_bwd_chain(const __grid_constant__ CUtensorMap mW_hi, const __grid_constant_
                     for (int k = 0; k < DW_BK / 8; ++k, ++j) {
                         const uint64_t adv = (uint64_t)((k * ds.kadv) >> 4);
                         umma_tf32(d_small_dw, a_lo + adv, b_hi + adv, idesc_dw, j != 0);
-                        if (!ds.two_products) umma_tf32(d_small_dw, a_hi + adv, b_lo + adv, idesc_dw, 1);
+                        umma_tf32(d_small_dw, a_hi + adv, b_lo + adv, idesc_dw, 1);
                         umma_tf32(tmem_base + (uint32_t)(j % kMainAcc) * DW_T, a_hi + adv, b_hi + adv, idesc_dw, j >= kMainAcc);
                     }
                     umma_commit(empty0 + 8 * stage);
@@ -425,12 +399,6 @@ k_tc_bwd_chain(const __grid_constant__ CUtensorMap mW_hi, const __grid_constant_
                 const int m_tile = tile % ts.MT, nt = tile / ts.MT, n0 = nt * ts.TN;
                 const int row = m_tile * BM + quarter * 32 + lane;
                 float tot[kMaxQ];
-                switch (q) {                       // warm L2 with this thread's first scratch groups while the tile is contracted
-                    case 0: chain_pre_tile<4>(a, row, nt, g, TNq); break;
-                    case 1: chain_pre_tile<3>(a, row, nt, g, TNq); break;
-                    case 2: chain_pre_tile<2>(a, row, nt, g, TNq); break;
-                    default: chain_pre_tile<1>(a, row, nt, g, TNq); break;
-                }
                 mbar_wait(tfull, tphase);
                 tc_fence_after();
                 const uint32_t lane_base = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(g * TNq);
@@ -506,12 +474,12 @@ k_tc_bwd_chain(const __grid_constant__ CUtensorMap mW_hi, const __grid_constant_
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// per-step operand setup: y_traj[n] (API layout) -> tile-major Y0T, r / phi' of stage 1, split operand with stimulus
+// per-step operand setup: y_traj[n] (API layout) -> tile-major Y0T, phi' of stage 1, split operand with stimulus
 // One CTA per group of four trials (one float4 of the tile-major layout), threads over populations.
 // ---------------------------------------------------------------------------------------------------------------
 __global__ void k_tc_step_begin(DevProblem p, TileGeom tg, const float* __restrict__ y, const float* __restrict__ t_ptr,
                                 float* __restrict__ hi0, float* __restrict__ lo0, float* __restrict__ Y0T,
-                                float* __restrict__ RT, float* __restrict__ DRT, int KPa) {
+                                float* __restrict__ DRT, int KPa) {
     const int b4 = blockIdx.x * 4, N = p.N;
     const int nt = b4 / tg.TN, g = (b4 % tg.TN) / tg.TNq, q = ((b4 % tg.TN) % tg.TNq) >> 2;
     const size_t pl = tg.plane();
@@ -535,7 +503,6 @@ __global__ void k_tc_step_begin(DevProblem p, TileGeom tg, const float* __restri
         st4(Y0T + o, make_float4(V[0], V[1], V[2], V[3]));
         st4(Y0T + pl + o, make_float4(A[0], A[1], A[2], A[3]));
         st4(Y0T + 2 * pl + o, make_float4(F[0], F[1], F[2], F[3]));
-        st4(RT + o, make_float4(R[0], R[1], R[2], R[3]));
         if (DRT) st4(DRT + o, make_float4(D[0], D[1], D[2], D[3]));
     }
     // stimulus channels, constant-one column
@@ -554,43 +521,26 @@ __global__ void k_tc_step_begin(DevProblem p, TileGeom tg, const float* __restri
 
 // checkpoint mode: every stage operand and phi' of step n from the saved V/A state and V slopes -- the forward stage
 // recurrences of FwdEpiT, elementwise, no contraction.  Work unit = (group of four trials, slice of 128 populations), done by
-// 128 threads: the stand-alone kernel below walks all slices of one trial group per CTA; the dW contraction kernel hands
-// units of the NEXT step to its epilogue warps, which idle between accumulator drains (ReplayJob).
+// 128 threads; one CTA walks all slices of one trial group.
 struct ReplayJob {
-    int valid;                 // 0: nothing to replay
     DevProblem p; TileGeom tg;
     const float* VA; const float* KV; const float* t;
-    int n, KPa, nblocks, slices;             // step, operand row length, trial groups (Bp / 4), population slices (Np / 128)
-    float* Rhi; float* Rlo; size_t rstride;  // four stacked operand buffers of the step's set
-    float* D[4];                             // phi' planes of the step's set
+    int n, KPa, slices;                      // step, operand row length, population slices (Np / 128)
+    float* Rhi; float* Rlo; size_t rstride;  // the four stacked operand buffers
+    float* D[4];                             // the four phi' planes
 };
 
-// the checkpoint values one thread needs for one unit: loaded ahead of their use where the caller pipelines units
-struct ReplayLoad { float4 V0, A0, k1V, k2V, k3V; };
-
-ODECOL_DEVINL size_t replay_offset(const ReplayJob& j, int blk, int i) {
-    const int b4 = blk * 4;
-    const TileGeom& tg = j.tg;
-    return tg.off(b4 / tg.TN, (b4 % tg.TN) / tg.TNq, ((b4 % tg.TN) % tg.TNq) >> 2, i);
-}
-
-ODECOL_DEVINL void replay_load(const ReplayJob& j, int blk, int slice, int tid, ReplayLoad& L) {
-    const int i = slice * 128 + tid;
-    if (i >= j.p.N) return;
-    const size_t o = replay_offset(j, blk, i), pl = j.tg.plane();
-    L.V0 = ld4s(j.VA + o); L.A0 = ld4s(j.VA + pl + o);
-    L.k1V = ld4s(j.KV + o); L.k2V = ld4s(j.KV + pl + o); L.k3V = ld4s(j.KV + 2 * pl + o);
-}
-
-ODECOL_DEVINL void replay_compute(const ReplayJob& j, int blk, int slice, int tid, const ReplayLoad& L) {
+ODECOL_DEVINL void replay_unit(const ReplayJob& j, int blk, int slice, int tid) {
     const DevProblem& p = j.p;
+    const TileGeom& tg = j.tg;
     const int b4 = blk * 4, N = p.N;
     const float t0 = __ldg(j.t + j.n), t1 = __ldg(j.t + j.n + 1), dt = __fsub_rn(t1, t0);
     const float third = kOneThirdL, inv_ta = 1.0f / p.c.tau_a;
     const int i = slice * 128 + tid;
     if (i < N) {
-        const size_t o = replay_offset(j, blk, i);
-        const float4 &V0 = L.V0, &A0 = L.A0, &k1V = L.k1V, &k2V = L.k2V, &k3V = L.k3V;
+        const size_t o = tg.off(b4 / tg.TN, (b4 % tg.TN) / tg.TNq, ((b4 % tg.TN) % tg.TNq) >> 2, i), pl = tg.plane();
+        const float4 V0 = ld4s(j.VA + o), A0 = ld4s(j.VA + pl + o);
+        const float4 k1V = ld4s(j.KV + o), k2V = ld4s(j.KV + pl + o), k3V = ld4s(j.KV + 2 * pl + o);
         const float kap = __ldg(p.kappa + i);
         float R[4][4], D[4][4];
 #pragma unroll
@@ -632,13 +582,7 @@ ODECOL_DEVINL void replay_compute(const ReplayJob& j, int blk, int slice, int ti
     stimulus_columns(p, j.KPa, idx, tcl, b4, 4, 0, 1, tid & 31, 32, j.Rhi + s * j.rstride, j.Rlo + s * j.rstride);
 }
 
-ODECOL_DEVINL void replay_unit(const ReplayJob& j, int blk, int slice, int tid) {
-    ReplayLoad L;
-    replay_load(j, blk, slice, tid, L);
-    replay_compute(j, blk, slice, tid, L);
-}
-
-// stand-alone: one CTA of 128 threads per group of four trials
+// one CTA of 128 threads per group of four trials
 __global__ void __launch_bounds__(128, 8) k_tc_replay(ReplayJob j) {
     for (int slice = 0; slice < j.slices; ++slice) replay_unit(j, blockIdx.x, slice, threadIdx.x);
 }
@@ -728,11 +672,9 @@ __global__ void k_tc_set_one(float* __restrict__ Rhi, int Bp, int B, int KPa, in
 #endif
 constexpr int DW_CHUNK = ODECOL_DW_CHUNK;
 
-template <bool TWO, bool REPLAY>
 __global__ void __launch_bounds__(kThreads, 1)
 k_tc_dw(const __grid_constant__ CUtensorMap mA_hi, const __grid_constant__ CUtensorMap mA_lo,
-        const __grid_constant__ CUtensorMap mB_hi, const __grid_constant__ CUtensorMap mB_lo, DwShape ds,
-        const __grid_constant__ ReplayJob rj) {
+        const __grid_constant__ CUtensorMap mB_hi, const __grid_constant__ CUtensorMap mB_lo, DwShape ds) {
     extern __shared__ uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t bars[2 * STAGES + 4];
     __shared__ uint32_t tmem_base_slot;
@@ -772,14 +714,14 @@ k_tc_dw(const __grid_constant__ CUtensorMap mA_hi, const __grid_constant__ CUten
             for (int kb = 0; kb < KB; ++kb) {
                 mbar_wait(empty0 + 8 * stage, phase ^ 1);
                 const uint32_t base = ring + stage * stage_bytes, fb = full0 + 8 * stage;
-                mbar_expect_tx(fb, TWO ? 3 * op_bytes : stage_bytes);
+                mbar_expect_tx(fb, stage_bytes);
                 const int row = r0 + kb * DW_BK;
 #pragma unroll
                 for (int m = 0; m < 4; ++m) {
                     tma_load_2d(base + m * box_bytes, &mA_hi, fb, i0 + 32 * m, row);
                     tma_load_2d(base + op_bytes + m * box_bytes, &mA_lo, fb, i0 + 32 * m, row);
                     tma_load_2d(base + 2 * op_bytes + m * box_bytes, &mB_hi, fb, k0 + 32 * m, row);
-                    if (!TWO) tma_load_2d(base + 3 * op_bytes + m * box_bytes, &mB_lo, fb, k0 + 32 * m, row);
+                    tma_load_2d(base + 3 * op_bytes + m * box_bytes, &mB_lo, fb, k0 + 32 * m, row);
                 }
                 if (++stage == STAGES) { stage = 0; phase ^= 1; }
             }
@@ -810,7 +752,7 @@ k_tc_dw(const __grid_constant__ CUtensorMap mA_hi, const __grid_constant__ CUten
                 for (int k = 0; k < DW_BK / 8; ++k, ++jj) {
                     const uint64_t adv = (uint64_t)((k * ds.kadv) >> 4);   // next 8-row swizzle atom
                     umma_tf32(d_cross, a_lo + adv, b_hi + adv, idesc, jj != 0);
-                    if (!TWO) umma_tf32(d_cross, a_hi + adv, b_lo + adv, idesc, 1);
+                    umma_tf32(d_cross, a_hi + adv, b_lo + adv, idesc, 1);
                     umma_tf32(d_main, a_hi + adv, b_hi + adv, idesc, jj != 0);
                 }
                 umma_commit(empty0 + 8 * stage);
@@ -821,24 +763,6 @@ k_tc_dw(const __grid_constant__ CUtensorMap mA_hi, const __grid_constant__ CUten
     } else if (warp >= kEpiWarp0) {
         const int ew = warp - kEpiWarp0, quarter = warp & 3, g = ew >> 2;
         const int i = i0 + quarter * 32 + lane;
-        // The epilogue warps only drain an accumulator set every DW_CHUNK K blocks; in between, each group of four warps (128
-        // threads) replays units of the NEXT reverse step (rj): elementwise work that needs nothing but the checkpoints and
-        // writes the other operand / phi' set, so it overlaps this contraction instead of running as a kernel of its own
-        // (which cannot share an SM with the 576-thread contraction CTAs: they hold the whole register file).
-        const int rtid = (ew & 3) * 32 + lane;
-        const int rtotal = (REPLAY && rj.valid) ? rj.nblocks * rj.slices : 0;      // REPLAY = false: the lean default kernel
-        const int rstep = (int)gridDim.x * 4;
-        int ru = (int)blockIdx.x * 4 + g;
-        ReplayLoad rl;                                // the next unit's checkpoint values, in flight while this one is processed
-        if (REPLAY && ru < rtotal) replay_load(rj, ru / rj.slices, ru % rj.slices, rtid, rl);
-        auto replay_next = [&]() {
-            if (!REPLAY) return;
-            const ReplayLoad cur = rl;
-            const int u = ru;
-            ru += rstep;
-            if (ru < rtotal) replay_load(rj, ru / rj.slices, ru % rj.slices, rtid, rl);
-            replay_compute(rj, u / rj.slices, u % rj.slices, rtid, cur);
-        };
         float acc[32];
         // fixed-order reduction: the running sum of this (tile, split) is fetched up front -- its latency hides behind the
         // contraction -- and stored back with the new contribution at the end (no read-modify-write in the kernel's tail)
@@ -865,9 +789,7 @@ k_tc_dw(const __grid_constant__ CUtensorMap mA_hi, const __grid_constant__ CUten
             tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive(tempty0 + 8 * set);
-            if (REPLAY && ru < rtotal) replay_next();
         }
-        while (REPLAY && ru < rtotal) replay_next();
         if (dst) {
 #pragma unroll
             for (int q = 0; q < 32; ++q) {
@@ -898,163 +820,15 @@ __global__ void k_dw_reduce_partials(const float* __restrict__ partial, int Z, s
     }
 }
 
-// CTA-pair variant of the dW contraction (tcgen05 cta_group::2, ODECOL_DW_PAIR=1): the output tiles (2m, k) and
-// (2m+1, k) run as one M = 256 MMA on the two SMs of a TPC; each CTA stages its own 128 columns of the A panel and HALF
-// (64 columns = two 32-wide boxes) of the shared B panel, i.e. 192 instead of 256 operand columns per K block and SM.
-// dW is the one contraction here without a heavy epilogue, bound purely by operand panels coming out of L2.
-// Barrier protocol as in k_tc_contract_pair (stage_tc.cuh).  Four ring stages of 48 KB.
-constexpr int DW_PSTAGES = 4;
-
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
-k_tc_dw_pair(const __grid_constant__ CUtensorMap mA_hi, const __grid_constant__ CUtensorMap mA_lo,
-             const __grid_constant__ CUtensorMap mB_hi, const __grid_constant__ CUtensorMap mB_lo, DwShape ds) {
-    extern __shared__ uint8_t smem_raw[];
-    __shared__ __align__(8) uint64_t bars[2 * DW_PSTAGES + 1];
-    __shared__ uint32_t tmem_base_slot;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t rank = cluster_ctarank();
-    const int pair = blockIdx.x >> 1;
-    const uint32_t ring = (smem_u32(smem_raw) + 1023u) & ~1023u;
-    constexpr uint32_t box_bytes = DW_BK * 128;                 // 32 rows x 32 floats
-    constexpr uint32_t a_bytes = 4 * box_bytes;                 // this CTA's 128 columns of A
-    constexpr uint32_t bh_bytes = 2 * box_bytes;                // this CTA's 64 of the 128 columns of B
-    constexpr uint32_t stage_bytes = 2 * a_bytes + 2 * bh_bytes;
-    const uint32_t full0 = smem_u32(&bars[0]), empty0 = smem_u32(&bars[DW_PSTAGES]), tfull = smem_u32(&bars[2 * DW_PSTAGES]);
-    constexpr uint32_t ncols = 512;
-    const int MT2 = ds.MT >> 1;
-    const int tile = pair % (MT2 * ds.NT), z = pair / (MT2 * ds.NT);
-    const int i0 = (2 * (tile % MT2) + (int)rank) * DW_T, k0 = (tile / MT2) * DW_T;
-    const int r0 = z * ds.rows_per_split;
-    int r1 = r0 + ds.rows_per_split;
-    if (r1 > ds.total_rows) r1 = ds.total_rows;
-    const int KB = (r1 - r0) / DW_BK;
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < DW_PSTAGES; ++s) { mbar_init(full0 + 8 * s, 1); mbar_init(empty0 + 8 * s, 1); }
-        mbar_init(tfull, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == kMmaWarp) {
-        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_slot)), "r"(ncols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    cluster_sync_all();
-    tc_fence_after();
-    const uint32_t tmem_base = tmem_base_slot;
-
-    if (warp == kTmaWarp) {
-        if (lane == 0) {
-            int stage = 0; uint32_t phase = 0;
-            for (int kb = 0; kb < KB; ++kb) {
-                mbar_wait(empty0 + 8 * stage, phase ^ 1);
-                const uint32_t base = ring + stage * stage_bytes;
-                const uint32_t fb = (full0 + 8 * stage) & kPeerBitMask;
-                if (rank == 0) mbar_expect_tx(full0 + 8 * stage, 2 * stage_bytes);
-                const int row = r0 + kb * DW_BK;
-#pragma unroll
-                for (int m = 0; m < 4; ++m) {
-                    tma_load_2d_pair(base + m * box_bytes, &mA_hi, fb, i0 + 32 * m, row);
-                    tma_load_2d_pair(base + a_bytes + m * box_bytes, &mA_lo, fb, i0 + 32 * m, row);
-                }
-#pragma unroll
-                for (int m = 0; m < 2; ++m) {
-                    tma_load_2d_pair(base + 2 * a_bytes + m * box_bytes, &mB_hi, fb, k0 + 64 * (int)rank + 32 * m, row);
-                    tma_load_2d_pair(base + 2 * a_bytes + bh_bytes + m * box_bytes, &mB_lo, fb, k0 + 64 * (int)rank + 32 * m, row);
-                }
-                if (++stage == DW_PSTAGES) { stage = 0; phase ^= 1; }
-            }
-        }
-    } else if (warp == kMmaWarp) {
-        if (lane == 0 && rank == 0) {
-            // c = F32, a = b = TF32, both MN-major, N = 128, M = 256 across the pair
-            const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ds.major_bits |
-                                   ((uint32_t)(DW_T >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
-            const uint32_t d_small = tmem_base + kMainAcc * DW_T;
-            int stage = 0; uint32_t phase = 0;
-            int j = 0;
-            for (int kb = 0; kb < KB; ++kb) {
-                mbar_wait(full0 + 8 * stage, phase);
-                tc_fence_after();
-                const uint32_t base = ring + stage * stage_bytes;
-                const uint64_t a_hi = make_smem_desc_mn(base, ds.lbo, ds.sbo), a_lo = make_smem_desc_mn(base + a_bytes, ds.lbo, ds.sbo);
-                const uint64_t b_hi = make_smem_desc_mn(base + 2 * a_bytes, ds.lbo, ds.sbo);
-                const uint64_t b_lo = make_smem_desc_mn(base + 2 * a_bytes + bh_bytes, ds.lbo, ds.sbo);
-#pragma unroll
-                for (int k = 0; k < DW_BK / 8; ++k, ++j) {
-                    const uint64_t adv = (uint64_t)((k * ds.kadv) >> 4);
-                    umma_tf32_pair(d_small, a_lo + adv, b_hi + adv, idesc, j != 0);
-                    umma_tf32_pair(d_small, a_hi + adv, b_lo + adv, idesc, 1);
-                    umma_tf32_pair(tmem_base + (uint32_t)(j % kMainAcc) * DW_T, a_hi + adv, b_hi + adv, idesc, j >= kMainAcc);
-                }
-                umma_commit_pair(empty0 + 8 * stage);
-                if (++stage == DW_PSTAGES) { stage = 0; phase ^= 1; }
-            }
-            umma_commit_pair(tfull);
-        }
-    } else if (KB > 0 && warp >= kEpiWarp0) {
-        const int ew = warp - kEpiWarp0, quarter = warp & 3, g = ew >> 2;
-        const int i = i0 + quarter * 32 + lane;
-        mbar_wait(tfull, 0);
-        tc_fence_after();
-        const uint32_t lane_base = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(g * 32);
-#pragma unroll
-        for (int q = 0; q < 8; ++q) {
-            uint32_t u[kMainAcc + 1][4];
-#pragma unroll
-            for (int a = 0; a <= kMainAcc; ++a) tmem_ld4_issue(lane_base + a * DW_T + 4 * q, u[a]);
-            tmem_ld_wait();
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-                float sum = __uint_as_float(u[kMainAcc][e]);
-#pragma unroll
-                for (int a = 0; a < kMainAcc; ++a) sum += __uint_as_float(u[a][e]);
-                const int k = k0 + g * 32 + 4 * q + e;
-                if (i < ds.N && k < ds.Kaug) atomicAdd(ds.grad_W + (size_t)i * ds.ld_w + k, sum);
-            }
-        }
-    }
-    tc_fence_before();
-    cluster_sync_all();
-    if (warp == kMmaWarp) {
-        asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(ncols) : "memory");
-    }
-}
-
-// launches the dW contraction (pair variant when enabled and the tile count allows)
-static bool dw_pair_enabled() {
-    static int use_pair = -1;
-    if (use_pair < 0) { const char* e = getenv("ODECOL_DW_PAIR"); use_pair = e ? (atoi(e) != 0) : 0; }
-    return use_pair != 0;
-}
-
-// rj: replay units of the next reverse step for the epilogue warps (k_tc_dw only; *rj_done says whether they were taken)
 static int launch_dw(const CUtensorMap& a_hi, const CUtensorMap& a_lo, const CUtensorMap& b_hi, const CUtensorMap& b_lo,
-                     const DwShape& ds, cudaStream_t s, const ReplayJob* rj = nullptr, bool* rj_done = nullptr) {
-    ReplayJob none;
-    none.valid = 0;
-    if (rj_done) *rj_done = false;
-    const bool use_pair = dw_pair_enabled();
+                     const DwShape& ds, cudaStream_t s) {
     static bool configured = false;
     if (!configured) {
-        if (cudaFuncSetAttribute(k_tc_dw<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess ||
-            cudaFuncSetAttribute(k_tc_dw<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess ||
-            cudaFuncSetAttribute(k_tc_dw<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess ||
-            cudaFuncSetAttribute(k_tc_dw_pair, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess)
+        if (cudaFuncSetAttribute(k_tc_dw, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess)
             return ODECOL_E_CUDA;
         configured = true;
     }
-    if (use_pair && ds.MT % 2 == 0 && !ds.two_products) {
-        const int pairs = (ds.MT / 2) * ds.NT * ds.Z;
-        k_tc_dw_pair<<<2 * pairs, kThreads, (size_t)DW_PSTAGES * (2 * 4 + 2 * 2) * DW_BK * 128 + 1024, s>>>(a_hi, a_lo, b_hi, b_lo, ds);
-    } else if (ds.two_products) {
-        k_tc_dw<true, false><<<ds.MT * ds.NT * ds.Z, kThreads, (size_t)STAGES * 4 * 4 * DW_BK * 128 + 1024, s>>>(a_hi, a_lo, b_hi, b_lo, ds, none);
-    } else if (rj) {
-        k_tc_dw<false, true><<<ds.MT * ds.NT * ds.Z, kThreads, (size_t)STAGES * 4 * 4 * DW_BK * 128 + 1024, s>>>(a_hi, a_lo, b_hi, b_lo, ds, *rj);
-        if (rj_done) *rj_done = true;
-    } else {
-        k_tc_dw<false, false><<<ds.MT * ds.NT * ds.Z, kThreads, (size_t)STAGES * 4 * 4 * DW_BK * 128 + 1024, s>>>(a_hi, a_lo, b_hi, b_lo, ds, none);
-    }
+    k_tc_dw<<<ds.MT * ds.NT * ds.Z, kThreads, (size_t)STAGES * 4 * 4 * DW_BK * 128 + 1024, s>>>(a_hi, a_lo, b_hi, b_lo, ds);
     count_launch();
     return cudaGetLastError() == cudaSuccess ? ODECOL_OK : ODECOL_E_CUDA;
 }
@@ -1077,7 +851,7 @@ __global__ void k_split_pad_T(const float* __restrict__ src, int n, int ld, floa
 struct TcBwdLayout {
     int Np, Bp, KPa, NPk, TN;
     size_t off_Whi, off_Wlo, off_WThi, off_WTlo, off_Rhi, off_Rlo, off_AVhi, off_AVlo;   // stacked x4 operand buffers
-    size_t off_K[3], off_Y, off_RT[3], off_DRT[8], off_lam, off_b4, off_b3, off_acur, off_inv, off_done, off_dwpart, total;
+    size_t off_K[3], off_Y, off_DRT[4], off_lam, off_b4, off_b3, off_acur, off_inv, off_done, off_dwpart, total;
     int dwZ;
 };
 
@@ -1092,15 +866,12 @@ static TcBwdLayout tc_bwd_layout(const DevProblem& p) {
     auto take = [&](size_t bytes) { const size_t r = o; o += (bytes + 1023) / 1024 * 1024; return r; };
     L.off_Whi = take(4ull * L.Np * L.KPa); L.off_Wlo = take(4ull * L.Np * L.KPa);
     L.off_WThi = take(4ull * L.Np * L.NPk); L.off_WTlo = take(4ull * L.Np * L.NPk);
-    // two sets of the four stacked r_aug operands and of the four phi' planes: in checkpoint mode the replay of step
-    // n-1 (done by the dW contraction kernel of step n) fills one set while the reverse stages of step n and that contraction read the other
-    L.off_Rhi = take(32ull * L.Bp * L.KPa); L.off_Rlo = take(32ull * L.Bp * L.KPa);
+    L.off_Rhi = take(16ull * L.Bp * L.KPa); L.off_Rlo = take(16ull * L.Bp * L.KPa);
     L.off_AVhi = take(32ull * L.Bp * L.NPk); L.off_AVlo = take(32ull * L.Bp * L.NPk);     // two sets of four slots
     const size_t plane = 4ull * L.Np * L.Bp;
     for (int i = 0; i < 3; ++i) L.off_K[i] = take(plane);
     L.off_Y = take(3 * plane);
-    for (int i = 0; i < 3; ++i) L.off_RT[i] = take(plane);
-    for (int i = 0; i < 8; ++i) L.off_DRT[i] = take(plane);
+    for (int i = 0; i < 4; ++i) L.off_DRT[i] = take(plane);
     L.off_lam = take(3 * plane); L.off_b4 = take(2 * plane); L.off_b3 = take(2 * plane); L.off_acur = take(2 * plane);
     L.off_inv = take(sizeof(int) * (3ull * p.N + 4));      // + the "an F component is selected" flag
     L.off_done = take(sizeof(unsigned int) * (size_t)(L.Bp / L.TN) + 256);
@@ -1144,7 +915,7 @@ int tc_contract_tn(const float* A, const float* B, float* C, int M, int N, int K
     int z = 2;
     int rows = (Kp / DW_BK + z - 1) / z * DW_BK;
     ds.rows_per_split = rows; ds.Z = (Kp + rows - 1) / rows;
-    ds.N = M; ds.Kaug = N; ds.ld_w = N; ds.grad_W = C; ds.two_products = 0; ds.partial = nullptr;
+    ds.N = M; ds.Kaug = N; ds.ld_w = N; ds.grad_W = C; ds.partial = nullptr;
     ds.lbo = DW_BK * 128; ds.sbo = 512; ds.major_bits = (1u << 15) | (1u << 16); ds.kadv = 1024;
     if (cudaMemsetAsync(C, 0, sizeof(float) * (size_t)M * N, s) != cudaSuccess) return ODECOL_E_CUDA;
     count_launch(2);
@@ -1169,7 +940,7 @@ int tc_dw_accumulate(const float* Ahi, const float* Alo, const float* Bhi, const
     int rps = (rows / DW_BK + z - 1) / z * DW_BK;
     if (rps < DW_BK) rps = DW_BK;
     ds.rows_per_split = rps; ds.Z = (rows + rps - 1) / rps;
-    ds.N = N; ds.Kaug = Kaug; ds.ld_w = ld_w; ds.grad_W = grad_W; ds.two_products = 0; ds.partial = nullptr;
+    ds.N = N; ds.Kaug = Kaug; ds.ld_w = ld_w; ds.grad_W = grad_W; ds.partial = nullptr;
     ds.lbo = DW_BK * 128; ds.sbo = 512; ds.major_bits = (1u << 15) | (1u << 16); ds.kadv = 1024;
     return launch_dw(a_hi, a_lo, b_hi, b_lo, ds, s);
 }
@@ -1189,9 +960,8 @@ static int tc_rk4_bwd_impl(const DevProblem& p, const float* t_dev, int T, const
     float *Rhi = F(L.off_Rhi), *Rlo = F(L.off_Rlo), *AVhi = F(L.off_AVhi), *AVlo = F(L.off_AVlo);
     float* KT[3] = {F(L.off_K[0]), F(L.off_K[1]), F(L.off_K[2])};
     float* YT = F(L.off_Y);
-    float* RT[3] = {F(L.off_RT[0]), F(L.off_RT[1]), F(L.off_RT[2])};
-    float* DRT[8];
-    for (int k = 0; k < 8; ++k) DRT[k] = F(L.off_DRT[k]);
+    float* DRT[4];
+    for (int k = 0; k < 4; ++k) DRT[k] = F(L.off_DRT[k]);
     float *lamT = F(L.off_lam), *b4T = F(L.off_b4), *b3T = F(L.off_b3), *acurT = F(L.off_acur);
     int* inv = reinterpret_cast<int*>(w + L.off_inv);
     const int Kaug = p.N + p.n_in + 1;
@@ -1204,7 +974,7 @@ static int tc_rk4_bwd_impl(const DevProblem& p, const float* t_dev, int T, const
     if (cudaMemsetAsync(w + L.off_Rhi, 0, L.off_K[0] - L.off_Rhi, s) != cudaSuccess) return ODECOL_E_CUDA;
     k_split_pad<<<296, 256, 0, s>>>(p.W_aug, p.N, Kaug, p.ld_w, Whi, Wlo, L.Np, L.KPa);
     k_split_pad_T<<<296, 256, 0, s>>>(p.W_aug, p.N, p.ld_w, WThi, WTlo, L.Np, L.NPk);
-    k_tc_set_one<<<(8 * p.B + 255) / 256, 256, 0, s>>>(Rhi, L.Bp, p.B, L.KPa, Kaug - 1, 8);
+    k_tc_set_one<<<(4 * p.B + 255) / 256, 256, 0, s>>>(Rhi, L.Bp, p.B, L.KPa, Kaug - 1, 4);
     k_tc_build_inv<<<1, 256, 0, s>>>(sel, G, 3 * p.N, inv);
     const size_t first = (size_t)(((T - 2) & 1) * 4 + 3);       // operand sets alternate per step: step n uses set n & 1
     k_tc_bwd_begin<<<L.Bp / 4, 128, 0, s>>>(p, tg, grad_y, inv, G, t_dev, T, gamma, lamT, acurT, AVhi + first * astride,
@@ -1213,7 +983,7 @@ static int tc_rk4_bwd_impl(const DevProblem& p, const float* t_dev, int T, const
     if (cudaMemsetAsync(done, 0, sizeof(unsigned int) * (size_t)(L.Bp / L.TN), s) != cudaSuccess) return ODECOL_E_CUDA;
     count_launch(5);
 
-    CUtensorMap mWhi, mWlo, mWThi, mWTlo, mRhi, mRlo, mAVhi, mAVlo, dAhi[2], dAlo[2], dBhi[2], dBlo[2];
+    CUtensorMap mWhi, mWlo, mWThi, mWTlo, mRhi, mRlo, mAVhi, mAVlo, dAhi[2], dAlo[2], dBhi, dBlo;
     bool ok = make_map(&mWhi, Whi, L.Np, L.KPa, L.KPa, BM) && make_map(&mWlo, Wlo, L.Np, L.KPa, L.KPa, BM) &&
               make_map(&mWThi, WThi, L.Np, L.NPk, L.NPk, BM) && make_map(&mWTlo, WTlo, L.Np, L.NPk, L.NPk, BM) &&
               make_map(&mRhi, Rhi, 4ull * L.Bp, L.KPa, L.KPa, L.TN) && make_map(&mRlo, Rlo, 4ull * L.Bp, L.KPa, L.KPa, L.TN) &&
@@ -1222,27 +992,21 @@ static int tc_rk4_bwd_impl(const DevProblem& p, const float* t_dev, int T, const
               make_map(&dAlo[0], AVlo, 4ull * L.Bp, L.NPk, L.NPk, DW_BK, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B) &&
               make_map(&dAhi[1], AVhi + 4 * astride, 4ull * L.Bp, L.NPk, L.NPk, DW_BK, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B) &&
               make_map(&dAlo[1], AVlo + 4 * astride, 4ull * L.Bp, L.NPk, L.NPk, DW_BK, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B) &&
-              make_map(&dBhi[0], Rhi, 4ull * L.Bp, L.KPa, L.KPa, DW_BK, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B) &&
-              make_map(&dBlo[0], Rlo, 4ull * L.Bp, L.KPa, L.KPa, DW_BK, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B) &&
-              make_map(&dBhi[1], Rhi + 4 * rstride, 4ull * L.Bp, L.KPa, L.KPa, DW_BK, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B) &&
-              make_map(&dBlo[1], Rlo + 4 * rstride, 4ull * L.Bp, L.KPa, L.KPa, DW_BK, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B);
+              make_map(&dBhi, Rhi, 4ull * L.Bp, L.KPa, L.KPa, DW_BK, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B) &&
+              make_map(&dBlo, Rlo, 4ull * L.Bp, L.KPa, L.KPa, DW_BK, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B);
     if (!ok) return ODECOL_E_CUDA;
 
-    // dW launch shape: output tiles x splits of the stacked rows, one wave of CTAs (ODECOL_DW_WAVES)
+    // dW launch shape: output tiles x splits of the stacked rows, one wave of CTAs (chunked accumulation: long items are
+    // accurate)
     DwShape ds;
     ds.MT = L.Np / DW_T; ds.NT = (L.KPa + DW_T - 1) / DW_T;
     ds.total_rows = 4 * L.Bp;
-    static const int dw_waves = getenv("ODECOL_DW_WAVES") ? atoi(getenv("ODECOL_DW_WAVES")) : 1;   // chunked accumulation: long items are accurate
-    int z = (dw_waves * num_sms()) / (ds.MT * ds.NT);
+    int z = num_sms() / (ds.MT * ds.NT);
     if (z < 1) z = 1;
     int rows = (ds.total_rows / DW_BK + z - 1) / z * DW_BK;
     if (rows < DW_BK) rows = DW_BK;
     ds.rows_per_split = rows; ds.Z = (ds.total_rows + rows - 1) / rows;
     ds.N = p.N; ds.Kaug = Kaug; ds.ld_w = p.ld_w; ds.grad_W = grad_W;
-    ds.two_products = 0;
-#ifdef ODECOL_DIAG
-    { const char* e2 = getenv("ODECOL_DW_2X"); ds.two_products = e2 ? (atoi(e2) != 0) : 0; }    // fails the gradient bar: experiment only
-#endif
     ds.lbo = DW_BK * 128; ds.sbo = 512; ds.major_bits = (1u << 15) | (1u << 16); ds.kadv = 1024;
     ds.partial = nullptr;
 
@@ -1257,13 +1021,13 @@ static int tc_rk4_bwd_impl(const DevProblem& p, const float* t_dev, int T, const
     // reduction, whose per-split copies live in the stand-alone kernel).
     const char* fe = getenv("ODECOL_FUSE_DW");
     const bool dw_fixed_order = (p.flags & ODECOL_FLAG_DETERMINISTIC) != 0;     // default: float atomics (2 % faster sweep)
-    const bool fuse_dw = use_chain && !dw_fixed_order && !dw_pair_enabled() && (fe ? atoi(fe) != 0 : true);
+    const bool fuse_dw = use_chain && !dw_fixed_order && (fe ? atoi(fe) != 0 : true);
     // ODECOL_FLAG_DETERMINISTIC: every (output tile, row split) accumulates into its own copy of grad_W_aug across the whole
     // sweep (one CTA per (tile, split) and launch, launches ordered on the stream; the running sum is fetched at kernel start
     // and stored back at the end), the copies are summed in a fixed order after the last step -- the gradient is
     // bit-reproducible.  Measured: reverse sweep 633-639 ms against 621-625 ms with float atomics (A/B on one box).
     float* dw_partial = nullptr;
-    if (dw_fixed_order && !fuse_dw && !(dw_pair_enabled() && ds.MT % 2 == 0) && ds.Z <= L.dwZ) {
+    if (dw_fixed_order && ds.Z <= L.dwZ) {
         dw_partial = reinterpret_cast<float*>(w + L.off_dwpart);
         if (cudaMemsetAsync(dw_partial, 0, sizeof(float) * (size_t)ds.Z * p.N * p.ld_w, s) != cudaSuccess) return ODECOL_E_CUDA;
         ds.partial = dw_partial;
@@ -1278,42 +1042,27 @@ static int tc_rk4_bwd_impl(const DevProblem& p, const float* t_dev, int T, const
             cudaOccupancyMaxActiveBlocksPerMultiprocessor(&max_blocks, k_tc_bwd_chain<true>, kThreads, chain_smem) != cudaSuccess || max_blocks < 1)
             use_chain = false;
     }
-    // Checkpoint mode: the replay of a step needs nothing but the checkpoints, so it runs one step AHEAD of the
-    // contractions, into the other operand / phi' set -- INSIDE the dW contraction of the step before: its epilogue warps
-    // idle between accumulator drains and take the replay's units (k_tc_dw / ReplayJob).  A kernel of its own cannot
-    // overlap anything here: the 576-thread contraction CTAs hold an SM's whole register file, so a side-stream replay ran
-    // in the gaps between launches only (measured: ODECOL_OVERLAP=0 changed nothing; replay alone 81 us per step).
-    // Default: every step's replay is a launch of its own on the caller's stream.
-    // MEASURED (round 2, one box): reverse sweep 632-641 ms with the replay as its own launch per step, 685 ms with the replay
-    // inside the dW contraction, 721 ms with its loads pipelined there -- the sixteen epilogue warps' arithmetic delays the two
-    // single-thread issue loops of the contraction more than the saved launch is worth.  Hence OFF by default
-    // (ODECOL_OVERLAP=1 turns it on).
-    const char* ov = getenv("ODECOL_OVERLAP");
-    const bool overlap = ckVA != nullptr && (ov ? atoi(ov) != 0 : false);
+    // Checkpoint mode: every step's operands and phi' planes are replayed from the checkpoints by a launch of their own.
+    // (Handing the replay to the idle epilogue warps of the previous step's dW contraction measured slower, DESIGN.md
+    // section 7: the epilogue warps' arithmetic delays the contraction's two single-thread issue loops.)
     const size_t ckpl = (size_t)L.Np * L.Bp;
-    auto replay_job = [&](int n) {
-        ReplayJob j;
-        const int rs = overlap ? (n & 1) : 0;
-        j.valid = 1; j.p = p; j.tg = tg;
-        j.VA = ckVA + 2 * ckpl * (size_t)n; j.KV = ckK + 3 * ckpl * (size_t)n; j.t = t_dev;
-        j.n = n; j.KPa = L.KPa; j.nblocks = L.Bp / 4; j.slices = L.Np / 128;
-        j.Rhi = Rhi + (size_t)rs * 4 * rstride; j.Rlo = Rlo + (size_t)rs * 4 * rstride; j.rstride = rstride;
-        for (int k = 0; k < 4; ++k) j.D[k] = DRT[4 * rs + k];
-        return j;
-    };
     auto replay = [&](int n) {
-        k_tc_replay<<<L.Bp / 4, 128, 0, s>>>(replay_job(n));
+        ReplayJob j;
+        j.p = p; j.tg = tg;
+        j.VA = ckVA + 2 * ckpl * (size_t)n; j.KV = ckK + 3 * ckpl * (size_t)n; j.t = t_dev;
+        j.n = n; j.KPa = L.KPa; j.slices = L.Np / 128;
+        j.Rhi = Rhi; j.Rlo = Rlo; j.rstride = rstride;
+        for (int k = 0; k < 4; ++k) j.D[k] = DRT[k];
+        k_tc_replay<<<L.Bp / 4, 128, 0, s>>>(j);
         count_launch();
     };
-    bool replayed_ahead = false;                     // step n's operands were produced inside dW(n+1)
     for (int n = T - 2; n >= 0; --n) {
         int rc = ODECOL_OK;
-        const int rset = overlap ? (n & 1) : 0;      // operand / phi' set of this step
         if (ckVA) {
-            if (!replayed_ahead) replay(n);
+            replay(n);
         } else {
         const float* yn = y_traj + (size_t)n * st;
-        k_tc_step_begin<<<L.Bp / 4, 128, 0, s>>>(p, tg, yn, t_dev + n, Rhi, Rlo, YT, RT[0], DRT[0], L.KPa);
+        k_tc_step_begin<<<L.Bp / 4, 128, 0, s>>>(p, tg, yn, t_dev + n, Rhi, Rlo, YT, DRT[0], L.KPa);
         count_launch();
         // recompute stages 1..3: operand s -> operand s+1, r and phi' of the next stage state
         auto fill_f = [&](auto& e, int S) {
@@ -1321,35 +1070,26 @@ static int tc_rk4_bwd_impl(const DevProblem& p, const float* t_dev, int T, const
             e.V0T = YT; e.A0T = YT + tg.plane(); e.F0T = nullptr;       // stages 1..3 never touch F
             e.V1T = e.A1T = e.F1T = nullptr; e.traj_row = nullptr; e.ysel_row = nullptr; e.inv = nullptr; e.G = 0;
             e.K1T = KT[0]; e.K2T = KT[1]; e.K3T = KT[2];
-            e.RsT[0] = RT[0]; e.RsT[1] = RT[1]; e.RsT[2] = RT[2]; e.RsT[3] = nullptr;
-            e.store_r = S < 3;                                  // r of stage 4 is only needed as the dW operand
-            e.Rhi_nxt = Rhi + S * rstride; e.Rlo_nxt = Rlo + S * rstride; e.DRT_nxt = DRT[S]; e.dbg_skip = 0;
+            e.Rhi_nxt = Rhi + S * rstride; e.Rlo_nxt = Rlo + S * rstride; e.DRT_nxt = DRT[S];
             e.inv_tm = 1.0f / p.c.tau_m; e.inv_ta = 1.0f / p.c.tau_a; e.inv_ts = 1.0f / p.c.tau_s;
             e.t0 = e.t1 = e.dt = 0.f;
         };
-        { FwdEpiT<1> e; fill_f(e, 1); rc = launch_contract(mWhi, mWlo, mRhi, mRlo, TileShape{MT, NT, L.TN, L.KPa / BK, 0 * L.Bp, nullptr}, e, s); if (rc) return rc; }
-        { FwdEpiT<2> e; fill_f(e, 2); rc = launch_contract(mWhi, mWlo, mRhi, mRlo, TileShape{MT, NT, L.TN, L.KPa / BK, 1 * L.Bp, nullptr}, e, s); if (rc) return rc; }
-        { FwdEpiT<3> e; fill_f(e, 3); rc = launch_contract(mWhi, mWlo, mRhi, mRlo, TileShape{MT, NT, L.TN, L.KPa / BK, 2 * L.Bp, nullptr}, e, s); if (rc) return rc; }
+        { FwdEpiT<1> e; fill_f(e, 1); rc = launch_contract(mWhi, mWlo, mRhi, mRlo, TileShape{MT, NT, L.TN, L.KPa / BK, 0 * L.Bp}, e, s); if (rc) return rc; }
+        { FwdEpiT<2> e; fill_f(e, 2); rc = launch_contract(mWhi, mWlo, mRhi, mRlo, TileShape{MT, NT, L.TN, L.KPa / BK, 1 * L.Bp}, e, s); if (rc) return rc; }
+        { FwdEpiT<3> e; fill_f(e, 3); rc = launch_contract(mWhi, mWlo, mRhi, mRlo, TileShape{MT, NT, L.TN, L.KPa / BK, 2 * L.Bp}, e, s); if (rc) return rc; }
         }
         // reverse stages 4, 3, 2, 1 (stage 1 writes kbar_4 of the next step into the OTHER operand set), then dW
         const int set = n & 1;
-#ifdef ODECOL_DIAG
-        static const int dbg_skip = getenv("ODECOL_DBG_BWD_SKIP") ? atoi(getenv("ODECOL_DBG_BWD_SKIP")) : 0;   // timing diagnostics only
-#else
-        constexpr int dbg_skip = 0;
-#endif
-        if (use_chain && (dbg_skip & 2)) {
-            // diagnostics: chain skipped
-        } else if (use_chain) {
+        if (use_chain) {
             BwdChainArgs a;
-            a.p = p; a.tg = tg; a.ts = TileShape{MT, NT, L.TN, L.NPk / BK, 0, nullptr}; a.t = t_dev; a.n = n; a.NPk = L.NPk; a.G = G;
+            a.p = p; a.tg = tg; a.ts = TileShape{MT, NT, L.TN, L.NPk / BK, 0}; a.t = t_dev; a.n = n; a.NPk = L.NPk; a.G = G;
             a.Bp = L.Bp; a.acurT = acurT; a.lamT = lamT; a.b4T = b4T; a.b3T = b3T;
-            for (int k = 0; k < 4; ++k) a.DRT[k] = DRT[4 * rset + k];
+            for (int k = 0; k < 4; ++k) a.DRT[k] = DRT[k];
             a.AVhi = AVhi; a.AVlo = AVlo; a.set = set; a.grad_y = grad_y; a.inv = inv; a.gamma = gamma;
             a.inv_tm = 1.0f / p.c.tau_m; a.inv_ta = 1.0f / p.c.tau_a; a.inv_ts = 1.0f / p.c.tau_s;
             a.done = done; a.done_base = (unsigned int)MT * 4u * (unsigned int)(T - 2 - n);
-            a.fuse_dw = fuse_dw ? 1 : 0; a.ds = ds;
-            void* args[] = {&mWThi, &mWTlo, &mAVhi, &mAVlo, &dAhi[set], &dAlo[set], &dBhi[rset], &dBlo[rset], &a};
+            a.ds = ds;
+            void* args[] = {&mWThi, &mWTlo, &mAVhi, &mAVlo, &dAhi[set], &dAlo[set], &dBhi, &dBlo, &a};
             const void* chain_fn = fuse_dw ? (const void*)k_tc_bwd_chain<true> : (const void*)k_tc_bwd_chain<false>;
             if (cudaLaunchCooperativeKernel(chain_fn, dim3(chain_grid), dim3(kThreads), args, chain_smem, s) != cudaSuccess)
                 return ODECOL_E_CUDA;
@@ -1357,7 +1097,7 @@ static int tc_rk4_bwd_impl(const DevProblem& p, const float* t_dev, int T, const
         } else {
             auto fill_b = [&](auto& e, int S) {
                 e.p = p; e.tg = tg; e.t = t_dev; e.n = n; e.NPk = L.NPk; e.G = G;
-                e.acurT = acurT; e.lamT = lamT; e.b4T = b4T; e.b3T = b3T; e.DRT = DRT[4 * rset + S - 1];
+                e.acurT = acurT; e.lamT = lamT; e.b4T = b4T; e.b3T = b3T; e.DRT = DRT[S - 1];
                 const size_t nxt = S == 1 ? (size_t)((set ^ 1) * 4 + 3) : (size_t)(set * 4 + S - 2);   // slot the epilogue writes
                 e.AVhi_nxt = AVhi + nxt * astride; e.AVlo_nxt = AVlo + nxt * astride;
                 e.grad_y = grad_y; e.inv = inv; e.gamma = gamma;
@@ -1365,17 +1105,13 @@ static int tc_rk4_bwd_impl(const DevProblem& p, const float* t_dev, int T, const
                 e.dt = e.h8p = 0.f;
             };
             const int r0 = set * 4 * L.Bp;
-            { BwdEpiT<4> e; fill_b(e, 4); rc = launch_contract(mWThi, mWTlo, mAVhi, mAVlo, TileShape{MT, NT, L.TN, L.NPk / BK, r0 + 3 * L.Bp, nullptr}, e, s); if (rc) return rc; }
-            { BwdEpiT<3> e; fill_b(e, 3); rc = launch_contract(mWThi, mWTlo, mAVhi, mAVlo, TileShape{MT, NT, L.TN, L.NPk / BK, r0 + 2 * L.Bp, nullptr}, e, s); if (rc) return rc; }
-            { BwdEpiT<2> e; fill_b(e, 2); rc = launch_contract(mWThi, mWTlo, mAVhi, mAVlo, TileShape{MT, NT, L.TN, L.NPk / BK, r0 + 1 * L.Bp, nullptr}, e, s); if (rc) return rc; }
-            { BwdEpiT<1> e; fill_b(e, 1); rc = launch_contract(mWThi, mWTlo, mAVhi, mAVlo, TileShape{MT, NT, L.TN, L.NPk / BK, r0 + 0 * L.Bp, nullptr}, e, s); if (rc) return rc; }
+            { BwdEpiT<4> e; fill_b(e, 4); rc = launch_contract(mWThi, mWTlo, mAVhi, mAVlo, TileShape{MT, NT, L.TN, L.NPk / BK, r0 + 3 * L.Bp}, e, s); if (rc) return rc; }
+            { BwdEpiT<3> e; fill_b(e, 3); rc = launch_contract(mWThi, mWTlo, mAVhi, mAVlo, TileShape{MT, NT, L.TN, L.NPk / BK, r0 + 2 * L.Bp}, e, s); if (rc) return rc; }
+            { BwdEpiT<2> e; fill_b(e, 2); rc = launch_contract(mWThi, mWTlo, mAVhi, mAVlo, TileShape{MT, NT, L.TN, L.NPk / BK, r0 + 1 * L.Bp}, e, s); if (rc) return rc; }
+            { BwdEpiT<1> e; fill_b(e, 1); rc = launch_contract(mWThi, mWTlo, mAVhi, mAVlo, TileShape{MT, NT, L.TN, L.NPk / BK, r0 + 0 * L.Bp}, e, s); if (rc) return rc; }
         }
-        replayed_ahead = false;
-        if (!(use_chain && fuse_dw) && !(dbg_skip & 1)) {
-            ReplayJob next;
-            const bool ahead = overlap && n > 0;      // replay(n-1) into the other set, inside this step's dW contraction
-            if (ahead) next = replay_job(n - 1);
-            const int rcd = launch_dw(dAhi[set], dAlo[set], dBhi[rset], dBlo[rset], ds, s, ahead ? &next : nullptr, &replayed_ahead);
+        if (!(use_chain && fuse_dw)) {
+            const int rcd = launch_dw(dAhi[set], dAlo[set], dBhi, dBlo, ds, s);
             if (rcd) return rcd;
         }
     }

@@ -23,7 +23,6 @@ struct PersistArgs {
     float* y_out;              // (rows, B, 3N)
     float* YT[2];              // tile-major state, ping-pong per step
     float* KT[3];
-    float* RT[4];              // r of stages 1..4 of the current step
     float* Rhi[2]; float* Rlo[2];
     uint16_t* R16[2]; size_t r16_plane; int KP16; const float* wscale;     // 16-bit operand format (F16 kernel)
     unsigned int* ovf;         // F16 kernel: raised when an operand value does not fit FP16
@@ -54,11 +53,9 @@ ODECOL_DEVINL FwdEpiT<S, F16> persist_epi(const PersistArgs& a, int n, int q) {
         e.traj_row = emit ? a.y_out + r * ((size_t)a.p.B * 3 * a.p.N) : nullptr;
         e.ysel_row = nullptr; e.inv = nullptr; e.G = 0;
     }
-    for (int k = 0; k < 4; ++k) e.RsT[k] = a.RT[k];
-    e.store_r = 1;
     e.Rhi_nxt = a.Rhi[(q + 1) & 1]; e.Rlo_nxt = a.Rlo[(q + 1) & 1];
     e.R16_nxt = a.R16[(q + 1) & 1]; e.r16_plane = a.r16_plane; e.KP16 = a.KP16; e.wscale = a.wscale; e.ovf = a.ovf;
-    e.DRT_nxt = nullptr; e.dbg_skip = 0;
+    e.DRT_nxt = nullptr;
     e.inv_tm = a.inv_tm; e.inv_ta = a.inv_ta; e.inv_ts = a.inv_ts;
     return e;
 }
@@ -196,12 +193,6 @@ k_tc_rk4_fwd_persistent(const __grid_constant__ CUtensorMap mW_hi, const __grid_
                 const int m_tile = tile % ts.MT, nt = tile / ts.MT, n0 = nt * ts.TN;
                 const int row = m_tile * BM + quarter * 32 + lane;
                 float tot[kMaxQ];
-                switch (s) {                       // warm L2 with this thread's first scratch groups while the tile is contracted
-                    case 1: { FwdEpiT<1, F16> e = persist_epi<1, F16>(a, n, q); e.needF = 1; e.pre_tile(row, nt, g, TNq); } break;
-                    case 2: { FwdEpiT<2, F16> e = persist_epi<2, F16>(a, n, q); e.needF = 1; e.pre_tile(row, nt, g, TNq); } break;
-                    case 3: { FwdEpiT<3, F16> e = persist_epi<3, F16>(a, n, q); e.needF = 1; e.pre_tile(row, nt, g, TNq); } break;
-                    default: { FwdEpiT<4, F16> e = persist_epi<4, F16>(a, n, q); e.needF = 0; e.pre_tile(row, nt, g, TNq); } break;
-                }
                 mbar_wait(tfull, tphase);
                 tc_fence_after();
                 const uint32_t lane_base = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(g * TNq);
@@ -252,25 +243,25 @@ k_tc_rk4_fwd_persistent(const __grid_constant__ CUtensorMap mW_hi, const __grid_
 // mx != NULL: buffers of the mixed 16-bit operand format (stage_tc.cuh) -- used unless ODECOL_FWD16=0.
 int tc_rk4_fwd_persistent(const DevProblem& p, const float* t_dev, int T, const float* y0, float* y_out, int out_every,
                           float* Whi, float* Wlo, float* const Rhi[2], float* const Rlo[2], float* const KT[3],
-                          float* const YT[2], float* const RT[4], unsigned int* done, int Np, int Bp, int KPa, int TN,
-                          const tc::CkptView* ck, const tc::Mixed16* mx, cudaStream_t s) {
+                          float* const YT[2], unsigned int* done, int Np, int Bp, int KPa, int TN, const tc::CkptView* ck,
+                          const tc::Mixed16* mx, cudaStream_t s) {
     using namespace tc;
     const int Kaug = p.N + p.n_in + 1;
     const size_t st = (size_t)p.B * 3 * p.N;
     const TileGeom tg{Bp / TN, Np, TN, TN / 4};
     static const bool fwd16_env = [] { const char* e = getenv("ODECOL_FWD16"); return e ? atoi(e) != 0 : true; }();
     const bool f16 = mx && fwd16_env;
-    const TileShape tsh{Np / BM, Bp / TN, TN, f16 ? mx->KP16 / BK16 : KPa / BK, 0, nullptr};
+    const TileShape tsh{Np / BM, Bp / TN, TN, f16 ? mx->KP16 / BK16 : KPa / BK, 0};
     const int tiles = tsh.MT * tsh.NT;
     int grid = tiles < num_sms() ? tiles : num_sms();
     // every trial tile's population tiles must be owned by co-resident CTAs: guaranteed by the cooperative launch
 
     k_split_pad<<<296, 256, 0, s>>>(p.W_aug, p.N, Kaug, p.ld_w, Whi, Wlo, Np, KPa);
     extern void tc_launch_init(const DevProblem&, const TileGeom&, const float*, const float*, float*, float*, float*, float*,
-                               float*, float*, float*, float*, int, int, cudaStream_t);
+                               float*, float*, float*, int, int, cudaStream_t);
     const size_t pl = tg.plane();
     float* V0 = ck ? ck->VA : YT[0];
-    tc_launch_init(p, tg, y0, t_dev, Rhi[0], Rlo[0], Rhi[1], Rlo[1], V0, V0 + pl, YT[0] + 2 * pl, RT[0], KPa, Bp, s);
+    tc_launch_init(p, tg, y0, t_dev, Rhi[0], Rlo[0], Rhi[1], Rlo[1], V0, V0 + pl, YT[0] + 2 * pl, KPa, Bp, s);
     count_launch(2);
     unsigned int* ovf = f16 ? reinterpret_cast<unsigned int*>(mx->wscale + 2) : nullptr;
     if (f16) {
@@ -304,7 +295,6 @@ int tc_rk4_fwd_persistent(const DevProblem& p, const float* t_dev, int T, const 
     for (int i = 0; i < 2; ++i) { a.YT[i] = YT[i]; a.Rhi[i] = Rhi[i]; a.Rlo[i] = Rlo[i]; a.R16[i] = f16 ? mx->R16[i] : nullptr; }
     a.r16_plane = f16 ? (size_t)Bp * mx->KP16 : 0; a.KP16 = f16 ? mx->KP16 : 0; a.wscale = f16 ? mx->wscale : nullptr;
     a.ovf = ovf; a.run_if = nullptr;
-    for (int i = 0; i < 4; ++i) a.RT[i] = RT[i];
     for (int i = 0; i < 3; ++i) a.KT[i] = KT[i];
     a.done = done;
     if (ck) a.ck = *ck; else a.ck = CkptView{nullptr, nullptr, nullptr, nullptr, 0};
@@ -324,7 +314,7 @@ int tc_rk4_fwd_persistent(const DevProblem& p, const float* t_dev, int T, const 
             return ODECOL_E_CUDA;
         count_launch();
         // fallback: the same solve in the TF32 format, from the start -- a no-op unless the 16-bit solve raised its flag
-        tc_launch_init(p, tg, y0, t_dev, Rhi[0], Rlo[0], Rhi[1], Rlo[1], V0, V0 + pl, YT[0] + 2 * pl, RT[0], KPa, Bp, s);
+        tc_launch_init(p, tg, y0, t_dev, Rhi[0], Rlo[0], Rhi[1], Rlo[1], V0, V0 + pl, YT[0] + 2 * pl, KPa, Bp, s);
         if (cudaMemsetAsync(done, 0, sizeof(unsigned int) * tsh.NT, s) != cudaSuccess) return ODECOL_E_CUDA;
         a.ts.KB = KPa / BK; a.run_if = ovf;
         count_launch();

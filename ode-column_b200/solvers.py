@@ -75,7 +75,7 @@ class _Setup:
         time_vec = func.time_vec.detach().to(device=dev, dtype=torch.float32)
         self.knot_t, self.knot_u = compress_knots(time_vec, table)
         if family not in (None, "staged", "tensor"):
-            raise ValueError("odecol: options['family'] must be None, 'staged' (FP32 FFMA) or 'tensor' (tcgen05 3xTF32)")
+            raise ValueError("odecol: options['family'] must be None, 'staged' or 'tensor' (both skip the on-chip family)")
         self.flags = {None: 0, "staged": self.ext.FLAG_FORCE_STAGED, "tensor": self.ext.FLAG_FORCE_TENSOR}[family]
         # bit-reproducible gradients on request, or whenever torch itself is asked for deterministic algorithms
         if deterministic if deterministic is not None else torch.are_deterministic_algorithms_enabled():
@@ -252,8 +252,9 @@ def odeint(func, y0, t, *, rtol=1e-7, atol=1e-9, method=None, options=None, even
     default the reference scripts get) or 'rk4' (3/8 rule on the grid ``t``); both for every network size, both
     differentiable (exact discrete adjoints).  Extras beyond torchdiffeq:
     ``components`` restricts the returned trajectory to those state components (T, B, len(components));
-    ``stats`` (a dict) receives per-trial n_accept / n_reject / status tensors; ``options['family']='staged'`` forces
-    the global-state kernel family, ``options['max_num_steps']`` bounds dopri5, ``options['deterministic']=True`` (default:
+    ``stats`` (a dict) receives per-trial n_accept / n_reject / status tensors; ``options['family']='staged'`` (or
+    ``'tensor'``, the same) forces the global-state kernel family, for rk4 the tcgen05 tensor family,
+    ``options['max_num_steps']`` bounds dopri5, ``options['deterministic']=True`` (default:
     ``torch.are_deterministic_algorithms_enabled()``) makes the tensor family's rk4 gradients bit-reproducible (fixed-order
     reduction over trials instead of float atomics, about 2 % slower)."""
     if event_fn is not None:

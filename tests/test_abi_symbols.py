@@ -220,8 +220,8 @@ def test_shape_and_pointer_validation_without_a_gpu(lib):
     fam.argtypes = [ctypes.c_void_p, ctypes.c_int]
     assert fam(ctypes.byref(p), 1) == 0 and fam(ctypes.byref(big), 1) == 2 and fam(ctypes.byref(_problem(N=0)), 1) == -1
     assert fam(ctypes.byref(_problem(N=160, n_in=20, ld_w=184)), 1) == 2            # beyond the on-chip family: tensor cores
-    assert fam(ctypes.byref(_problem(N=160, n_in=20, ld_w=184, flags=1)), 1) == 1   # ... unless the FFMA family is forced
-    assert fam(ctypes.byref(_problem(N=162, n_in=20, ld_w=184)), 1) == 1            # N not a multiple of 4
+    assert fam(ctypes.byref(_problem(N=160, n_in=20, ld_w=184, flags=1)), 1) == 2   # ... whichever staged family is forced
+    assert fam(ctypes.byref(_problem(N=162, n_in=20, ld_w=184)), 1) == 2            # N not a multiple of 4: unsupported there
     # the parity network (N = 104) fits the on-chip family, but from 4096 trials its rk4 runs on the tensor cores; the adaptive
     # and stochastic solvers stay on chip, and so do the small networks at any batch size
     par = dict(N=104, n_in=4, ld_w=112)

@@ -1,7 +1,7 @@
 """Differential test on problem shapes the reference networks do not reach: every register-tile size of the on-chip
 family (KP = 40 / 64 / 96 / 128), two trials per warp with and without it, more stimulus channels than lanes (the
 uncached knot path), ragged batches -- rk4 forward and reverse through the extension, against the CPU oracle's autograd;
-and the same problems forced through the staged FFMA and tensor families.  dopri5 is judged against a float64 replay of
+and the same problems forced through the tensor family.  dopri5 is judged against a float64 replay of
 the steps its record holds (the oracle's adaptive solve takes another step sequence)."""
 import numpy as np
 import pytest
@@ -39,7 +39,7 @@ def _problem(N, n_in, B, K, seed):
     return lf, tv, kt, ku, y0
 
 
-@pytest.mark.parametrize("family", [0, "staged", "tensor"])
+@pytest.mark.parametrize("family", [0, "tensor"])
 @pytest.mark.parametrize("shape", SHAPES, ids=lambda s: "N%d_in%d_B%d_K%d" % s)
 def test_rk4_forward_and_reverse_on_random_problems(shape, family):
     N, n_in, B, K = shape
@@ -57,10 +57,10 @@ def test_rk4_forward_and_reverse_on_random_problems(shape, family):
     ld = (N + n_in + 1 + 3) // 4 * 4
     W_aug = torch.zeros(N, ld)
     W_aug[:, :N] = torch.tensor(lf.W); W_aug[:, N:N + n_in] = torch.tensor(lf.U); W_aug[:, N + n_in] = torch.tensor(lf.bias)
-    flags = {0: 0, "staged": ext.FLAG_FORCE_STAGED, "tensor": ext.FLAG_FORCE_TENSOR}[family]
+    flags = {0: 0, "tensor": ext.FLAG_FORCE_TENSOR}[family]
     prob = ext.Problem(W_aug.to(DEV), torch.tensor(lf.kappa).to(DEV), None, torch.tensor(kt).to(DEV), torch.tensor(ku).to(DEV),
                        n_in, B, lf.tau_s, lf.tau_m, lf.tau_a, lf.resistance, flags)
-    assert prob.kernel_family(ext.OP_RK4_FWD) == {0: 0, "staged": 1, "tensor": 2}[family]
+    assert prob.kernel_family(ext.OP_RK4_FWD) == {0: 0, "tensor": 2}[family]
     t_dev = torch.tensor(tv).to(DEV)
     y = ext.rk4_fwd(prob, t_dev, torch.tensor(y0).to(DEV), 1)
     gy0, gW = ext.rk4_bwd(prob, t_dev, y, wgt.to(DEV).contiguous(), None)
