@@ -467,35 +467,216 @@ __global__ void k_em_fill_nan(DevProblem p, const int* __restrict__ status, cons
         for (int comp = threadIdx.x; comp < 3 * N; comp += blockDim.x) y_out[(size_t)j * total + (size_t)b * 3 * N + comp] = qnan;
 }
 
+// end of an adaptive solve: NaN for the outputs a stopped trial never reached, then the per-trial statistics
+template <class State>
+static int adaptive_finish(const DevProblem& p, const State& S, int T, float* y_out, int* n_accept, int* n_reject, int* status,
+                           cudaStream_t s) {
+    k_em_fill_nan<<<p.B, 128, 0, s>>>(p, S.status, S.next_out, T, y_out);
+    count_launch();
+    const size_t B = p.B;
+    if (n_accept && cudaMemcpyAsync(n_accept, S.n_acc, sizeof(int) * B, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
+    if (n_reject && cudaMemcpyAsync(n_reject, S.n_rej, sizeof(int) * B, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
+    if (status && cudaMemcpyAsync(status, S.status, sizeof(int) * B, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
+    return cudaGetLastError() == cudaSuccess ? ODECOL_OK : ODECOL_E_CUDA;
+}
+
+// grid of the elementwise kernels over n elements
+static int ew_grid(size_t n) {
+    const size_t g = (n + 255) / 256;
+    return (int)(g < 148 * 16 ? g : 148 * 16);
+}
+
+// workspace pieces, each 1024-byte aligned
+struct Carve {
+    size_t o = 0;
+    size_t take(size_t bytes) { const size_t r = o; o += (bytes + 1023) / 1024 * 1024; return r; }
+};
+
+// per-trial arrays carved one after another from one workspace piece, 16-byte aligned
+struct TrialCarve {
+    char* at;
+    template <class T> void operator()(T*& dst, size_t n) { dst = reinterpret_cast<T*>(at); at += (n * sizeof(T) + 15) / 16 * 16; }
+};
+
+// ---- one drift evaluation of the staged solvers on the tensor cores ----------------------------------------------------
+// The drift part of a staged workspace: W_aug split into two planes, `sets` operand sets of two planes, and on request
+// each set's within-column input plane (lateral-gain sweeps) and the aux slot of the 16-bit format.  The planes are sized
+// for TF32 pairs (KPa floats per row); the 16-bit format keeps its rows of KP16 halves in the same buffers
+// (2 KP16 <= 4 KPa bytes).  Operand planes have `rows` rows: Bp, or Bp rounded up to 32 for the adjoint, whose dW
+// contraction reads them in blocks of 32 trials; the tensor maps cover Bp.  StagedDrift::init zeroes the bytes from the
+// first operand plane up to zero_end.
+struct DriftLayout {
+    int Np, KPa, KP16, TN, Bp, rows, sets;
+    bool loc, aux;
+    size_t off_W[2], off_R[2][2], off_loc[2], off_aux, zero_end;
+};
+
+static DriftLayout drift_layout(Carve& c, const DevProblem& p, int sets, bool loc, bool aux, bool dw_rows) {
+    DriftLayout L;
+    L.Np = round_up(p.N, BM);
+    L.KPa = round_up(p.N + p.n_in + 1, BK);
+    L.KP16 = round_up(p.N + p.n_in + 1, BK16);
+    L.TN = pick_tile_n(L.Np / BM, p.B);
+    L.Bp = round_up(p.B, L.TN);
+    L.rows = dw_rows ? round_up(L.Bp, 32) : L.Bp;
+    L.sets = sets;
+    L.loc = loc && p.lat_gain;
+    L.aux = aux;
+    for (int i = 0; i < 2; ++i) L.off_W[i] = c.take(4ull * L.Np * L.KPa);
+    for (int q = 0; q < sets; ++q)
+        for (int i = 0; i < 2; ++i) L.off_R[q][i] = c.take(4ull * L.rows * L.KPa);
+    L.zero_end = c.o;
+    for (int q = 0; q < sets && L.loc; ++q) L.off_loc[q] = c.take(4ull * p.B * p.N);
+    if (aux) L.off_aux = c.take(64);
+    return L;
+}
+
+// kRetryTf32: a solve in the 16-bit operand format met a value that does not fit FP16 and has to be repeated in TF32
+static constexpr int kRetryTf32 = 1 << 20;
+
+// f[b] = drift(t_b, y_b): k_em_operand writes r_aug(t_b, y_b) into an operand set, the tensor-core contraction against the
+// split W_aug runs with the RhsEpi epilogue.  In the 16-bit format (f16) W_aug, scaled by a power of two, and the operands
+// are FP16 pairs, and an operand value that does not fit FP16 raises the overflow flag in aux[2].
+struct StagedDrift {
+    DevProblem p;
+    cudaStream_t s;
+    bool f16;
+    int KPr;                                      // elements per operand row in the format in use
+    float* W[2];                                  // split W_aug: hi, lo
+    float* R[2][2] = {};                          // operand sets: [set][hi, lo]
+    float* loc[2] = {};                           // within-column input plane of each set (lateral-gain sweeps), else NULL
+    float* aux = nullptr;                         // [0] 1 / weight scale, [1] max|W| bits, [2] overflow flag
+    CUtensorMap mW[2], mR[2][2];
+    TileShape tsh;
+
+    unsigned int* ovf() const { return f16 ? reinterpret_cast<unsigned int*>(aux + 2) : nullptr; }
+
+    // zero the operand planes (their padding stays zero) and the aux slot, split W_aug in the format, encode the maps
+    int init(const DevProblem& p_, char* w, const DriftLayout& L, bool f16_, cudaStream_t s_) {
+        p = p_; s = s_; f16 = f16_;
+        KPr = f16 ? L.KP16 : L.KPa;
+        auto F = [&](size_t off) { return reinterpret_cast<float*>(w + off); };
+        for (int i = 0; i < 2; ++i) W[i] = F(L.off_W[i]);
+        for (int q = 0; q < L.sets; ++q) {
+            for (int i = 0; i < 2; ++i) R[q][i] = F(L.off_R[q][i]);
+            loc[q] = L.loc ? F(L.off_loc[q]) : nullptr;
+        }
+        if (L.aux) aux = F(L.off_aux);
+        const int Kaug = p.N + p.n_in + 1;
+        if (cudaMemsetAsync(R[0][0], 0, L.zero_end - L.off_R[0][0], s) != cudaSuccess) return ODECOL_E_CUDA;
+        if (f16) {
+            if (cudaMemsetAsync(aux, 0, 64, s) != cudaSuccess) return ODECOL_E_CUDA;
+            k_absmax<<<148, 256, 0, s>>>(p.W_aug, p.N, Kaug, p.ld_w, reinterpret_cast<unsigned int*>(aux + 1));
+            k_split16_w<<<296, 256, 0, s>>>(p.W_aug, p.N, Kaug, p.ld_w, reinterpret_cast<__half*>(W[0]), reinterpret_cast<__half*>(W[1]),
+                                            L.Np, L.KP16, reinterpret_cast<unsigned int*>(aux + 1), aux);
+            count_launch(2);
+        } else {
+            k_split_pad<<<296, 256, 0, s>>>(p.W_aug, p.N, Kaug, p.ld_w, W[0], W[1], L.Np, L.KPa);
+            count_launch();
+        }
+        auto map = [&](CUtensorMap* m, const float* base, int rows, int box_rows) {
+            return f16 ? make_map16(m, base, rows, L.KP16, L.KP16, box_rows, false) : make_map(m, base, rows, L.KPa, L.KPa, box_rows);
+        };
+        for (int i = 0; i < 2; ++i)
+            if (!map(&mW[i], W[i], L.Np, BM)) return ODECOL_E_CUDA;
+        for (int q = 0; q < L.sets; ++q)
+            for (int i = 0; i < 2; ++i)
+                if (!map(&mR[q][i], R[q][i], L.Bp, L.TN)) return ODECOL_E_CUDA;
+        tsh = TileShape{L.Np / BM, L.Bp / L.TN, L.TN, f16 ? L.KP16 / BK16 : L.KPa / BK, 0};
+        return ODECOL_OK;
+    }
+    // r_aug(t, y) into operand set `set`; t_trial != NULL: one time per trial, else t_shared for all
+    void operand(int set, const float* y, const float* t_trial, float t_shared) {
+        k_em_operand<<<p.B, 128, 0, s>>>(p, y, t_trial, t_shared, R[set][0], R[set][1], KPr, nullptr, loc[set], ovf());
+        count_launch();
+    }
+    // where k_ad_half1 / k_ad_commit write the operand of set `set`
+    OperandDst dst(int set) const { return OperandDst{R[set][0], R[set][1], loc[set], KPr, ovf()}; }
+    // f = drift(y) from the operand in set `set`
+    int contract(int set, const float* y, float* f) const {
+        RhsEpi e;
+        e.p = p; e.y = y; e.Rhi = R[set][0]; e.Rlo = R[set][1]; e.f = f; e.KPa = KPr; e.loc = loc[set]; e.wscale = f16 ? aux : nullptr;
+        e.inv_tm = 1.0f / p.c.tau_m; e.inv_ta = 1.0f / p.c.tau_a; e.inv_ts = 1.0f / p.c.tau_s;
+        if (f16) return launch_contract16(mW[0], mW[1], mR[set][0], mR[set][1], tsh, e, s);
+        return launch_contract(mW[0], mW[1], mR[set][0], mR[set][1], tsh, e, s);
+    }
+    int eval(int set, const float* y, const float* t_trial, float t_shared, float* f) {
+        operand(set, y, t_trial, t_shared);
+        return contract(set, y, f);
+    }
+    // Synchronises the stream, in the 16-bit format after copying the overflow flag: kRetryTf32 when an operand value did
+    // not fit FP16, else ODECOL_OK (or ODECOL_E_CUDA)
+    int overflowed() const {
+        unsigned int h = 0;
+        if (f16 && cudaMemcpyAsync(&h, ovf(), sizeof(h), cudaMemcpyDeviceToHost, s) != cudaSuccess) return ODECOL_E_CUDA;
+        if (cudaStreamSynchronize(s) != cudaSuccess) return ODECOL_E_CUDA;
+        return h ? kRetryTf32 : ODECOL_OK;
+    }
+};
+
+// The forward solves read FP16 pairs in their drift contractions (half the tensor-core instructions and operand bytes of
+// the TF32 split: the contraction is 93 % of a round at N = 8192 and runs at 0.89 of the tensor roofline) unless their
+// switch is set to 0.  Each switch is read once per process.
+enum F16Switch { kEm16, kDp16, kSrk16 };
+static bool f16_switch(F16Switch sw) {
+    auto on = [](const char* name) { const char* e = getenv(name); return e ? atoi(e) != 0 : true; };
+    switch (sw) {
+        case kEm16: { static const bool v = on("ODECOL_EM16"); return v; }
+        case kDp16: { static const bool v = on("ODECOL_DP16"); return v; }
+        default: { static const bool v = on("ODECOL_SRK16"); return v; }
+    }
+}
+// solve(f16) in the 16-bit format when the switch and `allow` say so; kRetryTf32 (an operand value did not fit FP16, read
+// at the host's polls) repeats the solve in the TF32 format
+template <class Solve>
+static int solve_f16_or_tf32(F16Switch sw, bool allow, Solve&& solve) {
+    const int rc = solve(f16_switch(sw) && allow);
+    return rc == kRetryTf32 ? solve(false) : rc;
+}
+
+// torchsde's float32 fixed-step loop (integrate()), replayed on the host from a copy of ts (data independent):
+// step(k, t0, t1, j_lo, j_hi) runs step k from t0 to t1, after which the outputs ts[j], j in [j_lo, j_hi), are due.
+// n_steps receives the number of steps.
+template <class Step>
+static int fixed_step_walk(const float* ts_dev, int T, float dt, cudaStream_t s, long long& n_steps, Step&& step) {
+    std::vector<float> ts(T);
+    if (cudaMemcpyAsync(ts.data(), ts_dev, sizeof(float) * T, cudaMemcpyDeviceToHost, s) != cudaSuccess) return ODECOL_E_CUDA;
+    if (cudaStreamSynchronize(s) != cudaSuccess) return ODECOL_E_CUDA;
+    volatile float curr = ts[0];
+    const float t_end = ts[T - 1];
+    long long k = 0;
+    for (int j = 1; j < T;) {
+        const float c0 = curr;
+        volatile float nx = c0 + dt;
+        const float next_t = nx < t_end ? nx : t_end;
+        int j_hi = j;
+        while (j_hi < T && ts[j_hi] <= next_t) ++j_hi;            // outputs the loop emits once curr_t >= ts[j]
+        const int rc = step(k, c0, next_t, j, j_hi);
+        if (rc != ODECOL_OK) return rc;
+        curr = next_t;
+        j = j_hi;
+        if (++k > (1LL << 40)) return ODECOL_E_SHAPE;
+    }
+    n_steps = k;
+    return ODECOL_OK;
+}
+
 struct EmLayout {
-    int Np, Bp, KPa, TN;
-    size_t off_Whi, off_Wlo, off_Rhi, off_Rlo, off_Rhi1, off_Rlo1, off_f, off_fm, off_yfull, off_ymid, off_yhalf, off_y, off_yprev,
-           off_state, off_loc, off_loc1, off_aux, total;
-    int KP16;
+    DriftLayout drift;
+    size_t off_f, off_fm, off_yfull, off_ymid, off_yhalf, off_y, off_yprev, off_state, total;
 };
 
 static EmLayout em_layout(const DevProblem& p) {
     EmLayout L;
-    L.Np = round_up(p.N, BM);
-    L.KPa = round_up(p.N + p.n_in + 1, BK);
-    L.TN = pick_tile_n(L.Np / BM, p.B);
-    L.Bp = round_up(p.B, L.TN);
-    size_t o = 0;
-    auto take = [&](size_t bytes) { const size_t r = o; o += (bytes + 1023) / 1024 * 1024; return r; };
-    L.off_Whi = take(4ull * L.Np * L.KPa); L.off_Wlo = take(4ull * L.Np * L.KPa);
-    L.off_Rhi = take(4ull * L.Bp * L.KPa); L.off_Rlo = take(4ull * L.Bp * L.KPa);
-    // second operand set: the adaptive sweep keeps the operand of f(t_cur, y) (set 0) across a rejected attempt while the
+    Carve c;
+    // two operand sets: the adaptive sweep keeps the operand of f(t_cur, y) (set 0) across a rejected attempt while the
     // midpoint evaluation f(t_mid, y_mid) uses set 1
-    L.off_Rhi1 = take(4ull * L.Bp * L.KPa); L.off_Rlo1 = take(4ull * L.Bp * L.KPa);
+    L.drift = drift_layout(c, p, 2, /*loc=*/true, /*aux=*/true, /*dw_rows=*/false);
     const size_t st = 4ull * p.B * 3 * p.N;
-    L.off_f = take(st); L.off_fm = take(st); L.off_yfull = take(st); L.off_ymid = take(st); L.off_yhalf = take(st);
-    L.off_y = take(st); L.off_yprev = take(st);
-    L.off_state = take(128ull * p.B + 1024);
-    L.off_loc = take(p.lat_gain ? 4ull * p.B * p.N : 0);       // within-column input planes of the lateral-gain sweep
-    L.off_loc1 = take(p.lat_gain ? 4ull * p.B * p.N : 0);
-    L.off_aux = take(64);                                       // 16-bit operand format: 1 / weight scale, max|W| scratch, overflow flag
-    L.KP16 = round_up(p.N + p.n_in + 1, BK16);                  // its rows live in the same buffers (2 KP16 <= 4 KPa bytes)
-    L.total = o;
+    L.off_f = c.take(st); L.off_fm = c.take(st); L.off_yfull = c.take(st); L.off_ymid = c.take(st); L.off_yhalf = c.take(st);
+    L.off_y = c.take(st); L.off_yprev = c.take(st);
+    L.off_state = c.take(128ull * p.B + 1024);
+    L.total = c.o;
     return L;
 }
 
@@ -503,10 +684,6 @@ static EmLayout em_layout(const DevProblem& p) {
 
 size_t stage_em_fwd_workspace_bytes(const DevProblem& p, int) { return tc::em_layout(p).total; }
 
-// f16: the drift contractions read FP16 pairs (half the tensor-core instructions and operand bytes of the TF32 split: the
-// contraction is 93 % of a round at N = 8192 and runs at 0.89 of the tensor roofline).  Returns kRetryTf32 when an operand
-// value did not fit FP16 (the flag is read at the host's polls): the caller repeats the solve in the TF32 format.
-static constexpr int kRetryTf32 = 1 << 20;
 static int em_fwd_impl(const DevProblem& p, const float* ts_dev, int T, const float* y0, float* y_out, const float* dW,
                        uint64_t seed, int64_t trial_offset, float dt, int adaptive, float rtol, float atol, float dt_min,
                        int* n_accept, int* n_reject, int* status, float* y_steps, void* ws, size_t ws_bytes, cudaStream_t s,
@@ -517,106 +694,36 @@ static int em_fwd_impl(const DevProblem& p, const float* ts_dev, int T, const fl
     if (p.N % 4 != 0) return ODECOL_E_UNSUPPORTED;
     char* w = static_cast<char*>(ws);
     auto F = [&](size_t off) { return reinterpret_cast<float*>(w + off); };
-    float *Whi = F(L.off_Whi), *Wlo = F(L.off_Wlo), *Rhi = F(L.off_Rhi), *Rlo = F(L.off_Rlo);
     float *f0 = F(L.off_f), *fm = F(L.off_fm), *yfull = F(L.off_yfull), *ymid = F(L.off_ymid), *yhalf = F(L.off_yhalf);
     float *y = F(L.off_y), *yprev = F(L.off_yprev);
-    float* loc = p.lat_gain ? F(L.off_loc) : nullptr;
-    const int Kaug = p.N + p.n_in + 1;
     const size_t st = (size_t)p.B * 3 * p.N;
 
-    if (cudaMemsetAsync(w + L.off_Rhi, 0, L.off_f - L.off_Rhi, s) != cudaSuccess) return ODECOL_E_CUDA;
-    float* aux = F(L.off_aux);                                  // [0] 1 / weight scale, [1] max|W| bits, [2] overflow flag
-    unsigned int* ovf = f16 ? reinterpret_cast<unsigned int*>(aux + 2) : nullptr;
-    const int KPr = f16 ? L.KP16 : L.KPa;                       // elements per operand row in the format in use
-    if (f16) {
-        if (cudaMemsetAsync(aux, 0, 64, s) != cudaSuccess) return ODECOL_E_CUDA;
-        k_absmax<<<148, 256, 0, s>>>(p.W_aug, p.N, Kaug, p.ld_w, reinterpret_cast<unsigned int*>(aux + 1));
-        k_split16_w<<<296, 256, 0, s>>>(p.W_aug, p.N, Kaug, p.ld_w, reinterpret_cast<__half*>(Whi), reinterpret_cast<__half*>(Wlo),
-                                        L.Np, L.KP16, reinterpret_cast<unsigned int*>(aux + 1), aux);
-        count_launch(2);
-    } else {
-        k_split_pad<<<296, 256, 0, s>>>(p.W_aug, p.N, Kaug, p.ld_w, Whi, Wlo, L.Np, L.KPa);
-        count_launch();
-    }
+    StagedDrift drift;
+    int rc = drift.init(p, w, L.drift, f16, s);
+    if (rc != ODECOL_OK) return rc;
     if (cudaMemcpyAsync(y, y0, sizeof(float) * st, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
     if (cudaMemcpyAsync(yprev, y0, sizeof(float) * st, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
     if (cudaMemcpyAsync(y_out, y0, sizeof(float) * st, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
     if (y_steps && cudaMemcpyAsync(y_steps, y0, sizeof(float) * st, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
-    CUtensorMap mWhi, mWlo, mRhi, mRlo;
-    if (f16) {
-        if (!make_map16(&mWhi, Whi, L.Np, L.KP16, L.KP16, BM, false) || !make_map16(&mWlo, Wlo, L.Np, L.KP16, L.KP16, BM, false) ||
-            !make_map16(&mRhi, Rhi, L.Bp, L.KP16, L.KP16, L.TN, false) || !make_map16(&mRlo, Rlo, L.Bp, L.KP16, L.KP16, L.TN, false))
-            return ODECOL_E_CUDA;
-    } else if (!make_map(&mWhi, Whi, L.Np, L.KPa, L.KPa, BM) || !make_map(&mWlo, Wlo, L.Np, L.KPa, L.KPa, BM) ||
-               !make_map(&mRhi, Rhi, L.Bp, L.KPa, L.KPa, L.TN) || !make_map(&mRlo, Rlo, L.Bp, L.KPa, L.KPa, L.TN))
-        return ODECOL_E_CUDA;
-    const TileShape tsh{L.Np / BM, L.Bp / L.TN, L.TN, f16 ? L.KP16 / BK16 : L.KPa / BK, 0};
-    auto rhs = [&](const float* ysrc, float* fdst) {
-        RhsEpi e;
-        e.p = p; e.y = ysrc; e.Rhi = Rhi; e.Rlo = Rlo; e.f = fdst; e.KPa = KPr; e.loc = loc; e.wscale = f16 ? aux : nullptr;
-        e.inv_tm = 1.0f / p.c.tau_m; e.inv_ta = 1.0f / p.c.tau_a; e.inv_ts = 1.0f / p.c.tau_s;
-        if (f16) return launch_contract16(mWhi, mWlo, mRhi, mRlo, tsh, e, s);
-        return launch_contract(mWhi, mWlo, mRhi, mRlo, tsh, e, s);
-    };
-    // adaptive sweep: the midpoint evaluation f(t_mid, y_mid) reads operand set 1 (written by k_ad_half1), so that the
-    // operand of f(t_cur, y) in set 0 (written by k_ad_commit) survives a rejected attempt
-    float *Rhi1 = F(L.off_Rhi1), *Rlo1 = F(L.off_Rlo1);
-    float* loc1 = p.lat_gain ? F(L.off_loc1) : nullptr;
-    CUtensorMap mRhi1, mRlo1;
-    if (adaptive && f16) {
-        if (!make_map16(&mRhi1, Rhi1, L.Bp, L.KP16, L.KP16, L.TN, false) || !make_map16(&mRlo1, Rlo1, L.Bp, L.KP16, L.KP16, L.TN, false))
-            return ODECOL_E_CUDA;
-    } else if (adaptive) {
-        if (!make_map(&mRhi1, Rhi1, L.Bp, L.KPa, L.KPa, L.TN) || !make_map(&mRlo1, Rlo1, L.Bp, L.KPa, L.KPa, L.TN)) return ODECOL_E_CUDA;
-    }
-    auto rhs_mid = [&](const float* ysrc, float* fdst) {
-        RhsEpi e;
-        e.p = p; e.y = ysrc; e.Rhi = Rhi1; e.Rlo = Rlo1; e.f = fdst; e.KPa = KPr; e.loc = loc1; e.wscale = f16 ? aux : nullptr;
-        e.inv_tm = 1.0f / p.c.tau_m; e.inv_ta = 1.0f / p.c.tau_a; e.inv_ts = 1.0f / p.c.tau_s;
-        if (f16) return launch_contract16(mWhi, mWlo, mRhi1, mRlo1, tsh, e, s);
-        return launch_contract(mWhi, mWlo, mRhi1, mRlo1, tsh, e, s);
-    };
-    const int ew_grid = (int)((st + 255) / 256 < 148 * 16 ? (st + 255) / 256 : 148 * 16);
 
     if (!adaptive) {
-        // replay the float32 time loop of torchsde's integrate() on the host (data independent)
-        std::vector<float> ts(T);
-        if (cudaMemcpyAsync(ts.data(), ts_dev, sizeof(float) * T, cudaMemcpyDeviceToHost, s) != cudaSuccess) return ODECOL_E_CUDA;
-        if (cudaStreamSynchronize(s) != cudaSuccess) return ODECOL_E_CUDA;
-        volatile float curr = ts[0];
-        const float t_end = ts[T - 1];
-        long long k = 0;
-        int j = 1;
-        while (j < T) {
-            const float c0 = curr;
-            volatile float nx = c0 + dt;
-            const float next_t = nx < t_end ? nx : t_end;
-            int j_hi = j;
-            while (j_hi < T && ts[j_hi] <= next_t) ++j_hi;            // outputs the loop emits once curr_t >= ts[j]
-            k_em_operand<<<p.B, 128, 0, s>>>(p, y, nullptr, c0, Rhi, Rlo, KPr, nullptr, loc, ovf);
-            count_launch();
-            const int rc = rhs(y, f0);
-            if (rc != ODECOL_OK) return rc;
+        long long n_steps = 0;
+        rc = fixed_step_walk(ts_dev, T, dt, s, n_steps, [&](long long k, float t0, float t1, int j_lo, int j_hi) -> int {
+            const int r = drift.eval(0, y, nullptr, t0, f0);
+            if (r != ODECOL_OK) return r;
             EmStepArgs a;
             a.p = p; a.y = y; a.f = f0; a.y_prev = yprev; a.dW = dW; a.seed = seed; a.trial_offset = trial_offset; a.kstep = k;
-            a.t0 = c0; a.t1 = next_t; a.y_out = y_out; a.j_lo = j; a.j_hi = j_hi; a.ts = ts_dev;
-            k_em_step<<<ew_grid, 256, 0, s>>>(a);
+            a.t0 = t0; a.t1 = t1; a.y_out = y_out; a.j_lo = j_lo; a.j_hi = j_hi; a.ts = ts_dev;
+            k_em_step<<<ew_grid(st), 256, 0, s>>>(a);
             count_launch();
-            curr = next_t;
-            j = j_hi;
-            ++k;
-            if (y_steps && cudaMemcpyAsync(y_steps + (size_t)k * st, y, sizeof(float) * st, cudaMemcpyDeviceToDevice, s) != cudaSuccess)
+            if (y_steps && cudaMemcpyAsync(y_steps + (size_t)(k + 1) * st, y, sizeof(float) * st, cudaMemcpyDeviceToDevice, s) != cudaSuccess)
                 return ODECOL_E_CUDA;
-            if (k > (1LL << 40)) return ODECOL_E_SHAPE;
-        }
-        if (f16) {                                            // did every operand value fit FP16?
-            unsigned int h_ovf = 0;
-            if (cudaMemcpyAsync(&h_ovf, ovf, sizeof(h_ovf), cudaMemcpyDeviceToHost, s) != cudaSuccess) return ODECOL_E_CUDA;
-            if (cudaStreamSynchronize(s) != cudaSuccess) return ODECOL_E_CUDA;
-            if (h_ovf) return kRetryTf32;
-        }
+            return ODECOL_OK;
+        });
+        if (rc != ODECOL_OK) return rc;
+        if (f16 && (rc = drift.overflowed()) != ODECOL_OK) return rc;     // did every operand value fit FP16?
         if (n_accept || n_reject || status) {
-            std::vector<int> hk(p.B, (int)k), hz(p.B, 0);
+            std::vector<int> hk(p.B, (int)n_steps), hz(p.B, 0);
             if (n_accept && cudaMemcpyAsync(n_accept, hk.data(), sizeof(int) * p.B, cudaMemcpyHostToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
             if (n_reject && cudaMemcpyAsync(n_reject, hz.data(), sizeof(int) * p.B, cudaMemcpyHostToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
             if (status && cudaMemcpyAsync(status, hz.data(), sizeof(int) * p.B, cudaMemcpyHostToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
@@ -626,21 +733,14 @@ static int em_fwd_impl(const DevProblem& p, const float* ts_dev, int T, const fl
     }
 
     // ---- adaptive: per-trial controller state carved from the workspace
-    char* sb = w + L.off_state;
     TrialState S;
     const size_t B = p.B;
-    auto grab = [&](size_t bytes) { char* r = sb; sb += (bytes + 15) / 16 * 16; return r; };
-    S.step = reinterpret_cast<double*>(grab(8 * B)); S.prev_ratio = reinterpret_cast<double*>(grab(8 * B));
-    S.err2 = reinterpret_cast<double*>(grab(8 * B));
-    S.t_cur = reinterpret_cast<float*>(grab(4 * B)); S.t_prev = reinterpret_cast<float*>(grab(4 * B));
-    S.t_mid = reinterpret_cast<float*>(grab(4 * B)); S.t_next = reinterpret_cast<float*>(grab(4 * B));
-    S.w_cur = reinterpret_cast<float*>(grab(4 * B)); S.dw_full = reinterpret_cast<float*>(grab(4 * B));
-    S.dw_1 = reinterpret_cast<float*>(grab(4 * B)); S.dw_2 = reinterpret_cast<float*>(grab(4 * B));
-    S.has_prev = reinterpret_cast<int*>(grab(4 * B)); S.next_out = reinterpret_cast<int*>(grab(4 * B));
-    S.n_acc = reinterpret_cast<int*>(grab(4 * B)); S.n_rej = reinterpret_cast<int*>(grab(4 * B));
-    S.status = reinterpret_cast<int*>(grab(4 * B)); S.active = reinterpret_cast<int*>(grab(4 * B));
-    S.accept = reinterpret_cast<int*>(grab(4 * B));
-    S.n_active = reinterpret_cast<int*>(grab(16));
+    TrialCarve g{w + L.off_state};
+    g(S.step, B); g(S.prev_ratio, B); g(S.err2, B);
+    g(S.t_cur, B); g(S.t_prev, B); g(S.t_mid, B); g(S.t_next, B);
+    g(S.w_cur, B); g(S.dw_full, B); g(S.dw_1, B); g(S.dw_2, B);
+    g(S.has_prev, B); g(S.next_out, B); g(S.n_acc, B); g(S.n_rej, B); g(S.status, B); g(S.active, B); g(S.accept, B);
+    g(S.n_active, 1);
 
     std::vector<float> tse(2);
     if (cudaMemcpyAsync(&tse[0], ts_dev, sizeof(float), cudaMemcpyDeviceToHost, s) != cudaSuccess) return ODECOL_E_CUDA;
@@ -650,50 +750,35 @@ static int em_fwd_impl(const DevProblem& p, const float* ts_dev, int T, const fl
     const long long max_attempts = (long long)(4.0 * span / dt_min) + 4LL * T + 1024;
     const int tb = (p.B + 127) / 128;
     k_ad_init<<<tb, 128, 0, s>>>(p, S, ts_dev, T, dt, seed, trial_offset);
-    k_em_operand<<<p.B, 128, 0, s>>>(p, y, S.t_cur, 0.f, Rhi, Rlo, KPr, nullptr, loc, ovf);
-    count_launch(2);
+    count_launch();
+    drift.operand(0, y, S.t_cur, 0.f);
     int h_active = p.B;
-    unsigned int h_ovf = 0;
     for (long long round = 0; round < max_attempts && h_active > 0; ++round) {
-        int rc = rhs(y, f0);
-        if (rc != ODECOL_OK) return rc;
-        k_ad_half1<<<p.B, 256, 0, s>>>(p, S, y, f0, yfull, ymid, OperandDst{Rhi1, Rlo1, loc1, KPr, ovf});
-        rc = rhs_mid(ymid, fm);
-        if (rc != ODECOL_OK) return rc;
+        // the midpoint evaluation f(t_mid, y_mid) reads operand set 1 (written by k_ad_half1), so that the operand of
+        // f(t_cur, y) in set 0 (written by k_ad_commit) survives a rejected attempt
+        if ((rc = drift.contract(0, y, f0)) != ODECOL_OK) return rc;
+        k_ad_half1<<<p.B, 256, 0, s>>>(p, S, y, f0, yfull, ymid, drift.dst(1));
+        if ((rc = drift.contract(1, ymid, fm)) != ODECOL_OK) return rc;
         k_ad_half2<<<p.B, 256, 0, s>>>(p, S, ymid, fm, yfull, yhalf, rtol, atol);
         k_ad_control<<<tb, 128, 0, s>>>(p, S, ts_dev, T, dt_min, seed, trial_offset, max_attempts);
-        k_ad_commit<<<p.B, 256, 0, s>>>(p, S, ts_dev, T, y, yprev, yhalf, y_out, OperandDst{Rhi, Rlo, loc, KPr, ovf});
+        k_ad_commit<<<p.B, 256, 0, s>>>(p, S, ts_dev, T, y, yprev, yhalf, y_out, drift.dst(0));
         count_launch(4);
         if ((round & 15) == 15) {
             if (cudaMemcpyAsync(&h_active, S.n_active, sizeof(int), cudaMemcpyDeviceToHost, s) != cudaSuccess) return ODECOL_E_CUDA;
-            if (f16 && cudaMemcpyAsync(&h_ovf, ovf, sizeof(h_ovf), cudaMemcpyDeviceToHost, s) != cudaSuccess) return ODECOL_E_CUDA;
-            if (cudaStreamSynchronize(s) != cudaSuccess) return ODECOL_E_CUDA;
-            if (h_ovf) return kRetryTf32;
+            if ((rc = drift.overflowed()) != ODECOL_OK) return rc;
         }
     }
-    if (f16) {                                                // rounds since the last poll
-        if (cudaMemcpyAsync(&h_ovf, ovf, sizeof(h_ovf), cudaMemcpyDeviceToHost, s) != cudaSuccess) return ODECOL_E_CUDA;
-        if (cudaStreamSynchronize(s) != cudaSuccess) return ODECOL_E_CUDA;
-        if (h_ovf) return kRetryTf32;
-    }
-    k_em_fill_nan<<<p.B, 128, 0, s>>>(p, S.status, S.next_out, T, y_out);
-    count_launch();
-    if (n_accept && cudaMemcpyAsync(n_accept, S.n_acc, sizeof(int) * B, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
-    if (n_reject && cudaMemcpyAsync(n_reject, S.n_rej, sizeof(int) * B, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
-    if (status && cudaMemcpyAsync(status, S.status, sizeof(int) * B, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
-    return cudaGetLastError() == cudaSuccess ? ODECOL_OK : ODECOL_E_CUDA;
+    if (f16 && (rc = drift.overflowed()) != ODECOL_OK) return rc;         // rounds since the last poll
+    return adaptive_finish(p, S, T, y_out, n_accept, n_reject, status, s);
 }
 
 int stage_em_fwd(const DevProblem& p, const float* ts_dev, int T, const float* y0, float* y_out, const float* dW,
                  uint64_t seed, int64_t trial_offset, float dt, int adaptive, float rtol, float atol, float dt_min,
                  int* n_accept, int* n_reject, int* status, float* y_steps, void* ws, size_t ws_bytes, cudaStream_t s) {
-    static const bool f16_env = [] { const char* e = getenv("ODECOL_EM16"); return e ? atoi(e) != 0 : true; }();
-    int rc = em_fwd_impl(p, ts_dev, T, y0, y_out, dW, seed, trial_offset, dt, adaptive, rtol, atol, dt_min, n_accept, n_reject,
-                         status, y_steps, ws, ws_bytes, s, f16_env);
-    if (rc == kRetryTf32)
-        rc = em_fwd_impl(p, ts_dev, T, y0, y_out, dW, seed, trial_offset, dt, adaptive, rtol, atol, dt_min, n_accept, n_reject,
-                         status, y_steps, ws, ws_bytes, s, false);
-    return rc;
+    return tc::solve_f16_or_tf32(tc::kEm16, true, [&](bool f16) {
+        return em_fwd_impl(p, ts_dev, T, y0, y_out, dW, seed, trial_offset, dt, adaptive, rtol, atol, dt_min, n_accept, n_reject,
+                           status, y_steps, ws, ws_bytes, s, f16);
+    });
 }
 
 
@@ -704,24 +789,9 @@ int stage_drift(const DevProblem& p, const float* t_trial, const float* y, float
     const EmLayout L = em_layout(p);
     if (!ws || ws_bytes < L.total) return ODECOL_E_WORKSPACE;
     if (p.N % 4 != 0) return ODECOL_E_UNSUPPORTED;
-    char* w = static_cast<char*>(ws);
-    auto F = [&](size_t off) { return reinterpret_cast<float*>(w + off); };
-    float *Whi = F(L.off_Whi), *Wlo = F(L.off_Wlo), *Rhi = F(L.off_Rhi), *Rlo = F(L.off_Rlo);
-    const int Kaug = p.N + p.n_in + 1;
-    if (cudaMemsetAsync(w + L.off_Rhi, 0, L.off_f - L.off_Rhi, s) != cudaSuccess) return ODECOL_E_CUDA;
-    k_split_pad<<<296, 256, 0, s>>>(p.W_aug, p.N, Kaug, p.ld_w, Whi, Wlo, L.Np, L.KPa);
-    float* loc = p.lat_gain ? F(L.off_loc) : nullptr;
-    k_em_operand<<<p.B, 128, 0, s>>>(p, y, t_trial, 0.f, Rhi, Rlo, L.KPa, nullptr, loc);
-    count_launch(2);
-    CUtensorMap mWhi, mWlo, mRhi, mRlo;
-    if (!make_map(&mWhi, Whi, L.Np, L.KPa, L.KPa, BM) || !make_map(&mWlo, Wlo, L.Np, L.KPa, L.KPa, BM) ||
-        !make_map(&mRhi, Rhi, L.Bp, L.KPa, L.KPa, L.TN) || !make_map(&mRlo, Rlo, L.Bp, L.KPa, L.KPa, L.TN))
-        return ODECOL_E_CUDA;
-    const TileShape tsh{L.Np / BM, L.Bp / L.TN, L.TN, L.KPa / BK, 0};
-    RhsEpi e;
-    e.p = p; e.y = y; e.Rhi = Rhi; e.Rlo = Rlo; e.f = f; e.KPa = L.KPa; e.loc = loc;
-    e.inv_tm = 1.0f / p.c.tau_m; e.inv_ta = 1.0f / p.c.tau_a; e.inv_ts = 1.0f / p.c.tau_s;
-    return launch_contract(mWhi, mWlo, mRhi, mRlo, tsh, e, s);
+    StagedDrift drift;
+    const int rc = drift.init(p, static_cast<char*>(ws), L.drift, false, s);
+    return rc != ODECOL_OK ? rc : drift.eval(0, y, t_trial, 0.f, f);
 }
 
 
@@ -923,27 +993,19 @@ __global__ void k_dp_finish(DevProblem p, DpState s, const float* __restrict__ t
 }
 
 struct DpLayout {
-    int Np, Bp, KPa, KP16, TN;
-    size_t off_Whi, off_Wlo, off_Rhi, off_Rlo, off_k[7], off_y, off_ys, off_state, off_aux, total;
+    DriftLayout drift;
+    size_t off_k[7], off_y, off_ys, off_state, total;
 };
 
 static DpLayout dp_layout(const DevProblem& p) {
     DpLayout L;
-    L.Np = round_up(p.N, BM);
-    L.KPa = round_up(p.N + p.n_in + 1, BK);
-    L.TN = pick_tile_n(L.Np / BM, p.B);
-    L.Bp = round_up(p.B, L.TN);
-    size_t o = 0;
-    auto take = [&](size_t bytes) { const size_t r = o; o += (bytes + 1023) / 1024 * 1024; return r; };
-    L.off_Whi = take(4ull * L.Np * L.KPa); L.off_Wlo = take(4ull * L.Np * L.KPa);
-    L.off_Rhi = take(4ull * L.Bp * L.KPa); L.off_Rlo = take(4ull * L.Bp * L.KPa);
+    Carve c;
+    L.drift = drift_layout(c, p, 1, /*loc=*/false, /*aux=*/true, /*dw_rows=*/false);
     const size_t st = 4ull * p.B * 3 * p.N;
-    for (int i = 0; i < 7; ++i) L.off_k[i] = take(st);
-    L.off_y = take(st); L.off_ys = take(st);
-    L.off_state = take(64ull * p.B + 1024);
-    L.off_aux = take(64);                                       // 16-bit operand format: 1 / weight scale, max|W| scratch, overflow flag
-    L.KP16 = round_up(p.N + p.n_in + 1, BK16);                  // its rows live in the same buffers (2 KP16 <= 4 KPa bytes)
-    L.total = o;
+    for (int i = 0; i < 7; ++i) L.off_k[i] = c.take(st);
+    L.off_y = c.take(st); L.off_ys = c.take(st);
+    L.off_state = c.take(64ull * p.B + 1024);
+    L.total = c.o;
     return L;
 }
 
@@ -960,113 +1022,59 @@ static int dopri5_fwd_impl(const DevProblem& p, const float* ts_dev, int T, cons
     if (!ws || ws_bytes < L.total) return ODECOL_E_WORKSPACE;
     if (p.N % 4 != 0) return ODECOL_E_UNSUPPORTED;
     char* w = static_cast<char*>(ws);
-    auto F = [&](size_t off) { return reinterpret_cast<float*>(w + off); };
-    float *Whi = F(L.off_Whi), *Wlo = F(L.off_Wlo), *Rhi = F(L.off_Rhi), *Rlo = F(L.off_Rlo);
-    const int Kaug = p.N + p.n_in + 1;
     const size_t st = (size_t)p.B * 3 * p.N;
     const size_t B = p.B;
     DpState S;
-    for (int i = 0; i < 7; ++i) S.k[i] = F(L.off_k[i]);
-    S.y = F(L.off_y); S.ys = F(L.off_ys);
-    char* sb = w + L.off_state;
-    auto grab = [&](size_t bytes) { char* r = sb; sb += (bytes + 15) / 16 * 16; return r; };
-    S.t = reinterpret_cast<double*>(grab(8 * B)); S.dt = reinterpret_cast<double*>(grab(8 * B));
-    S.red = reinterpret_cast<double*>(grab(16 * B));
-    S.t_stage = reinterpret_cast<float*>(grab(4 * B));
-    S.next_out = reinterpret_cast<int*>(grab(4 * B)); S.n_acc = reinterpret_cast<int*>(grab(4 * B));
-    S.n_rej = reinterpret_cast<int*>(grab(4 * B)); S.status = reinterpret_cast<int*>(grab(4 * B));
-    S.active = reinterpret_cast<int*>(grab(4 * B));
-    S.n_active = reinterpret_cast<int*>(grab(16));
+    for (int i = 0; i < 7; ++i) S.k[i] = reinterpret_cast<float*>(w + L.off_k[i]);
+    S.y = reinterpret_cast<float*>(w + L.off_y); S.ys = reinterpret_cast<float*>(w + L.off_ys);
+    TrialCarve g{w + L.off_state};
+    g(S.t, B); g(S.dt, B); g(S.red, 2 * B); g(S.t_stage, B);
+    g(S.next_out, B); g(S.n_acc, B); g(S.n_rej, B); g(S.status, B); g(S.active, B);
+    g(S.n_active, 1);
 
-    if (cudaMemsetAsync(w + L.off_Rhi, 0, L.off_k[0] - L.off_Rhi, s) != cudaSuccess) return ODECOL_E_CUDA;
-    float* aux = F(L.off_aux);                                  // [0] 1 / weight scale, [1] max|W| bits, [2] overflow flag
-    unsigned int* ovf = f16 ? reinterpret_cast<unsigned int*>(aux + 2) : nullptr;
-    const int KPr = f16 ? L.KP16 : L.KPa;                       // elements per operand row in the format in use
-    if (f16) {
-        if (cudaMemsetAsync(aux, 0, 64, s) != cudaSuccess) return ODECOL_E_CUDA;
-        k_absmax<<<148, 256, 0, s>>>(p.W_aug, p.N, Kaug, p.ld_w, reinterpret_cast<unsigned int*>(aux + 1));
-        k_split16_w<<<296, 256, 0, s>>>(p.W_aug, p.N, Kaug, p.ld_w, reinterpret_cast<__half*>(Whi), reinterpret_cast<__half*>(Wlo),
-                                        L.Np, L.KP16, reinterpret_cast<unsigned int*>(aux + 1), aux);
-        count_launch(2);
-    } else {
-        k_split_pad<<<296, 256, 0, s>>>(p.W_aug, p.N, Kaug, p.ld_w, Whi, Wlo, L.Np, L.KPa);
-        count_launch();
-    }
+    StagedDrift drift;
+    int rc = drift.init(p, w, L.drift, f16, s);
+    if (rc != ODECOL_OK) return rc;
     if (cudaMemcpyAsync(S.y, y0, sizeof(float) * st, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
     if (cudaMemcpyAsync(y_out, y0, sizeof(float) * st, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
-    CUtensorMap mWhi, mWlo, mRhi, mRlo;
-    if (f16) {
-        if (!make_map16(&mWhi, Whi, L.Np, L.KP16, L.KP16, BM, false) || !make_map16(&mWlo, Wlo, L.Np, L.KP16, L.KP16, BM, false) ||
-            !make_map16(&mRhi, Rhi, L.Bp, L.KP16, L.KP16, L.TN, false) || !make_map16(&mRlo, Rlo, L.Bp, L.KP16, L.KP16, L.TN, false))
-            return ODECOL_E_CUDA;
-    } else if (!make_map(&mWhi, Whi, L.Np, L.KPa, L.KPa, BM) || !make_map(&mWlo, Wlo, L.Np, L.KPa, L.KPa, BM) ||
-               !make_map(&mRhi, Rhi, L.Bp, L.KPa, L.KPa, L.TN) || !make_map(&mRlo, Rlo, L.Bp, L.KPa, L.KPa, L.TN))
-        return ODECOL_E_CUDA;
-    const TileShape tsh{L.Np / BM, L.Bp / L.TN, L.TN, f16 ? L.KP16 / BK16 : L.KPa / BK, 0};
-    // f(t_stage[b], ysrc[b]) -> fdst for every trial (finished trials compute along harmlessly: rows are independent)
-    auto rhs = [&](const float* ysrc, const float* t_trial, float t_shared, float* fdst) {
-        k_em_operand<<<p.B, 128, 0, s>>>(p, ysrc, t_trial, t_shared, Rhi, Rlo, KPr, nullptr, nullptr, ovf);
-        count_launch();
-        RhsEpi e;
-        e.p = p; e.y = ysrc; e.Rhi = Rhi; e.Rlo = Rlo; e.f = fdst; e.KPa = KPr; e.loc = nullptr; e.wscale = f16 ? aux : nullptr;
-        e.inv_tm = 1.0f / p.c.tau_m; e.inv_ta = 1.0f / p.c.tau_a; e.inv_ts = 1.0f / p.c.tau_s;
-        if (f16) return launch_contract16(mWhi, mWlo, mRhi, mRlo, tsh, e, s);
-        return launch_contract(mWhi, mWlo, mRhi, mRlo, tsh, e, s);
-    };
-    const int ew_grid = (int)((st + 255) / 256 < 148 * 16 ? (st + 255) / 256 : 148 * 16);
+    const int eg = ew_grid(st);
     float t_first = 0.f;
     if (cudaMemcpyAsync(&t_first, ts_dev, sizeof(float), cudaMemcpyDeviceToHost, s) != cudaSuccess) return ODECOL_E_CUDA;
     if (cudaStreamSynchronize(s) != cudaSuccess) return ODECOL_E_CUDA;
-    int rc = rhs(S.y, nullptr, t_first, S.k[0]);                    // f0 = f(t[0], y0)
-    if (rc != ODECOL_OK) return rc;
+    // f(t_stage[b], ys[b]) -> k[stage] for every trial (finished trials compute along harmlessly: rows are independent)
+    if ((rc = drift.eval(0, S.y, nullptr, t_first, S.k[0])) != ODECOL_OK) return rc;        // f0 = f(t[0], y0)
     k_dp_init1<<<p.B, 256, 0, s>>>(p, S, ts_dev, rtol, atol);
-    rc = rhs(S.ys, S.t_stage, 0.f, S.k[1]);                         // f(t0 + h0, y0 + h0 f0)
-    if (rc != ODECOL_OK) return rc;
+    if ((rc = drift.eval(0, S.ys, S.t_stage, 0.f, S.k[1])) != ODECOL_OK) return rc;         // f(t0 + h0, y0 + h0 f0)
     k_dp_init2<<<p.B, 256, 0, s>>>(p, S, rtol, atol);
     count_launch(2);
     int h_active = p.B;
-    unsigned int h_ovf = 0;
     for (long long round = 0; round < (long long)max_steps && h_active > 0; ++round) {
-        k_dp_stage<1><<<ew_grid, 256, 0, s>>>(p, S); rc = rhs(S.ys, S.t_stage, 0.f, S.k[1]); if (rc) return rc;
-        k_dp_stage<2><<<ew_grid, 256, 0, s>>>(p, S); rc = rhs(S.ys, S.t_stage, 0.f, S.k[2]); if (rc) return rc;
-        k_dp_stage<3><<<ew_grid, 256, 0, s>>>(p, S); rc = rhs(S.ys, S.t_stage, 0.f, S.k[3]); if (rc) return rc;
-        k_dp_stage<4><<<ew_grid, 256, 0, s>>>(p, S); rc = rhs(S.ys, S.t_stage, 0.f, S.k[4]); if (rc) return rc;
-        k_dp_stage<5><<<ew_grid, 256, 0, s>>>(p, S); rc = rhs(S.ys, S.t_stage, 0.f, S.k[5]); if (rc) return rc;
-        k_dp_stage<6><<<ew_grid, 256, 0, s>>>(p, S); rc = rhs(S.ys, S.t_stage, 0.f, S.k[6]); if (rc) return rc;
+        k_dp_stage<1><<<eg, 256, 0, s>>>(p, S); rc = drift.eval(0, S.ys, S.t_stage, 0.f, S.k[1]); if (rc) return rc;
+        k_dp_stage<2><<<eg, 256, 0, s>>>(p, S); rc = drift.eval(0, S.ys, S.t_stage, 0.f, S.k[2]); if (rc) return rc;
+        k_dp_stage<3><<<eg, 256, 0, s>>>(p, S); rc = drift.eval(0, S.ys, S.t_stage, 0.f, S.k[3]); if (rc) return rc;
+        k_dp_stage<4><<<eg, 256, 0, s>>>(p, S); rc = drift.eval(0, S.ys, S.t_stage, 0.f, S.k[4]); if (rc) return rc;
+        k_dp_stage<5><<<eg, 256, 0, s>>>(p, S); rc = drift.eval(0, S.ys, S.t_stage, 0.f, S.k[5]); if (rc) return rc;
+        k_dp_stage<6><<<eg, 256, 0, s>>>(p, S); rc = drift.eval(0, S.ys, S.t_stage, 0.f, S.k[6]); if (rc) return rc;
         k_dp_finish<<<p.B, 256, 0, s>>>(p, S, ts_dev, T, rtol, atol, max_steps, y_out, rec);
         count_launch(7);
         if ((round & 15) == 15) {
             if (cudaMemcpyAsync(&h_active, S.n_active, sizeof(int), cudaMemcpyDeviceToHost, s) != cudaSuccess) return ODECOL_E_CUDA;
-            if (f16 && cudaMemcpyAsync(&h_ovf, ovf, sizeof(h_ovf), cudaMemcpyDeviceToHost, s) != cudaSuccess) return ODECOL_E_CUDA;
-            if (cudaStreamSynchronize(s) != cudaSuccess) return ODECOL_E_CUDA;
-            if (h_ovf) return kRetryTf32;
+            if ((rc = drift.overflowed()) != ODECOL_OK) return rc;
         }
     }
-    if (f16) {                                                // rounds since the last poll
-        if (cudaMemcpyAsync(&h_ovf, ovf, sizeof(h_ovf), cudaMemcpyDeviceToHost, s) != cudaSuccess) return ODECOL_E_CUDA;
-        if (cudaStreamSynchronize(s) != cudaSuccess) return ODECOL_E_CUDA;
-        if (h_ovf) return kRetryTf32;
-    }
-    k_em_fill_nan<<<p.B, 128, 0, s>>>(p, S.status, S.next_out, T, y_out);
-    count_launch();
-    if (n_accept && cudaMemcpyAsync(n_accept, S.n_acc, sizeof(int) * B, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
-    if (n_reject && cudaMemcpyAsync(n_reject, S.n_rej, sizeof(int) * B, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
-    if (status && cudaMemcpyAsync(status, S.status, sizeof(int) * B, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
-    return cudaGetLastError() == cudaSuccess ? ODECOL_OK : ODECOL_E_CUDA;
+    if (f16 && (rc = drift.overflowed()) != ODECOL_OK) return rc;         // rounds since the last poll
+    return adaptive_finish(p, S, T, y_out, n_accept, n_reject, status, s);
 }
 
 int stage_dopri5_fwd(const DevProblem& p, const float* ts_dev, int T, const float* y0, float* y_out, float rtol, float atol,
                      int max_steps, int* n_accept, int* n_reject, int* status, const Dopri5Record& rec, void* ws,
                      size_t ws_bytes, cudaStream_t s) {
-    static const bool f16_env = [] { const char* e = getenv("ODECOL_DP16"); return e ? atoi(e) != 0 : true; }();
     // Forward-only solves take the 16-bit format.  Training (rec.y != NULL) stays on TF32 pairs: on the stiff parity network the
     // discrete adjoint through a stability-limited step sequence is ill-conditioned (on-chip and staged TF32 gradients already
     // differ by 2e-2 there), and the step sequence the FP16 rounding produced amplified it 300-fold (profiles/r2_session4.md).
-    const bool f16 = f16_env && rec.y == nullptr;
-    int rc = dopri5_fwd_impl(p, ts_dev, T, y0, y_out, rtol, atol, max_steps, n_accept, n_reject, status, rec, ws, ws_bytes, s, f16);
-    if (rc == kRetryTf32)
-        rc = dopri5_fwd_impl(p, ts_dev, T, y0, y_out, rtol, atol, max_steps, n_accept, n_reject, status, rec, ws, ws_bytes, s, false);
-    return rc;
+    return tc::solve_f16_or_tf32(tc::kDp16, rec.y == nullptr, [&](bool f16) {
+        return dopri5_fwd_impl(p, ts_dev, T, y0, y_out, rtol, atol, max_steps, n_accept, n_reject, status, rec, ws, ws_bytes, s, f16);
+    });
 }
 
 
@@ -1159,89 +1167,40 @@ static int srk_fwd_impl(const DevProblem& p, const float* ts_dev, int T, const f
     if (p.N % 4 != 0) return ODECOL_E_UNSUPPORTED;
     char* w = static_cast<char*>(ws);
     auto F = [&](size_t off) { return reinterpret_cast<float*>(w + off); };
-    float *Whi = F(L.off_Whi), *Wlo = F(L.off_Wlo), *Rhi = F(L.off_Rhi), *Rlo = F(L.off_Rlo);
     float *f0 = F(L.off_f), *f1 = F(L.off_fm), *f2 = F(L.off_yfull), *H = F(L.off_ymid);
     float *y = F(L.off_y), *yprev = F(L.off_yprev);
     SrkNoise nz;
     nz.dw = F(L.off_state); nz.du = nz.dw + p.B; nz.gw = nz.du + p.B;          // 6 floats per trial of the 128-byte slot
-    const int Kaug = p.N + p.n_in + 1;
     const size_t st = (size_t)p.B * 3 * p.N;
-    if (cudaMemsetAsync(w + L.off_Rhi, 0, L.off_f - L.off_Rhi, s) != cudaSuccess) return ODECOL_E_CUDA;
-    float* aux = F(L.off_aux);                                  // [0] 1 / weight scale, [1] max|W| bits, [2] overflow flag
-    unsigned int* ovf = f16 ? reinterpret_cast<unsigned int*>(aux + 2) : nullptr;
-    const int KPr = f16 ? L.KP16 : L.KPa;                       // elements per operand row in the format in use
-    if (f16) {
-        if (cudaMemsetAsync(aux, 0, 64, s) != cudaSuccess) return ODECOL_E_CUDA;
-        k_absmax<<<148, 256, 0, s>>>(p.W_aug, p.N, Kaug, p.ld_w, reinterpret_cast<unsigned int*>(aux + 1));
-        k_split16_w<<<296, 256, 0, s>>>(p.W_aug, p.N, Kaug, p.ld_w, reinterpret_cast<__half*>(Whi), reinterpret_cast<__half*>(Wlo),
-                                        L.Np, L.KP16, reinterpret_cast<unsigned int*>(aux + 1), aux);
-        count_launch(2);
-    } else {
-        k_split_pad<<<296, 256, 0, s>>>(p.W_aug, p.N, Kaug, p.ld_w, Whi, Wlo, L.Np, L.KPa);
-        count_launch();
-    }
+    StagedDrift drift;
+    int rc = drift.init(p, w, L.drift, f16, s);
+    if (rc != ODECOL_OK) return rc;
     if (cudaMemcpyAsync(y, y0, sizeof(float) * st, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
     if (cudaMemcpyAsync(y_out, y0, sizeof(float) * st, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
     if (y_steps && cudaMemcpyAsync(y_steps, y0, sizeof(float) * st, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
-    CUtensorMap mWhi, mWlo, mRhi, mRlo;
-    if (f16) {
-        if (!make_map16(&mWhi, Whi, L.Np, L.KP16, L.KP16, BM, false) || !make_map16(&mWlo, Wlo, L.Np, L.KP16, L.KP16, BM, false) ||
-            !make_map16(&mRhi, Rhi, L.Bp, L.KP16, L.KP16, L.TN, false) || !make_map16(&mRlo, Rlo, L.Bp, L.KP16, L.KP16, L.TN, false))
-            return ODECOL_E_CUDA;
-    } else if (!make_map(&mWhi, Whi, L.Np, L.KPa, L.KPa, BM) || !make_map(&mWlo, Wlo, L.Np, L.KPa, L.KPa, BM) ||
-               !make_map(&mRhi, Rhi, L.Bp, L.KPa, L.KPa, L.TN) || !make_map(&mRlo, Rlo, L.Bp, L.KPa, L.KPa, L.TN))
-        return ODECOL_E_CUDA;
-    const TileShape tsh{L.Np / BM, L.Bp / L.TN, L.TN, f16 ? L.KP16 / BK16 : L.KPa / BK, 0};
-    auto rhs = [&](const float* ysrc, float tq, float* fdst) {
-        k_em_operand<<<p.B, 128, 0, s>>>(p, ysrc, nullptr, tq, Rhi, Rlo, KPr, nullptr, nullptr, ovf);
-        count_launch();
-        RhsEpi e;
-        e.p = p; e.y = ysrc; e.Rhi = Rhi; e.Rlo = Rlo; e.f = fdst; e.KPa = KPr; e.loc = nullptr; e.wscale = f16 ? aux : nullptr;
-        e.inv_tm = 1.0f / p.c.tau_m; e.inv_ta = 1.0f / p.c.tau_a; e.inv_ts = 1.0f / p.c.tau_s;
-        if (f16) return launch_contract16(mWhi, mWlo, mRhi, mRlo, tsh, e, s);
-        return launch_contract(mWhi, mWlo, mRhi, mRlo, tsh, e, s);
-    };
-    const int ew_grid = (int)((st + 255) / 256 < 148 * 16 ? (st + 255) / 256 : 148 * 16);
-    std::vector<float> ts(T);
-    if (cudaMemcpyAsync(ts.data(), ts_dev, sizeof(float) * T, cudaMemcpyDeviceToHost, s) != cudaSuccess) return ODECOL_E_CUDA;
-    if (cudaStreamSynchronize(s) != cudaSuccess) return ODECOL_E_CUDA;
-    volatile float curr = ts[0];
-    const float t_end = ts[T - 1];
-    long long k = 0;
-    int j = 1;
-    while (j < T) {
-        const float c0 = curr;
-        volatile float nx = c0 + dt;
-        const float next_t = nx < t_end ? nx : t_end;
-        volatile float hv = next_t - c0;
+    const int eg = ew_grid(st);
+    long long n_steps = 0;
+    rc = fixed_step_walk(ts_dev, T, dt, s, n_steps, [&](long long k, float t0, float t1, int j_lo, int j_hi) -> int {
+        volatile float hv = t1 - t0;
         const float h = hv;
-        volatile float t1v = c0 + h, thv = c0 + 0.5f * h;           // stage times in float32, as the on-chip kernel forms them
-        int j_hi = j;
-        while (j_hi < T && ts[j_hi] <= next_t) ++j_hi;
+        volatile float t1v = t0 + h, thv = t0 + 0.5f * h;           // stage times in float32, as the on-chip kernel forms them
         k_srk_noise<<<(p.B + 127) / 128, 128, 0, s>>>(p, nz, dW, dU, (unsigned long long)seed, (long long)trial_offset, k, h);
-        int rc = rhs(y, c0, f0); if (rc) return rc;
-        k_srk_stage<<<ew_grid, 256, 0, s>>>(p, nz, 1, y, f0, f1, h, H);
-        rc = rhs(H, t1v, f1); if (rc) return rc;
-        k_srk_stage<<<ew_grid, 256, 0, s>>>(p, nz, 2, y, f0, f1, h, H);
-        rc = rhs(H, thv, f2); if (rc) return rc;
+        int r = drift.eval(0, y, nullptr, t0, f0); if (r) return r;
+        k_srk_stage<<<eg, 256, 0, s>>>(p, nz, 1, y, f0, f1, h, H);
+        r = drift.eval(0, H, nullptr, t1v, f1); if (r) return r;
+        k_srk_stage<<<eg, 256, 0, s>>>(p, nz, 2, y, f0, f1, h, H);
+        r = drift.eval(0, H, nullptr, thv, f2); if (r) return r;
         SrkStepArgs a;
-        a.p = p; a.nz = nz; a.y = y; a.y_prev = yprev; a.f0 = f0; a.f1 = f1; a.f2 = f2; a.t0 = c0; a.t1 = next_t;
-        a.y_out = y_out; a.j_lo = j; a.j_hi = j_hi; a.ts = ts_dev;
-        k_srk_step<<<ew_grid, 256, 0, s>>>(a);
+        a.p = p; a.nz = nz; a.y = y; a.y_prev = yprev; a.f0 = f0; a.f1 = f1; a.f2 = f2; a.t0 = t0; a.t1 = t1;
+        a.y_out = y_out; a.j_lo = j_lo; a.j_hi = j_hi; a.ts = ts_dev;
+        k_srk_step<<<eg, 256, 0, s>>>(a);
         count_launch(4);
-        curr = next_t;
-        j = j_hi;
-        ++k;
-        if (y_steps && cudaMemcpyAsync(y_steps + (size_t)k * st, y, sizeof(float) * st, cudaMemcpyDeviceToDevice, s) != cudaSuccess)
+        if (y_steps && cudaMemcpyAsync(y_steps + (size_t)(k + 1) * st, y, sizeof(float) * st, cudaMemcpyDeviceToDevice, s) != cudaSuccess)
             return ODECOL_E_CUDA;
-        if (k > (1LL << 40)) return ODECOL_E_SHAPE;
-    }
-    if (f16) {                                                // did every operand value fit FP16?
-        unsigned int h_ovf = 0;
-        if (cudaMemcpyAsync(&h_ovf, ovf, sizeof(h_ovf), cudaMemcpyDeviceToHost, s) != cudaSuccess) return ODECOL_E_CUDA;
-        if (cudaStreamSynchronize(s) != cudaSuccess) return ODECOL_E_CUDA;
-        if (h_ovf) return kRetryTf32;
-    }
+        return ODECOL_OK;
+    });
+    if (rc != ODECOL_OK) return rc;
+    if (f16 && (rc = drift.overflowed()) != ODECOL_OK) return rc;         // did every operand value fit FP16?
     if (status) { k_status_finite<<<p.B, 128, 0, s>>>(p, y, status); count_launch(); }
     return cudaGetLastError() == cudaSuccess ? ODECOL_OK : ODECOL_E_CUDA;
 }
@@ -1249,11 +1208,9 @@ static int srk_fwd_impl(const DevProblem& p, const float* ts_dev, int T, const f
 int stage_srk_fwd(const DevProblem& p, const float* ts_dev, int T, const float* y0, float* y_out, const float* dW,
                   const float* dU, uint64_t seed, int64_t trial_offset, float dt, int* status, float* y_steps, void* ws,
                   size_t ws_bytes, cudaStream_t s) {
-    static const bool f16_env = [] { const char* e = getenv("ODECOL_SRK16"); return e ? atoi(e) != 0 : true; }();
-    int rc = srk_fwd_impl(p, ts_dev, T, y0, y_out, dW, dU, seed, trial_offset, dt, status, y_steps, ws, ws_bytes, s, f16_env);
-    if (rc == kRetryTf32)
-        rc = srk_fwd_impl(p, ts_dev, T, y0, y_out, dW, dU, seed, trial_offset, dt, status, y_steps, ws, ws_bytes, s, false);
-    return rc;
+    return tc::solve_f16_or_tf32(tc::kSrk16, true, [&](bool f16) {
+        return srk_fwd_impl(p, ts_dev, T, y0, y_out, dW, dU, seed, trial_offset, dt, status, y_steps, ws, ws_bytes, s, f16);
+    });
 }
 
 
@@ -1358,33 +1315,30 @@ __global__ void k_add_out_grad(DevProblem p, const float* __restrict__ grad_row,
 }
 
 struct AdjLayout {
-    int Np, Bp, Bp32, KPa, NPk, TN;
-    size_t off_Whi, off_Wlo, off_WThi, off_WTlo, off_Rhi, off_Rlo, off_AVhi, off_AVlo, off_D;
+    DriftLayout drift;          // TF32; operand planes of Bp32 rows
+    int NPk;
+    size_t off_AVhi, off_AVlo, off_WThi, off_WTlo, off_D;
     size_t off_lam, off_pend, off_a, off_b[3], off_f[2], off_H[2], off_noise, total;
 };
 
 static AdjLayout adj_layout(const DevProblem& p) {
     AdjLayout L;
-    L.Np = round_up(p.N, BM);
-    L.NPk = L.Np;
-    L.KPa = round_up(p.N + p.n_in + 1, BK);
-    L.TN = pick_tile_n(L.Np / BM, p.B);
-    L.Bp = round_up(p.B, L.TN);
-    L.Bp32 = round_up(L.Bp, 32);
-    size_t o = 0;
-    auto take = [&](size_t bytes) { const size_t r = o; o += (bytes + 1023) / 1024 * 1024; return r; };
-    L.off_Whi = take(4ull * L.Np * L.KPa); L.off_Wlo = take(4ull * L.Np * L.KPa);
-    L.off_WThi = take(4ull * L.Np * L.NPk); L.off_WTlo = take(4ull * L.Np * L.NPk);
-    L.off_Rhi = take(4ull * L.Bp32 * L.KPa); L.off_Rlo = take(4ull * L.Bp32 * L.KPa);
-    L.off_AVhi = take(4ull * L.Bp32 * L.NPk); L.off_AVlo = take(4ull * L.Bp32 * L.NPk);
-    L.off_D = take(4ull * p.B * p.N);
+    Carve c;
+    L.drift = drift_layout(c, p, 1, /*loc=*/false, /*aux=*/false, /*dw_rows=*/true);
+    const int Np = L.drift.Np, rows = L.drift.rows;
+    L.NPk = Np;
+    // the gamma a_V operand right behind r_aug: the drift's init zeroes both
+    L.off_AVhi = c.take(4ull * rows * L.NPk); L.off_AVlo = c.take(4ull * rows * L.NPk);
+    L.drift.zero_end = c.o;
+    L.off_WThi = c.take(4ull * Np * L.NPk); L.off_WTlo = c.take(4ull * Np * L.NPk);
+    L.off_D = c.take(4ull * p.B * p.N);
     const size_t st = 4ull * p.B * 3 * p.N;
-    L.off_lam = take(st); L.off_pend = take(st); L.off_a = take(st);
-    for (int i = 0; i < 3; ++i) L.off_b[i] = take(st);
-    for (int i = 0; i < 2; ++i) L.off_f[i] = take(st);
-    for (int i = 0; i < 2; ++i) L.off_H[i] = take(st);
-    L.off_noise = take(32ull * p.B + 64);
-    L.total = o;
+    L.off_lam = c.take(st); L.off_pend = c.take(st); L.off_a = c.take(st);
+    for (int i = 0; i < 3; ++i) L.off_b[i] = c.take(st);
+    for (int i = 0; i < 2; ++i) L.off_f[i] = c.take(st);
+    for (int i = 0; i < 2; ++i) L.off_H[i] = c.take(st);
+    L.off_noise = c.take(32ull * p.B + 64);
+    L.total = c.o;
     return L;
 }
 
@@ -1404,8 +1358,9 @@ static __global__ void k_split_pad_WT(const float* __restrict__ src, int n, int 
 // shared state of a staged reverse sweep
 struct AdjCtx {
     DevProblem p; AdjLayout L; cudaStream_t s; char* w;
-    CUtensorMap mWhi, mWlo, mWThi, mWTlo, mRhi, mRlo, mAVhi, mAVlo;
-    TileShape tsF, tsB;
+    StagedDrift drift;                  // f = drift(Y, t); its operand set also holds r_aug(Y, t) for the VJPs
+    CUtensorMap mWThi, mWTlo, mAVhi, mAVlo;
+    TileShape tsB;
     float gamma;
     float* grad_W;
     float* F(size_t off) const { return reinterpret_cast<float*>(w + off); }
@@ -1415,71 +1370,39 @@ struct AdjCtx {
         if (!ws || ws_bytes < L.total) return ODECOL_E_WORKSPACE;
         if (p.N % 4 != 0) return ODECOL_E_UNSUPPORTED;
         gamma = p.c.tau_s * p.c.R / p.c.tau_m;
-        const int Kaug = p.N + p.n_in + 1;
-        if (cudaMemsetAsync(w + L.off_Rhi, 0, L.off_D - L.off_Rhi, s) != cudaSuccess) return ODECOL_E_CUDA;
         if (cudaMemsetAsync(w + L.off_lam, 0, L.off_a - L.off_lam, s) != cudaSuccess) return ODECOL_E_CUDA;
         if (cudaMemsetAsync(grad_W, 0, sizeof(float) * (size_t)p.N * p.ld_w, s) != cudaSuccess) return ODECOL_E_CUDA;
-        k_split_pad<<<296, 256, 0, s>>>(p.W_aug, p.N, Kaug, p.ld_w, F(L.off_Whi), F(L.off_Wlo), L.Np, L.KPa);
-        k_split_pad_WT<<<296, 256, 0, s>>>(p.W_aug, p.N, p.ld_w, F(L.off_WThi), F(L.off_WTlo), L.Np, L.NPk);
-        count_launch(2);
-        if (!make_map(&mWhi, F(L.off_Whi), L.Np, L.KPa, L.KPa, BM) || !make_map(&mWlo, F(L.off_Wlo), L.Np, L.KPa, L.KPa, BM) ||
-            !make_map(&mWThi, F(L.off_WThi), L.Np, L.NPk, L.NPk, BM) || !make_map(&mWTlo, F(L.off_WTlo), L.Np, L.NPk, L.NPk, BM) ||
-            !make_map(&mRhi, F(L.off_Rhi), L.Bp, L.KPa, L.KPa, L.TN) || !make_map(&mRlo, F(L.off_Rlo), L.Bp, L.KPa, L.KPa, L.TN) ||
-            !make_map(&mAVhi, F(L.off_AVhi), L.Bp, L.NPk, L.NPk, L.TN) || !make_map(&mAVlo, F(L.off_AVlo), L.Bp, L.NPk, L.NPk, L.TN))
+        const int rc = drift.init(p, w, L.drift, false, s);
+        if (rc != ODECOL_OK) return rc;
+        const DriftLayout& D = L.drift;
+        k_split_pad_WT<<<296, 256, 0, s>>>(p.W_aug, p.N, p.ld_w, F(L.off_WThi), F(L.off_WTlo), D.Np, L.NPk);
+        count_launch();
+        if (!make_map(&mWThi, F(L.off_WThi), D.Np, L.NPk, L.NPk, BM) || !make_map(&mWTlo, F(L.off_WTlo), D.Np, L.NPk, L.NPk, BM) ||
+            !make_map(&mAVhi, F(L.off_AVhi), D.Bp, L.NPk, L.NPk, D.TN) || !make_map(&mAVlo, F(L.off_AVlo), D.Bp, L.NPk, L.NPk, D.TN))
             return ODECOL_E_CUDA;
-        tsF = TileShape{L.Np / BM, L.Bp / L.TN, L.TN, L.KPa / BK, 0};
-        tsB = TileShape{L.Np / BM, L.Bp / L.TN, L.TN, L.NPk / BK, 0};
+        tsB = TileShape{D.Np / BM, D.Bp / D.TN, D.TN, L.NPk / BK, 0};
         return ODECOL_OK;
     }
-    int grid(size_t n) const { return (int)((n + 255) / 256 < 148 * 16 ? (n + 255) / 256 : 148 * 16); }
     size_t st() const { return (size_t)p.B * 3 * p.N; }
 
-    // f = drift(Y, t)
-    int rhs(const float* Y, float tq, float* f) {
-        k_em_operand<<<p.B, 128, 0, s>>>(p, Y, nullptr, tq, F(L.off_Rhi), F(L.off_Rlo), L.KPa);
-        count_launch();
-        RhsEpi e;
-        e.p = p; e.y = Y; e.Rhi = F(L.off_Rhi); e.Rlo = F(L.off_Rlo); e.f = f; e.KPa = L.KPa; e.loc = nullptr;
-        e.inv_tm = 1.0f / p.c.tau_m; e.inv_ta = 1.0f / p.c.tau_a; e.inv_ts = 1.0f / p.c.tau_s;
-        return launch_contract(mWhi, mWlo, mRhi, mRlo, tsF, e, s);
-    }
-    // b = J(Y, t)^T a;  grad_W += (gamma a_V)^T r_aug(Y, t)
-    int vjp(const float* Y, float tq, const float* a, float* b) {
-        k_vjp_prep<<<p.B, 128, 0, s>>>(p, Y, tq, a, gamma, F(L.off_Rhi), F(L.off_Rlo), L.KPa, F(L.off_AVhi), F(L.off_AVlo), L.NPk,
-                                       F(L.off_D));
+    // b = J(Y, t)^T a;  grad_W += (gamma a_V)^T r_aug(Y, t).  t_trial != NULL: one time per trial, else t_shared for all;
+    // active != NULL: trials with active[b] == 0 are masked (adaptive solvers)
+    int vjp(const float* Y, const float* t_trial, float t_shared, const int* active, const float* a, float* b) {
+        const DriftLayout& D = L.drift;
+        k_vjp_prep<<<p.B, 128, 0, s>>>(p, Y, t_shared, a, gamma, drift.R[0][0], drift.R[0][1], D.KPa, F(L.off_AVhi), F(L.off_AVlo),
+                                       L.NPk, F(L.off_D), t_trial, active);
         count_launch();
         VjpEpi e;
         e.p = p; e.a = a; e.D = F(L.off_D); e.b = b;
         e.inv_tm = 1.0f / p.c.tau_m; e.inv_ta = 1.0f / p.c.tau_a; e.inv_ts = 1.0f / p.c.tau_s;
         int rc = launch_contract(mWThi, mWTlo, mAVhi, mAVlo, tsB, e, s);
         if (rc) return rc;
-        return tc_dw_accumulate(F(L.off_AVhi), F(L.off_AVlo), F(L.off_Rhi), F(L.off_Rlo), L.Bp32, L.Np, L.KPa, p.N,
-                                p.N + p.n_in + 1, p.ld_w, grad_W, s);
-    }
-    // per-trial evaluation times (adaptive solvers): f = drift(Y, t[b]);  b = J(Y, t[b])^T a with inactive trials masked
-    int rhs_t(const float* Y, const float* t_trial, float* f) {
-        k_em_operand<<<p.B, 128, 0, s>>>(p, Y, t_trial, 0.f, F(L.off_Rhi), F(L.off_Rlo), L.KPa);
-        count_launch();
-        RhsEpi e;
-        e.p = p; e.y = Y; e.Rhi = F(L.off_Rhi); e.Rlo = F(L.off_Rlo); e.f = f; e.KPa = L.KPa; e.loc = nullptr;
-        e.inv_tm = 1.0f / p.c.tau_m; e.inv_ta = 1.0f / p.c.tau_a; e.inv_ts = 1.0f / p.c.tau_s;
-        return launch_contract(mWhi, mWlo, mRhi, mRlo, tsF, e, s);
-    }
-    int vjp_t(const float* Y, const float* t_trial, const int* active, const float* a, float* b) {
-        k_vjp_prep<<<p.B, 128, 0, s>>>(p, Y, 0.f, a, gamma, F(L.off_Rhi), F(L.off_Rlo), L.KPa, F(L.off_AVhi), F(L.off_AVlo), L.NPk,
-                                       F(L.off_D), t_trial, active);
-        count_launch();
-        VjpEpi e;
-        e.p = p; e.a = a; e.D = F(L.off_D); e.b = b;
-        e.inv_tm = 1.0f / p.c.tau_m; e.inv_ta = 1.0f / p.c.tau_a; e.inv_ts = 1.0f / p.c.tau_s;
-        int rc = launch_contract(mWThi, mWTlo, mAVhi, mAVlo, tsB, e, s);
-        if (rc) return rc;
-        return tc_dw_accumulate(F(L.off_AVhi), F(L.off_AVlo), F(L.off_Rhi), F(L.off_Rlo), L.Bp32, L.Np, L.KPa, p.N,
+        return tc_dw_accumulate(F(L.off_AVhi), F(L.off_AVlo), drift.R[0][0], drift.R[0][1], D.rows, D.Np, D.KPa, p.N,
                                 p.N + p.n_in + 1, p.ld_w, grad_W, s);
     }
     void lincomb(float* out, float c0, const float* x0, float c1 = 0.f, const float* x1 = nullptr, float c2 = 0.f,
                  const float* x2 = nullptr, float c3 = 0.f, const float* x3 = nullptr) {
-        k_lincomb<<<grid(st()), 256, 0, s>>>(st(), out, c0, x0, c1, x1, c2, x2, c3, x3);
+        k_lincomb<<<ew_grid(st()), 256, 0, s>>>(st(), out, c0, x0, c1, x1, c2, x2, c3, x3);
         count_launch();
     }
 };
@@ -1539,7 +1462,7 @@ int stage_sde_bwd(int which, const DevProblem& p, const float* ts_dev, int T, co
     float *f0 = cx.F(L.off_f[0]), *f1 = cx.F(L.off_f[1]), *H1 = cx.F(L.off_H[0]), *H2 = cx.F(L.off_H[1]);
     SrkNoise nz;
     nz.dw = cx.F(L.off_noise); nz.du = nz.dw + p.B; nz.gw = nz.du + p.B;
-    const int gg = cx.grid((size_t)p.B * G);
+    const int gg = ew_grid((size_t)p.B * G);
     int j = T - 1;
     for (int k = nsteps - 1; k >= 0; --k) {
         cx.lincomb(lam, 1.f, lam, 1.f, pend);                               // lam += pend
@@ -1555,24 +1478,24 @@ int stage_sde_bwd(int which, const DevProblem& p, const float* ts_dev, int T, co
         const float* yk = y_steps + (size_t)k * st;
         if (which == 0) {
             cx.lincomb(a, h, lam);
-            rc = cx.vjp(yk, t0, a, b0); if (rc) return rc;
+            rc = cx.vjp(yk, nullptr, t0, nullptr, a, b0); if (rc) return rc;
             cx.lincomb(lam, 1.f, lam, 1.f, b0);
         } else {
             volatile float t1v = t0 + h, thv = t0 + 0.5f * h;
             k_srk_noise<<<(p.B + 127) / 128, 128, 0, s>>>(p, nz, dW, dU, (unsigned long long)seed, (long long)trial_offset, k, h);
             count_launch();
-            rc = cx.rhs(yk, t0, f0); if (rc) return rc;
-            k_srk_stage<<<cx.grid(st), 256, 0, s>>>(p, nz, 1, yk, f0, f1, h, H1);
-            rc = cx.rhs(H1, t1v, f1); if (rc) return rc;
-            k_srk_stage<<<cx.grid(st), 256, 0, s>>>(p, nz, 2, yk, f0, f1, h, H2);
+            rc = cx.drift.eval(0, yk, nullptr, t0, f0); if (rc) return rc;
+            k_srk_stage<<<ew_grid(st), 256, 0, s>>>(p, nz, 1, yk, f0, f1, h, H1);
+            rc = cx.drift.eval(0, H1, nullptr, t1v, f1); if (rc) return rc;
+            k_srk_stage<<<ew_grid(st), 256, 0, s>>>(p, nz, 2, yk, f0, f1, h, H2);
             count_launch(2);
             const float h23 = h * Srid2::a2, h6 = h * Srid2::a0, h4 = h * 0.25f;
             cx.lincomb(a, h23, lam);
-            rc = cx.vjp(H2, thv, a, b2); if (rc) return rc;
+            rc = cx.vjp(H2, nullptr, thv, nullptr, a, b2); if (rc) return rc;
             cx.lincomb(a, h6, lam, h4, b2);
-            rc = cx.vjp(H1, t1v, a, b1); if (rc) return rc;
+            rc = cx.vjp(H1, nullptr, t1v, nullptr, a, b1); if (rc) return rc;
             cx.lincomb(a, h6, lam, h4, b2, h, b1);
-            rc = cx.vjp(yk, t0, a, b0); if (rc) return rc;
+            rc = cx.vjp(yk, nullptr, t0, nullptr, a, b0); if (rc) return rc;
             cx.lincomb(lam, 1.f, lam, 1.f, b2, 1.f, b1, 1.f, b0);
         }
     }
@@ -1698,18 +1621,16 @@ __global__ void k_dpb_init(DevProblem p, DpAdj d, int T) {
     if (b < p.B) d.jptr[b] = T - 1;
 }
 
-struct DpAdjLayout { AdjLayout A; DpLayout D; size_t off_planes, off_small, off_inv, total; };
+struct DpAdjLayout { AdjLayout A; size_t off_planes, off_small, off_inv, total; };
 static DpAdjLayout dp_adj_layout(const DevProblem& p) {
     DpAdjLayout L;
     L.A = adj_layout(p);
-    L.D = dp_layout(p);
-    size_t o = L.A.total;
-    auto take = [&](size_t bytes) { const size_t r = o; o += (bytes + 1023) / 1024 * 1024; return r; };
+    Carve c{L.A.total};
     const size_t st = 4ull * p.B * 3 * p.N;
-    L.off_planes = take(26 * st);                                     // Ys, k, kb (7 each), yb0, yb1, lam, carry, bout
-    L.off_small = take(256ull * p.B + 4096);
-    L.off_inv = take(4ull * (3 * p.N + 4));
-    L.total = o;
+    L.off_planes = c.take(26 * st);                                   // Ys, k, kb (7 each), yb0, yb1, lam, carry, bout
+    L.off_small = c.take(256ull * p.B + 4096);
+    L.off_inv = c.take(4ull * (3 * p.N + 4));
+    L.total = c.o;
     return L;
 }
 
@@ -1732,14 +1653,11 @@ int stage_dopri5_bwd(const DevProblem& p, int T, const Dopri5Record& rec, const 
     DpAdj d;
     for (int i = 0; i < 7; ++i) { d.Ys[i] = pl + (size_t)i * st; d.k[i] = pl + (size_t)(7 + i) * st; d.kb[i] = pl + (size_t)(14 + i) * st; }
     d.yb0 = pl + 21 * st; d.yb1 = pl + 22 * st; d.lam = pl + 23 * st; d.carry = pl + 24 * st; d.bout = pl + 25 * st;
-    char* sb = w + L.off_small;
-    auto grab = [&](size_t bytes) { char* r = sb; sb += (bytes + 15) / 16 * 16; return r; };
-    d.nidx = reinterpret_cast<int*>(grab(4 * B)); d.act = reinterpret_cast<int*>(grab(4 * B));
-    d.first = reinterpret_cast<int*>(grab(4 * B)); d.jptr = reinterpret_cast<int*>(grab(4 * B));
-    d.dtf = reinterpret_cast<float*>(grab(4 * B));
-    for (int i = 0; i < 7; ++i) d.tst[i] = reinterpret_cast<float*>(grab(4 * B));
+    TrialCarve g{w + L.off_small};
+    g(d.nidx, B); g(d.act, B); g(d.first, B); g(d.jptr, B); g(d.dtf, B);
+    for (int i = 0; i < 7; ++i) g(d.tst[i], B);
     DpState S;                                        // the forward stage kernels (k_dp_stage) run on this view
-    S.t = reinterpret_cast<double*>(grab(8 * B)); S.dt = reinterpret_cast<double*>(grab(8 * B));
+    g(S.t, B); g(S.dt, B);
     S.red = nullptr; S.next_out = S.n_acc = S.n_rej = S.status = nullptr; S.n_active = nullptr;
     S.active = d.act;
     for (int i = 0; i < 7; ++i) S.k[i] = d.k[i];
@@ -1756,32 +1674,32 @@ int stage_dopri5_bwd(const DevProblem& p, int T, const Dopri5Record& rec, const 
     for (int b = 0; b < p.B; ++b) { if (nacc[b] > rec.cap) return ODECOL_E_SHAPE; if (nacc[b] > rounds) rounds = nacc[b]; }
     std::vector<char> has_first(rounds + 1, 0);
     for (int b = 0; b < p.B; ++b) if (nacc[b] >= 1) has_first[nacc[b] - 1] = 1;
-    const int eg = cx.grid(st);
+    const int eg = ew_grid(st);
     for (int r = 0; r < rounds; ++r) {
         k_dpb_begin<<<p.B, 256, 0, s>>>(p, d, S, rec, n_accept, r);
         count_launch();
         // ---- recompute the seven stages (stage 0 = the recorded start state at t0)
-        rc = cx.rhs_t(d.Ys[0], d.tst[0], d.k[0]); if (rc) return rc;
+        rc = cx.drift.eval(0, d.Ys[0], d.tst[0], 0.f, d.k[0]); if (rc) return rc;
 #define ODECOL_DPB_STAGE(ST)                                                        \
         S.ys = d.Ys[ST]; S.t_stage = d.tst[ST];                                     \
         k_dp_stage<ST><<<eg, 256, 0, s>>>(p, S); count_launch();                    \
-        rc = cx.rhs_t(d.Ys[ST], d.tst[ST], d.k[ST]); if (rc) return rc;
+        rc = cx.drift.eval(0, d.Ys[ST], d.tst[ST], 0.f, d.k[ST]); if (rc) return rc;
         ODECOL_DPB_STAGE(1) ODECOL_DPB_STAGE(2) ODECOL_DPB_STAGE(3) ODECOL_DPB_STAGE(4) ODECOL_DPB_STAGE(5) ODECOL_DPB_STAGE(6)
 #undef ODECOL_DPB_STAGE
         // ---- dense output adjoint, then stages 7 .. 2
         k_dpb_dense<<<p.B, 256, 0, s>>>(p, d, rec, T, grad_y, inv, G);
         count_launch();
 #define ODECOL_DPB_BACK(ST)                                                                            \
-        rc = cx.vjp_t(d.Ys[ST], d.tst[ST], d.act, d.kb[ST], d.bout); if (rc) return rc;               \
+        rc = cx.vjp(d.Ys[ST], d.tst[ST], 0.f, d.act, d.kb[ST], d.bout); if (rc) return rc;            \
         k_dpb_push<ST><<<eg, 256, 0, s>>>(p, d); count_launch();
         ODECOL_DPB_BACK(6) ODECOL_DPB_BACK(5) ODECOL_DPB_BACK(4) ODECOL_DPB_BACK(3) ODECOL_DPB_BACK(2) ODECOL_DPB_BACK(1)
 #undef ODECOL_DPB_BACK
-        if (has_first[r]) { rc = cx.vjp_t(d.Ys[0], d.tst[0], d.first, d.kb[0], d.bout); if (rc) return rc; }
+        if (has_first[r]) { rc = cx.vjp(d.Ys[0], d.tst[0], 0.f, d.first, d.kb[0], d.bout); if (rc) return rc; }
         k_dpb_end<<<eg, 256, 0, s>>>(p, d, has_first[r] ? 1 : 0);
         count_launch();
     }
     // output 0 is y0 itself
-    k_add_out_grad<<<cx.grid((size_t)p.B * G), 256, 0, s>>>(p, grad_y, sel, G, 1.f, 0.f, d.lam, nullptr);
+    k_add_out_grad<<<ew_grid((size_t)p.B * G), 256, 0, s>>>(p, grad_y, sel, G, 1.f, 0.f, d.lam, nullptr);
     count_launch();
     if (grad_y0 && cudaMemcpyAsync(grad_y0, d.lam, sizeof(float) * st, cudaMemcpyDeviceToDevice, s) != cudaSuccess) return ODECOL_E_CUDA;
     return cudaGetLastError() == cudaSuccess ? ODECOL_OK : ODECOL_E_CUDA;
