@@ -151,9 +151,11 @@ size_t odecol_workspace_bytes(const odecol_problem* p, int op, int32_t T, int64_
  * (src/utils.py:13-46). */
 int odecol_rhs(const odecol_problem* p, const float* t, const float* y, float* f, void* stream);
 
-/* The same evaluation through the staged tensor-core path the large-network solvers use (operand split, 3xTF32
- * tcgen05 contraction with chunked accumulation for long rows, fast FP32-accurate phi): the unit the N = 8192 sweep
- * (BASELINE.json configs[4]) spends its time in.  Any N that is a multiple of 4; workspace:
+/* The same evaluation through the staged tensor-core path the large-network solvers use (operand split, tcgen05
+ * contraction with chunked accumulation for long rows, fast FP32-accurate phi), always in TF32 operand pairs (3xTF32).
+ * The solvers' forward solves, among them the N = 8192 sweep (BASELINE.json configs[4]), evaluate the same drift in
+ * FP16 operand pairs unless ODECOL_EM16 / ODECOL_DP16 / ODECOL_SRK16 is 0; sdeint(method='euler', dt=1, ts=[0, 1]) with
+ * zero increments returns y0 + f in that format.  Any N that is a multiple of 4; workspace:
  * odecol_workspace_bytes(p, ODECOL_OP_EM_FWD, 0, 0) sized for the STAGED family (set ODECOL_FLAG_FORCE_STAGED or
  * ODECOL_FLAG_FORCE_TENSOR on problems that would otherwise pick the on-chip family). */
 int odecol_drift_staged(const odecol_problem* p, const float* t, const float* y, float* f,

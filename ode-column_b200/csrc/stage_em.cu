@@ -783,7 +783,8 @@ int stage_em_fwd(const DevProblem& p, const float* ts_dev, int T, const float* y
 
 
 // One drift evaluation of the staged solvers, f[b] = forward(t[b], y[b]), as the sweeps above run it: operand kernel,
-// tensor-core contraction, RhsEpi.  Lets callers (and the parity tests) reach the unit C5 spends its time in.
+// tensor-core contraction, RhsEpi -- always in TF32 operand pairs.  The forward solves run the same unit in FP16 pairs
+// unless their switch is 0 (f16_switch below).
 int stage_drift(const DevProblem& p, const float* t_trial, const float* y, float* f, void* ws, size_t ws_bytes, cudaStream_t s) {
     using namespace tc;
     const EmLayout L = em_layout(p);

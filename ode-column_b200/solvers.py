@@ -349,7 +349,9 @@ def sdeint(sde, y0, ts, bm=None, method=None, dt=1e-3, adaptive=False, rtol=1e-5
     fresh BrownianInterval gives; ``torch.manual_seed`` reproduces a run); an int fixes the paths.  ``trial_offset``: the
     GLOBAL index of this call's first trial.  A job sharded over ranks or chunks passes ONE seed everywhere and
     ``trial_offset = lo`` of its block (``distributed.shard_bounds``): trial t then sees the same Brownian path wherever
-    it runs, and results do not depend on the sharding.
+    it runs, and results do not depend on the sharding -- with one exception: when a firing rate of some trial does not
+    fit the FP16 operand pairs of the staged solvers, they repeat the whole call in TF32 pairs, so that trial's batch mates
+    change in the last bits.
     ``options['sigma_scale']``: (B,) per-trial factor on the diffusion -- the noise-amplitude axis of a parameter sweep
     (trial b integrates with g = sigma_scale[b] * diffusion); ``options['lateral_gain']``: (B,) positive per-trial gain on
     the between-column recurrent weights (networks with ``lateral_split()``, e.g. ``SyntheticColumnSheet``; Euler-Maruyama,

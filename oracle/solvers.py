@@ -335,7 +335,7 @@ def adaptive_update(err: float, step: float, prev_ratio: Optional[float], safety
         pfactor, ifactor = 0.0, 1 / 1.5
     else:
         pfactor, ifactor = 0.13, 1 / 4.5
-    ratio = safety / err
+    ratio = safety / err if err > 0 else math.inf       # torchsde divides tensors: a zero error gives an infinite ratio
     if prev_ratio is None:
         prev_ratio = ratio
     factor = ratio ** ifactor * (ratio / prev_ratio) ** pfactor
@@ -347,10 +347,13 @@ def adaptive_update(err: float, step: float, prev_ratio: Optional[float], safety
 
 
 def sdeint_euler(sde, y0: torch.Tensor, ts: torch.Tensor, bm, dt: float = 1e-3, adaptive: bool = False,
-                 rtol: float = 1e-5, atol: float = 1e-4, dt_min: float = 1e-5, stats: Optional[Dict] = None):
+                 rtol: float = 1e-5, atol: float = 1e-4, dt_min: float = 1e-5, stats: Optional[Dict] = None,
+                 trace: Optional[List] = None):
     """torchsde ``BaseSDESolver.integrate`` with the Euler step.  Times stay in ts.dtype (float32 in the
     reference).  ``bm`` is any callable (t0, t1) -> (B, 1) increment (see TabulatedBrownian).  For the adaptive
-    controller bm must be a consistent path (W(a,c) = W(a,b) + W(b,c)), e.g. oracle.brownian.VirtualBrownianTree."""
+    controller bm must be a consistent path (W(a,c) = W(a,b) + W(b,c)), e.g. oracle.brownian.VirtualBrownianTree.
+    ``trace`` (a list, adaptive mode) receives one tuple (t0, t1, err, accepted) per attempted step, so a caller can
+    check which regime the controller ran in."""
     step = dt
     prev_t = curr_t = ts[0]
     prev_y = curr_y = y0
@@ -372,7 +375,10 @@ def sdeint_euler(sde, y0: torch.Tensor, ts: torch.Tensor, bm, dt: float = 1e-3, 
                 if step < dt_min:
                     step = dt_min
                     prev_ratio = None
-                if err <= 1 or step <= dt_min:
+                accepted = err <= 1 or step <= dt_min
+                if trace is not None:
+                    trace.append((float(curr_t), float(next_t), err, accepted))
+                if accepted:
                     prev_t, prev_y = curr_t, curr_y
                     curr_t, curr_y = next_t, y_half
                     n_acc += 1

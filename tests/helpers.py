@@ -100,6 +100,22 @@ def ext_problem(ext, lf, kt, ku, flags=0, device="cuda"):
                        n_in, ku.shape[0], lf.tau_s, lf.tau_m, lf.tau_a, lf.resistance, flags)
 
 
+class TreeBrownian:
+    """bm(t0, t1) for the oracle, reading the virtual Brownian tree of ONE trial through odecol_brownian_query -- the
+    path the kernels integrate against.  shape = (1, 1) like a torchsde Brownian object for one scalar-noise solve."""
+
+    def __init__(self, seed, trial, t_begin, t_end, device="cuda"):
+        self.ext = odecol._native.ext()
+        self.seed, self.trial, self.t_begin, self.t_end = seed, trial, float(t_begin), float(t_end)
+        self.device = device
+        self.shape = (1, 1)
+
+    def __call__(self, t0, t1):
+        q = torch.tensor([float(t0), float(t1)], dtype=torch.float32, device=self.device)
+        w = self.ext.brownian_query(self.seed, self.trial, 1, self.t_begin, self.t_end, q).cpu()
+        return (w[1] - w[0]).reshape(1, 1)
+
+
 def dopri5_controller_factor(ratio):
     """torchdiffeq's step factor after an ACCEPTED step with error ratio r: min(10, max(0.9 r^-1/5, 1))."""
     return 10.0 if ratio == 0 else min(10.0, max(0.9 * ratio ** -0.2, 1.0))

@@ -8,7 +8,8 @@
     trial by trial (torchsde controls the step of each solve on its own), first without noise, then on the SAME
     Brownian path (odecol_brownian_query exposes the virtual tree the kernels draw from);
   * C5: one drift evaluation at N = 8192 (K_aug = 9217: chunked accumulation, grouped tile order, 64 population tiles)
-    against the float64 oracle right-hand side.
+    against the float64 oracle right-hand side -- in TF32 pairs through odecol_drift_staged, and in the FP16 pairs the
+    sweep runs, with and without the per-member lateral gain, through one noiseless sdeint step.
 """
 import os
 
@@ -18,7 +19,7 @@ import torch
 
 import odecol
 from oracle import rhs as orhs, solvers as S
-from helpers import XOR_DICT, oracle_form, product_network, sheet_oracle_form
+from helpers import XOR_DICT, TreeBrownian, oracle_form, product_network, sheet_oracle_form
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
@@ -272,21 +273,6 @@ def test_staged_dopri5_and_srk_repeat_in_tf32_when_fp16_cannot_hold_the_operand(
 # ----------------------------------------------------------------------------------------------------------------------
 # adaptive Euler-Maruyama vs the oracle's step-doubling loop
 # ----------------------------------------------------------------------------------------------------------------------
-class _TreeBrownian:
-    """bm(t0, t1) for the oracle, reading the virtual Brownian tree of ONE trial through odecol_brownian_query -- the
-    path the kernels integrate against.  shape = (1, 1) like a torchsde Brownian object for one scalar-noise solve."""
-
-    def __init__(self, seed, trial, t_begin, t_end):
-        self.ext = odecol._native.ext()
-        self.seed, self.trial, self.t_begin, self.t_end = seed, trial, float(t_begin), float(t_end)
-        self.shape = (1, 1)
-
-    def __call__(self, t0, t1):
-        q = torch.tensor([float(t0), float(t1)], dtype=torch.float32, device=DEV)
-        w = self.ext.brownian_query(self.seed, self.trial, 1, self.t_begin, self.t_end, q).cpu()
-        return (w[1] - w[0]).reshape(1, 1)
-
-
 class _NoBrownian:
     shape = (1, 1)
 
@@ -362,7 +348,7 @@ def test_adaptive_euler_maruyama_matches_the_oracle_controller(kind, noise, cfg,
     blk = lambda a, c: a[..., c * N:(c + 1) * N]
 
     def both(tgrid):
-        bms = [(_TreeBrownian(seed, trial_offset + b, tgrid[0], tgrid[-1]) if noise else _NoBrownian()) for b in range(B)]
+        bms = [(TreeBrownian(seed, trial_offset + b, tgrid[0], tgrid[-1]) if noise else _NoBrownian()) for b in range(B)]
         yo_, nao_, nro_ = _oracle_adaptive(lf, kt, ku, tgrid, y0, sc.numpy(), bms, rtol, atol, dt, dt_min)
         st_ = {}
         with torch.no_grad():
@@ -436,6 +422,65 @@ def test_c5_drift_evaluation_matches_the_float64_oracle(cfg):
     print(f"\n[C5 drift N={N} B={B}] dV err / (sum|w||r| scale) {eV:.2e}; dA {eA:.1e}; dF {eF:.1e}; "
           f"dV rel to max|dV| {_relmax(f[:, :N].double(), fo[:, :N]):.1e}")
     assert eV < 4e-6 and eA < 2e-6 and eF < 2e-6
+
+
+@pytest.mark.parametrize("gain", [False, True], ids=["plain", "lateral_gain"])
+@pytest.mark.parametrize("cols,B", [(1024, 300), (125, 37)], ids=["N8192", "N1000"])
+def test_c5_sweep_drift_in_fp16_pairs_matches_the_float64_oracle(cfg, cols, B, gain):
+    """The drift the C5 sweep runs: FP16 operand pairs (ODECOL_EM16, on by default), chunked contraction (K_aug = 9217 /
+    1126), per-member lateral gain -- reached through the public sdeint.  One Euler-Maruyama step of h = 1 without noise
+    writes y[1] = y0 + f rounded once, so y[1] - y0 is the drift to ~1e-7.  N = 8192 with B = 300 leaves the last trial tile
+    ragged; N = 1000 pads the last population tile.  The stimulus ramp's knots straddle t = 0, where the step evaluates."""
+    N = 8 * cols
+    sheet = odecol.SyntheticColumnSheet(cfg, cols, seed=0, device=DEV)
+    gen = torch.Generator().manual_seed(cols + int(gain))
+    amp = torch.rand(B, cols, generator=gen) * 30.0
+    kt = torch.tensor([-0.25, 0.75])
+    ku = torch.stack((amp, amp * 0.5), 1)
+    sheet.set_knots(kt.to(DEV), ku.to(DEV))
+    y0 = torch.cat((torch.rand(B, N, generator=gen) * 10 - 8, torch.rand(B, N, generator=gen) * 2,
+                    torch.rand(B, N, generator=gen) * 3), 1).to(DEV)
+    g = torch.ones(B, dtype=torch.float64)
+    options = {}
+    if gain:
+        g = torch.rand(B, generator=gen).double() + 0.5
+        g[B // 3] = 1.0
+        options = {"lateral_gain": g.float()}
+    with torch.no_grad():
+        ys = odecol.sdeint(sheet, y0, torch.tensor([0.0, 1.0], device=DEV), bm=torch.zeros(1, B), method="euler", dt=1.0,
+                           options=dict(options))
+        # the same inputs through odecol_drift_staged, which evaluates in TF32 pairs
+        from ode_column_b200.solvers import _Setup
+        setup = _Setup(sheet, y0, torch.tensor([0.0, 1.0], device=DEV), None)
+        if gain:
+            setup.set_lateral_gain(sheet, options["lateral_gain"])
+        f32 = odecol._native.ext().drift_staged(setup.problem(setup.lf.W_aug), torch.zeros(B, device=DEV), y0)
+        y1_tf32 = y0 + f32
+    torch.cuda.synchronize()
+    assert torch.equal(ys[0], y0)
+    f = ys[1].double() - y0.double()
+    # float64 oracle (on the device, as plain torch): g_b (W_lat r) + W_loc (*) r + U s + bias
+    lf = sheet_oracle_form(sheet)
+    W_lat, W_loc = (x.detach().double() for x in sheet.lateral_split())
+    U, bias = torch.tensor(lf.U, dtype=torch.float64, device=DEV), torch.tensor(lf.bias, dtype=torch.float64, device=DEV)
+    kappa = torch.tensor(lf.kappa, dtype=torch.float64, device=DEV)
+    yd = y0.double()
+    V, A, F = yd[:, :N], yd[:, N:2 * N], yd[:, 2 * N:]
+    r = orhs.phi(V - A)
+    s = orhs.interp_knots(torch.tensor(0.0, dtype=torch.float64), kt.double(), ku.double()).to(DEV)
+    gd = g.to(DEV)[:, None]
+    loc = lambda W8, x: torch.einsum("cpj,bcj->bcp", W8.reshape(cols, 8, 8), x.reshape(B, cols, 8)).reshape(B, N)
+    cur = gd * (r @ W_lat.T) + loc(W_loc, r) + s @ U.T + bias
+    c = lf.tau_s * lf.resistance / lf.tau_m
+    fo = torch.cat(((cur * lf.tau_s * lf.resistance - V) / lf.tau_m, (kappa * r - A) / lf.tau_a, (r - F) / lf.tau_s), 1)
+    mag = (gd * (r.abs() @ W_lat.abs().T) + loc(W_loc.abs(), r.abs()) + s.abs() @ U.abs().T + bias.abs()) * c + V.abs() / lf.tau_m
+    eV = float(((f[:, :N] - fo[:, :N]).abs() / mag).max())
+    eA, eF = _relmax(f[:, N:2 * N], fo[:, N:2 * N]), _relmax(f[:, 2 * N:], fo[:, 2 * N:])
+    d16 = float((ys[1] - y1_tf32).abs().max()) / _scale(fo)
+    print(f"\n[C5 sweep drift, FP16 pairs, N={N} B={B} gain={gain}] dV err / (sum|w||r| scale) {eV:.2e}; dA {eA:.1e}; "
+          f"dF {eF:.1e}; FP16 vs TF32 pairs {d16:.1e} of max|f|")
+    assert eV < 4e-6 and eA < 2e-6 and eF < 2e-6
+    assert not torch.equal(ys[1], y1_tf32)                     # the FP16 contraction is the one that ran
 
 
 # ----------------------------------------------------------------------------------------------------------------------

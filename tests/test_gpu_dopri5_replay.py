@@ -1,5 +1,5 @@
-"""dopri5 beyond the random problems: the staged family on column sheets (N = 256, and N = 200, not a multiple of the
-128-row population tile) against a float64 replay of the recorded steps; the public odeint entry point on the same
+"""dopri5 beyond the random problems: the staged family on column sheets (N = 256; N = 200, not a multiple of the
+128-row population tile; N = 1024, whose contractions accumulate in chunks) against a float64 replay of the recorded steps; the public odeint entry point on the same
 computation at any record capacity; inputs the dopri5 path must reject (a time grid that is not strictly increasing)
 and repeated read-out components, which every solver must treat as torch.index_select does."""
 import numpy as np
@@ -34,8 +34,8 @@ def _sheet(cfg, cols, B, seed):
     return sheet, kt, ku, y0, gen
 
 
-@pytest.mark.parametrize("grid", list(SHEET_GRIDS))
-@pytest.mark.parametrize("cols", [32, 25], ids=["N256", "N200"])
+@pytest.mark.parametrize("cols,grid", [pytest.param(c, g, id=f"N{8 * c}-{g}") for g in SHEET_GRIDS for c in (32, 25)] +
+                         [pytest.param(128, "defaults", id="N1024-defaults")])      # K_aug = 1153: chunked contractions
 def test_staged_dopri5_on_column_sheets_against_a_float64_replay(cfg, cols, grid):
     rtol, atol, T = SHEET_GRIDS[grid]
     sheet, kt, ku, y0, _ = _sheet(cfg, cols, 3, seed=cols)

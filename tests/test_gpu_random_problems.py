@@ -163,16 +163,17 @@ def test_sde_solvers_on_random_problems(shape, method):
     assert et < 1e-5 and es < 2e-5 and e0 < 5e-5 and eW < 5e-5 and e0s < 5e-5 and eWs < 5e-5
 
 
-@pytest.mark.parametrize("method", ["srk", "euler"])
-def test_large_network_sde_gradients_through_the_public_api(method):
-    """N = 256 (two population tiles, beyond the on-chip family): sdeint(...).backward() through the staged reverse sweep
-    against the oracle's autograd, with the sheet module (W, U trainable) and a component selection."""
+@pytest.mark.parametrize("method,cols", [pytest.param(m, c, id=m if c == 32 else f"{m}-N1024") for c in (32, 128) for m in ("srk", "euler")])
+def test_large_network_sde_gradients_through_the_public_api(method, cols):
+    """N = 256 (two population tiles, beyond the on-chip family) and N = 1024 (K_aug = 1153: chunked contractions in the
+    FP16 forward solve and in the reverse sweep's VJP): sdeint(...).backward() through the staged reverse sweep against
+    the oracle's autograd, with the sheet module (W, U trainable) and a component selection."""
     import os
     cfg = odecol.load_config(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "config", "model.toml"))
-    sheet = odecol.SyntheticColumnSheet(cfg, 32, seed=1, device=DEV, sigma_v=2.0)
-    B, T, N = 3, 21, 256
+    sheet = odecol.SyntheticColumnSheet(cfg, cols, seed=1, device=DEV, sigma_v=2.0)
+    B, T, N = 3, 21, 8 * cols
     gen = torch.Generator().manual_seed(4)
-    amp = torch.rand(B, 32, generator=gen) * 20
+    amp = torch.rand(B, cols, generator=gen) * 20
     kt, ku = odecol.step_knots(5e-4, 1.5e-3, 2e-3, amp, 1e-4)
     sheet.set_knots(kt.to(DEV), ku.to(DEV))
     tv = torch.linspace(0, 2e-3, T)
@@ -180,12 +181,12 @@ def test_large_network_sde_gradients_through_the_public_api(method):
     n_steps = len(S.em_step_schedule(tv, dt))
     W, U = S.sample_w_u(n_steps, B, dt, gen)
     y0 = torch.cat((torch.rand(B, N, generator=gen) * 6 - 8, torch.rand(B, N, generator=gen), torch.rand(B, N, generator=gen)), 1)
-    sel = [0, 9, 255, 256 + 17, 512 + 3]
+    sel = [0, 9, N - 1, N + 17, 2 * N + 3]
     wgt = torch.randn(T, B, len(sel), generator=gen)
     # oracle on the sheet's linear form
     lfp = sheet.export_linear_form()
     Wa = lfp.W_aug.detach().cpu().numpy()
-    lf = LinearForm(W=Wa[:, :N], U=Wa[:, N:N + 32], bias=Wa[:, N + 32], kappa=lfp.kappa.cpu().numpy(), sigma=lfp.sigma.cpu().numpy(),
+    lf = LinearForm(W=Wa[:, :N], U=Wa[:, N:N + cols], bias=Wa[:, N + cols], kappa=lfp.kappa.cpu().numpy(), sigma=lfp.sigma.cpu().numpy(),
                     tau_s=lfp.tau_s, tau_m=lfp.tau_m, tau_a=lfp.tau_a, resistance=lfp.resistance)
     ode = orhs.UnifiedColumnODE(lf, kt.numpy(), ku.numpy(), requires_grad=True)
     y0o = y0.clone().requires_grad_(True)
@@ -204,7 +205,7 @@ def test_large_network_sde_gradients_through_the_public_api(method):
     e0 = float((y0p.grad.cpu() - y0o.grad).abs().max()) / scale(y0o.grad)
     eW = float((sheet.recurrent_weights.grad.cpu() - ode.W.grad).abs().max()) / scale(ode.W.grad)
     eU = float((sheet.input_weights.grad.cpu() - ode.U.grad).abs().max()) / scale(ode.U.grad)
-    print(f"\n[{method} N=256] trajectory {et:.1e}  grad y0 {e0:.1e}  grad W {eW:.1e}  grad U {eU:.1e}")
+    print(f"\n[{method} N={N}] trajectory {et:.1e}  grad y0 {e0:.1e}  grad W {eW:.1e}  grad U {eU:.1e}")
     assert et < 1e-5 and e0 < 5e-5 and eW < 5e-5 and eU < 5e-5
 
 

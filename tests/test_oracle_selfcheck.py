@@ -133,6 +133,44 @@ def test_adaptive_controller_limits():
     assert s == 1.0
 
 
+class _PiecewiseLinearPath:
+    """A consistent Brownian path for the adaptive loop: W linear between the points of a fine random walk."""
+    shape = (1, 1)
+
+    def __init__(self, span, n, seed):
+        g = torch.Generator().manual_seed(seed)
+        self.t = torch.linspace(0.0, span, n + 1, dtype=torch.float64)
+        self.w = torch.cat((torch.zeros(1), torch.randn(n, generator=g).double().cumsum(0) * math.sqrt(span / n)))
+
+    def _at(self, t):
+        return float(np.interp(float(t), self.t.numpy(), self.w.numpy()))
+
+    def __call__(self, t0, t1):
+        return torch.tensor([[self._at(t1) - self._at(t0)]], dtype=torch.float32)
+
+
+@pytest.mark.parametrize("rtol,atol", [(1e-3, 1e-3), (1e-12, 1e-12)], ids=["controlled", "at_dt_min"])
+def test_adaptive_euler_trace_records_the_attempts_and_changes_no_result(rtol, atol):
+    ts = torch.linspace(0.0, 0.5, 6)
+    y0 = torch.tensor([[1.0], [-0.5]])
+    bm = _PiecewiseLinearPath(0.5, 4096, seed=3)
+    kw = dict(dt=0.05, adaptive=True, rtol=rtol, atol=atol, dt_min=5e-3)
+    st_a, st_b, trace = {}, {}, []
+    ya = S.sdeint_euler(_OU(2.0, 0.7), y0, ts, bm, stats=st_a, **kw)
+    yb = S.sdeint_euler(_OU(2.0, 0.7), y0, ts, bm, stats=st_b, trace=trace, **kw)
+    assert torch.equal(ya, yb) and st_a == st_b
+    assert len(trace) == st_a["n_accept"] + st_a["n_reject"] and sum(a for *_, a in trace) == st_a["n_accept"]
+    assert st_a["n_reject"] > 0
+    # accepted attempts tile [ts[0], ts[-1]]; a rejected one restarts from the same t0
+    t_cur = float(ts[0])
+    for t0, t1, err, accepted in trace:
+        assert t0 == t_cur and t1 > t0 and err >= 0
+        assert accepted or err > 1
+        if accepted:
+            t_cur = t1
+    assert t_cur == float(ts[-1])
+
+
 # ---------------------------------------------------------------------------------------------------------------
 # torchsde method='srk' (SRI2 / "SRID2" tableau) restatement
 # ---------------------------------------------------------------------------------------------------------------
