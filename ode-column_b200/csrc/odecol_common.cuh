@@ -36,7 +36,8 @@ ODECOL_DEVINL void phi_dphi(float x, float& r, float& dr) {
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// fast, FP32-accurate (about 1e-7 relative) elementwise math (the staged families' epilogues; the on-chip family on request)
+// fast, FP32-accurate elementwise math (the staged families' epilogues; the on-chip family on request); phi within 5e-6 of
+// float64 over its whole range (tests/test_gpu_rate_range.py)
 // ---------------------------------------------------------------------------------------------------------------
 ODECOL_DEVINL float exp_fast(float x) {            // |x| < 87
     const float n = rintf(x * 1.4426950408889634f);
@@ -77,19 +78,46 @@ ODECOL_DEVINL float rcp_fast(float x) {
     asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
     return r;
 }
+// phi's removable pole at x = 981/48 (x_nom = 0, phi -> 1/0.0089 = 112.36 Hz, phi' -> 24): phi is smooth there, but the
+// quotient x_nom / (1 - exp(z)) cancels.  An error eps in exp(z) becomes eps / |v| in phi and about 2 eps / v^2 in phi'
+// (v = -z, about 0.43 (x - 981/48)); at the pole itself the quotient is 0 * inf = NaN.  Inside |v| < kPhiPoleBand
+// (|x - 981/48| < 0.58) the fast path takes the same function without a quotient of small numbers: phi = G(v) / 0.0089 with
+// G = R(u) B(v), R = u / tanh u (u = 0.0089 x_nom / 80 = atanh(v / 80), so R = 1 + v^2 / 19200 + O(v^4 1e-8)) and
+// B(v) = v / (1 - exp(-v)) = 1 + v/2 + v^2/12 - v^4/720 + O(v^6 / 30240); phi' = 48 G'(v) (1 - tanh^2 u).  In the band
+// the series is off by less than 1e-7 in phi and 6e-7 in phi' (float32 emulation against float64); the quotient, with
+// ex2.approx one ulp off, would be off by 2e-7 and 2e-6 at the band's edge.  The choice is a select, not a branch.
+// The reference arithmetic (phi, phi_dphi above) keeps the quotient, NaN included.
+constexpr float kPhiPoleBand = 0.25f;
+constexpr float kG2 = 1.0f / 12.0f + 1.0f / 19200.0f, kG3 = 1.0f / 38400.0f, kG4 = -1.0f / 720.0f + 1.0f / 230400.0f;
+
 ODECOL_DEVINL float phi_fast(float x) {
     const float x_nom = fmaf(48.0f, x, -981.0f);
     const float th = tanh_small(x_nom * (-0.0089f / 80.0f));
-    return x_nom * rcp_fast(1.0f - exp80_fast(th));
+    const float v = -80.0f * th;
+    const float G = fmaf(v, fmaf(v, fmaf(v, fmaf(v, kG4, kG3), kG2), 0.5f), 1.0f);
+    const float r = x_nom * rcp_fast(1.0f - exp80_fast(th));
+    return fabsf(v) < kPhiPoleBand ? (1.0f / 0.0089f) * G : r;
 }
 
+// phi' = 48 (s1 + s2 (1 - th^2)): s1 = inv and s2 = -0.0089 r inv e from the quotient; in the band, with G = R(u) B(v)
+// differentiated factor by factor, s1 = R'(u) B / 80 (R' = 2u/3) and s2 = R B'(v).  (This form, rather than G'(v), is
+// the one that keeps the register-resident reverse kernel k_rk4_bwd_small<40, true> within 168 registers without spilling.)
 ODECOL_DEVINL void phi_dphi_fast(float x, float& r, float& dr) {
     const float x_nom = fmaf(48.0f, x, -981.0f);
-    const float th = tanh_small(x_nom * (-0.0089f / 80.0f));
+    const float a = x_nom * (-0.0089f / 80.0f);          // -u
+    const float th = tanh_small(a);
     const float e = exp80_fast(th);
     const float inv = rcp_fast(1.0f - e);
-    r = x_nom * inv;
-    dr = 48.0f * (inv + r * inv * e * (1.0f - th * th) * (-0.0089f));
+    const float v = -80.0f * th, w = v * v;
+    const float R = fmaf(a * a, 1.0f / 3.0f, 1.0f);
+    const float B = fmaf(v, fmaf(v, fmaf(w, -1.0f / 720.0f, 1.0f / 12.0f), 0.5f), 1.0f);   // 1 + v/2 + v^2/12 - v^4/720
+    const float dB = fmaf(v, fmaf(w, -1.0f / 180.0f, 1.0f / 6.0f), 0.5f);                 // 1/2 + v/6 - v^3/180
+    const bool near = fabsf(v) < kPhiPoleBand;
+    const float rq = x_nom * inv;
+    r = near ? (1.0f / 0.0089f) * R * B : rq;
+    const float s1 = near ? a * B * (-1.0f / 120.0f) : inv;
+    const float s2 = near ? R * dB : rq * inv * e * (-0.0089f);
+    dr = 48.0f * fmaf(s2, 1.0f - th * th, s1);
 }
 
 // ---- stimulus lookup (reference src/utils.py:31-46) ------------------------------------------------------------
